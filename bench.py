@@ -4,6 +4,10 @@ the dominant kernel and the reference CPU engine timed beside it.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            our CUDA path (one process per GPU)
   python bench.py --impl reference [--gpus N] [--steps K] ...    the reference CPU engine on the host cores
+  python bench.py --dump-outputs DIR ...                          also write the last timed step's outputs to DIR/*.npy
+
+The headline figure is ONE timed region of exactly K steps after W warm-up steps, so the engines' state after it
+depends on the arguments alone: two builds run with the same arguments can be compared output for output.
 
 Workload (BASELINE.json configs[2], "C3"): 40x40 battle, 64 v 64 agents, 4096 lock-stepped environments per
 GPU, synthetic uniform-random actions, episodes auto-reset at done / 400 steps.  One "step" = one lockstep
@@ -27,7 +31,7 @@ REPO = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(REPO, "mean-field-multi-agent-reinforcement-learning_b200")
 if os.path.join(PKG, "python") not in sys.path:
     sys.path.insert(0, os.path.join(PKG, "python"))
-MIN_REGION_SECONDS = 0.5      # the K-step timed region is repeated until this much device time has been measured
+DUMP_BYTES = 64 << 20        # --dump-outputs: budget of the .npy files
 
 
 def _checker_paths():
@@ -264,13 +268,9 @@ class Ctx:
             self.dist.destroy_process_group()
 
 
-def repeat_count(ctx, first_region_ms, min_seconds, cap=400):
-    """how often the K-step region is timed: enough for min_seconds of device time and at least 3 times (a median needs
-    them) unless one region already takes seconds; the same number on every rank"""
-    r = int(min(cap, max(1, -(-min_seconds * 1e3 // max(first_region_ms, 1e-3)))))
-    if first_region_ms < 2000.0:
-        r = max(r, 3)
-    return int(ctx.reduce([r], "max")[0])
+def reduce_region(ctx, region_ms, region_work):
+    """one timed region over the ranks: time = max, work = sum"""
+    return ctx.reduce([region_ms], "max")[0], ctx.reduce([region_work], "sum")[0]
 
 
 def pick_median(ctx, region_ms, region_work):
@@ -284,10 +284,45 @@ def pick_median(ctx, region_ms, region_work):
                         "reported": t[m]}
 
 
-def measure_battle(ctx, args, workload, K, W, min_seconds, envs_per_gpu=0, pipeline=None, obs_tile=None, extras=True):
-    """One battle workload on this rank's GPU: W warm-up steps, then the region of EXACTLY K lockstep steps timed
-    `repeats` times (each bracketed by a barrier + synchronize; CUDA events on the launching streams), the e2e variant
-    the same way.  Returns the JSON fields of the workload (rank 0) -- every rank must call it."""
+def dump_battle_outputs(out_dir, last, nums):
+    """--dump-outputs: what the last timed step handed its caller, as float32 .npy files.  From k_step: reward, alive
+    and mean_action per env and group, done per env; from k_obs: view and feature rows.  Rows at or past an env's agent
+    count `num` (taken before the step) are stale in the engine's buffers and written as zeros.  The observations of a
+    fixed, seeded sample of whole environments (obs_envs) fill half of the DUMP_BYTES budget; the step outputs cover
+    every environment unless they would not fit the other half either (step_envs)."""
+    import numpy as np
+    import torch
+    num = torch.cat(nums).long()                                        # [E, 2]
+    reward, alive, done, mean = (torch.cat([l[1][i] for l in last]) for i in range(4))
+    E, _, cap = reward.shape
+    Eh = E // len(last)
+    view_row, feat_row = last[0][0][0][0, 0, 0].numel(), last[0][0][1].shape[-1]
+    rng = np.random.RandomState(0)
+
+    def envs_within(per_env_bytes):
+        n = min(E, max(1, (DUMP_BYTES // 2) // per_env_bytes))
+        return np.arange(E) if n == E else np.sort(rng.choice(E, n, replace=False))
+
+    obs_envs = envs_within(2 * cap * (view_row + feat_row) * 4)
+    step_envs = envs_within(2 * cap * 8 + mean.shape[-1] * 8 + 12)
+    live = torch.arange(cap, device=num.device) < num[..., None]       # [E, 2, cap]
+    view = torch.stack([last[e // Eh][0][0][e % Eh] for e in obs_envs])
+    feat = torch.stack([last[e // Eh][0][1][e % Eh] for e in obs_envs])
+    lo, ls = live[torch.from_numpy(obs_envs).to(num.device)], torch.from_numpy(step_envs).to(num.device)
+    out = {"num": num[ls], "reward": torch.where(live, reward, 0.0)[ls], "alive": torch.where(live, alive.float(), 0.0)[ls],
+           "done": done[ls], "mean_action": mean[ls], "step_envs": torch.from_numpy(step_envs),
+           "view": torch.where(lo[..., None, None, None], view, 0.0), "feature": torch.where(lo[..., None], feat, 0.0),
+           "obs_envs": torch.from_numpy(obs_envs)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
+def measure_battle(ctx, args, workload, K, W, envs_per_gpu=0, pipeline=None, obs_tile=None, extras=True, dump=None):
+    """One battle workload on this rank's GPU: W warm-up steps, then ONE region of exactly K lockstep steps (bracketed
+    by a barrier + synchronize; CUDA events on the launching streams), the e2e variant the same way.  With `dump` (a
+    directory), rank 0 writes what the last timed step returned before anything else runs.  Returns the JSON fields of
+    the workload (rank 0) -- every rank must call it."""
     torch = ctx.torch
     from mfmarl_b200 import BatchedGridWorld
     wl = WORKLOADS[workload]
@@ -321,13 +356,15 @@ def measure_battle(ctx, args, workload, K, W, min_seconds, envs_per_gpu=0, pipel
     def agent_steps_total():
         return sum(int(env.get("agent_steps").sum()) for env in envs)
 
+    last = [None] * P                                  # per engine: (observe(), step()) of its latest step
+
     def one_step(h, env, k, events=None):
         st = streams[h]
         with torch.cuda.stream(st):
             if events: events[0].record(st)
-            env.observe()
+            obs = env.observe()
             if events: events[1].record(st)
-            env.step(pool[h][k % POOL])
+            last[h] = (obs, env.step(pool[h][k % POOL]))
             if events: events[2].record(st)
 
     for k in range(W):
@@ -335,7 +372,11 @@ def measure_battle(ctx, args, workload, K, W, min_seconds, envs_per_gpu=0, pipel
             one_step(h, env, k)
     ctx.barrier()
 
-    def timed_region(with_events):
+    dump = dump if rank == 0 else None
+    num_alias = [env.device_state("num") for env in envs] if dump else None
+    nums = [None] * P
+
+    def timed_region(with_events, keep_num=False):
         ev = [[[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(K)] for _ in range(P)] if with_events else None
         t0 = torch.cuda.Event(enable_timing=True)
         t1 = [torch.cuda.Event(enable_timing=True) for _ in range(P)]
@@ -347,28 +388,28 @@ def measure_battle(ctx, args, workload, K, W, min_seconds, envs_per_gpu=0, pipel
             streams[h].wait_event(t0)
         for k in range(K):
             for h, env in enumerate(envs):
+                if keep_num and k == K - 1:            # agent counts the last step starts from (the dump's row mask)
+                    with torch.cuda.stream(streams[h]):
+                        nums[h] = num_alias[h].clone()
                 one_step(h, env, k, ev[h][k] if ev else None)
         for h in range(P):
             t1[h].record(streams[h])
         ctx.barrier()
         return max(t0.elapsed_time(t) for t in t1), agent_steps_total() - a0, ev
 
-    # ---- timed regions: exactly K steps each ----
+    # ---- the timed region: exactly K steps ----
     with ClockSampler(local) as clocks:
-        ms0, work0, ev = timed_region(True)
-        R = repeat_count(ctx, ms0, min_seconds)
-        region_ms, region_work = [ms0], [work0]
-        for _ in range(R - 1):
-            m, w_, _e = timed_region(False)
-            region_ms.append(m); region_work.append(w_)
-    ms, agent_steps_all, regions = pick_median(ctx, region_ms, region_work)
-    agent_steps = work0                                                             # this rank, first region (kernel attribution)
+        ms0, work0, _e = timed_region(False, keep_num=bool(dump))
+    if dump:
+        dump_battle_outputs(dump, last, nums)
+    ms, agent_steps_all = reduce_region(ctx, ms0, work0)
+    # ---- kernel attribution: the next K steps again, with event pairs around every launch ----
+    _m, agent_steps, ev = timed_region(True)                                        # this rank
     obs_ms = sum(e[0].elapsed_time(e[1]) for evh in ev for e in evh) / (K * P)     # per k_obs launch
     step_ms = sum(e[1].elapsed_time(e[2]) for evh in ev for e in evh) / (K * P)    # per k_step launch
 
     # ---- the same region on FRESH episodes (armies at full strength), as round 1 measured it: reset, W warm-up steps,
-    #      K timed steps, five times.  The regions above run on into the steady state of the 400-step episodes, where
-    #      uniform random actions have killed ~8 % of the agents and the per-step fixed costs weigh a little more. ----
+    #      K timed steps, five times; the median and the spread of the five sit beside the single timed region. ----
     fresh = None
     if extras:
         f_ms, f_work = [], []
@@ -449,12 +490,7 @@ def measure_battle(ctx, args, workload, K, W, min_seconds, envs_per_gpu=0, pipel
         return max(e0.elapsed_time(t) for t in e1), agent_steps_total() - a0
 
     m0, w0 = e2e_region()
-    Re = repeat_count(ctx, m0, min_seconds)
-    e_ms, e_work = [m0], [w0]
-    for _ in range(Re - 1):
-        m, w_ = e2e_region()
-        e_ms.append(m); e_work.append(w_)
-    e2e_ms, e2e_all, e2e_regions = pick_median(ctx, e_ms, e_work)
+    e2e_ms, e2e_all = reduce_region(ctx, m0, w0)
     h2d = P * h_act[0][0].numel() * 4
     d2h = P * sum(t.numel() * t.element_size() for t in results[0][0])
 
@@ -508,14 +544,13 @@ def measure_battle(ctx, args, workload, K, W, min_seconds, envs_per_gpu=0, pipel
                    "sharding": "envs [r*E,(r+1)*E) on rank r, no collective on the env path",
                    "pipeline": "%d engine(s) x %d envs on %d stream(s)" % (P, Eh, P),
                    "obs_tile_agents": tile or "engine default",
-                   "timed_region": "exactly %d steps, repeated %d times (>= %.2f s of device time); the repeat with the "
-                                   "median time is reported" % (K, regions["repeats"], min_seconds)},
-        "region_ms": regions,
+                   "timed_region": "exactly %d steps, once, after %d warm-up steps" % (K, W)},
+        "region_ms": ms,
         "agents_per_step": agent_steps_all / K,
         "fresh_episodes": fresh,
         "gpu_launches": 2 * K * P,
         "kernels_ms": {"k_obs": obs_ms, "k_step": step_ms,
-                       "note": "event pairs on the launching streams inside the first timed region" +
+                       "note": "event pairs on the launching streams, in a second region of K steps after the timed one" +
                                ("; with %d streams they include time shared with the other engine's kernel" % P
                                 if P > 1 else "")},
         "kernels_alone_ms": alone,
@@ -538,12 +573,15 @@ def measure_battle(ctx, args, workload, K, W, min_seconds, envs_per_gpu=0, pipel
                          "frac": alone["agents_per_launch"] * BYTES_PER_AGENT_OBS / (alone["k_obs"] * 1e-3) / 1e9 / peak,
                          "note": "k_obs launched with nothing else on the GPU (short run after the timed regions)"}},
         "e2e": {"value": e2e_all / (e2e_ms * 1e-3), "unit": "agent-steps/s", "h2d_bytes_per_step": h2d,
-                "d2h_bytes_per_step": d2h, "region_ms": e2e_regions,
+                "d2h_bytes_per_step": d2h, "region_ms": e2e_ms,
                 "note": "mfb_step_host_async: actions from pinned host memory, rewards/alive/done/mean action "
                         "copied back to pinned host memory and waited for every step (copies pipelined under "
                         "k_obs); observations stay in HBM for the policy network",
                 "with_observations_to_host": obs_host},
         "clocks": clocks.summary(),
+        "dump_outputs": None if not dump else {
+            "dir": dump, "note": "the timed region also held %d device copies of the agent counts (%d B each), "
+                                 "enqueued before its last step for the dump's row mask" % (P, Eh * 2 * 4)},
     }
 
 
@@ -581,13 +619,13 @@ def measure_grad_allreduce(ctx, iters=20):
 
 def run_ours(args):
     ctx = Ctx()
-    main = measure_battle(ctx, args, args.workload, args.steps, args.warmup, MIN_REGION_SECONDS,
-                          envs_per_gpu=args.envs, obs_tile=args.obs_tile)
+    main = measure_battle(ctx, args, args.workload, args.steps, args.warmup,
+                          envs_per_gpu=args.envs, obs_tile=args.obs_tile, dump=args.dump_outputs)
     also = {}
     if args.workload == "c3" and not args.no_also:
         # the other two named shapes under the same clock (BASELINE configs[3] and [4]): shorter legs, same rules
-        c4 = measure_battle(ctx, args, "c4", 200, max(3, min(args.warmup, 10)), 0.25, pipeline=2, obs_tile=0, extras=False)
-        c5 = measure_ising(ctx, args, min(max(args.steps, 100), 200), max(3, args.warmup), 0.25)
+        c4 = measure_battle(ctx, args, "c4", 200, max(3, min(args.warmup, 10)), pipeline=2, obs_tile=0, extras=False)
+        c5 = measure_ising(ctx, args, min(max(args.steps, 100), 200), max(3, args.warmup))
         if ctx.rank == 0:
             keep = ("metric", "value", "unit", "ms_per_step", "scaling", "config", "region_ms", "roofline", "e2e",
                     "gpu_launches", "kernels_alone_ms", "sweeps_per_launch")
@@ -637,9 +675,9 @@ def ising_cpu_sample(side, lattices, sweeps, T, lr):
     return lattices * side * side * sweeps / secs, secs
 
 
-def measure_ising(ctx, args, K, W, min_seconds):
-    """BASELINE configs[4] on this rank's shard of the lattices: the region of exactly K sweeps, repeated to
-    min_seconds; every rank must call it, rank 0 gets the JSON fields."""
+def measure_ising(ctx, args, K, W):
+    """BASELINE configs[4] on this rank's shard of the lattices: one region of exactly K sweeps; every rank must call
+    it, rank 0 gets the JSON fields."""
     torch = ctx.torch
     from mfmarl_b200 import IsingMFQ
     dev, world, rank, local = ctx.dev, ctx.world, ctx.rank, ctx.local
@@ -680,9 +718,7 @@ def measure_ising(ctx, args, K, W, min_seconds):
 
     with ClockSampler(local) as clocks:
         m0 = region()
-        R = repeat_count(ctx, m0, min_seconds, cap=50)
-        r_ms = [m0] + [region() for _ in range(R - 1)]
-    ms, _w, regions = pick_median(ctx, r_ms, [B * L * L * K] * len(r_ms))
+    ms = ctx.reduce([m0], "max")[0]
     # e2e: what the driver loop of main_MFQ_Ising.py reads every sweep (up counts -> order parameter) lands in
     # pinned host memory; the temperature schedule goes host -> device with every launch
     h_up = torch.empty((S, B), dtype=torch.int32).pin_memory()
@@ -705,10 +741,7 @@ def measure_ising(ctx, args, K, W, min_seconds):
         ctx.barrier()
         return e0.elapsed_time(e1)
 
-    e0_ = e2e_region()
-    Re = repeat_count(ctx, e0_, min_seconds, cap=50)
-    e_ms = [e0_] + [e2e_region() for _ in range(Re - 1)]
-    e2e_ms, _w2, e2e_regions = pick_median(ctx, e_ms, [B * L * L * K] * len(e_ms))
+    e2e_ms = ctx.reduce([e2e_region()], "max")[0]
     order_mean = float(model.order_param().mean())
     del model
     torch.cuda.empty_cache()
@@ -726,9 +759,8 @@ def measure_ising(ctx, args, K, W, min_seconds):
         "config": {"workload": wl["name"], "lattices_total": B * world, "lattices_per_gpu": B, "side": L,
                    "temperature": T, "lr": wl["lr"], "rng": "philox(seed, lattice, column, band, step)",
                    "l2": "Q + spins per GPU (%.1f GB) exceed the 126 MB L2" % (B * L * L * 41 / 1e9),
-                   "timed_region": "exactly %d sweeps, repeated %d times; the repeat with the median time is reported"
-                                   % (K, regions["repeats"])},
-        "region_ms": regions,
+                   "timed_region": "exactly %d sweeps, once, after the warm-up" % K},
+        "region_ms": ms,
         "gpu_launches": K // S,
         "sweeps_per_launch": S,
         "roofline": {"bound": "hbm", "kernel": kernel, "achieved": achieved, "peak": peak, "unit": "GB/s",
@@ -742,7 +774,7 @@ def measure_ising(ctx, args, K, W, min_seconds):
                               "site-step, so frac > 1 means it beats the streaming bound" % (S, S)) if resident else
                              "streaming kernel: Q pair read + one value written + spins per site-step"},
         "e2e": {"value": sites * K / (e2e_ms * 1e-3), "unit": "site-steps/s", "h2d_bytes_per_step": 4 if resident else 0,
-                "d2h_bytes_per_step": B * 4, "region_ms": e2e_regions,
+                "d2h_bytes_per_step": B * 4, "region_ms": e2e_ms,
                 "note": "temperatures from pinned host memory per launch (a scalar argument when streaming); the "
                         "per-sweep up counts (order parameter) are read back to pinned host memory and waited "
                         "for after every launch"},
@@ -753,7 +785,7 @@ def measure_ising(ctx, args, K, W, min_seconds):
 
 def run_ising(args):
     ctx = Ctx()
-    line = measure_ising(ctx, args, args.steps, args.warmup, MIN_REGION_SECONDS)
+    line = measure_ising(ctx, args, args.steps, args.warmup)
     if ctx.rank == 0:
         wl = WORKLOADS["c5"]
         if ctx.world == 1 and not args.no_cpu:
@@ -911,7 +943,13 @@ def main():
     ap.add_argument("--step-threads", type=int, default=0, help="threads per k_step CTA (tuning; 0 = auto)")
     ap.add_argument("--no-also", action="store_true",
                     help="skip the extra legs of the default line (C4, C5, and the gradient all-reduce when N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="battle workloads: write what the last timed step returned (rank 0's environments) to "
+                         "DIR/<name>.npy, float32, at most 64 MB.  The row mask needs the agent counts the last step "
+                         "starts from, so one small device copy per engine is enqueued inside the timed region")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in ("c3", "c4")):
+        ap.error("--dump-outputs: only the battle workloads c3 and c4 of --impl ours")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

@@ -1,6 +1,7 @@
 """CPU: pins the numpy Ising oracle against the UNMODIFIED reference classes (run under the gym/imp shim
-of oracle/ising_ref_shim) with injected uniforms -- exact float64 equality.  Skipped when /root/reference
-is absent (e.g. on the GPU box); the golden fixture test in test_golden.py covers that case."""
+of oracle/ising_ref_shim) with injected uniforms -- exact float64 equality.  The comparison is skipped when the
+reference tree is absent.  Without it only test_golden.py checks the oracle against the reference, on the one stored
+20x20 run at T = 0.8 (tests/golden/ising20.npz); the other sizes and temperatures below are not covered then."""
 import os
 import sys
 
@@ -13,8 +14,6 @@ sys.path.insert(0, os.path.join(REPO, "oracle"))
 import ising_oracle  # noqa: E402
 
 REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "examples", "ising_model")),
-                                reason="reference tree not present")
 
 
 def reference_env(n_agents, seed):
@@ -31,6 +30,7 @@ def reference_env(n_agents, seed):
     return env
 
 
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "examples", "ising_model")), reason="reference tree not present")
 @pytest.mark.filterwarnings("ignore::DeprecationWarning")
 @pytest.mark.parametrize("n,T,steps", [(400, 0.8, 25), (100, 0.297, 40), (49, 2.0, 30)])
 def test_oracle_equals_reference_loop_body(n, T, steps):

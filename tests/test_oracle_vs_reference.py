@@ -1,6 +1,6 @@
 """Pins the plain-C oracle (oracle/magent_oracle.c) against the reference engine itself
 (oracle/_ref/libmagent_ref.so, built from /root/reference by oracle/Makefile, OMP_NUM_THREADS=1).
-CPU only.  Skipped when the reference build is not present."""
+CPU only.  The tests that run the reference are skipped when its build is not present."""
 import numpy as np
 import pytest
 
@@ -8,9 +8,10 @@ from engines import OracleEngine, RefEngine, have_ref
 from lockstep import assert_same, run_lockstep, setup_pair
 from scenarios import c4_positions, generate_map_positions
 
-pytestmark = pytest.mark.skipif(not have_ref(), reason="oracle/_ref/libmagent_ref.so not built")
+needs_ref = pytest.mark.skipif(not have_ref(), reason="oracle/_ref/libmagent_ref.so not built")
 
 
+@needs_ref
 def test_spaces_and_action_table():
     ref, ora = RefEngine(40), OracleEngine(40)
     assert ref.env.view_space[0] == (ora.vs, ora.vs, ora.nc) == (13, 13, 7)
@@ -32,6 +33,7 @@ def test_minstd_rand0_matches_libstdcxx():
     assert [ora.rng_next() for _ in range(4)] == [16807, 282475249, 1622650073, 984943658]
 
 
+@needs_ref
 @pytest.mark.parametrize("seed", [0, 1])
 def test_battle40_fight_stream(seed):
     ref, ora = RefEngine(40), OracleEngine(40)
@@ -42,12 +44,14 @@ def test_battle40_fight_stream(seed):
     assert st["deaths"] > 20, st
 
 
+@needs_ref
 def test_battle40_uniform_stream():
     ref, ora = RefEngine(40), OracleEngine(40)
     setup_pair([ref, ora], *generate_map_positions(40))
     run_lockstep(ref, ora, steps=60, seed=3, stream="uniform")
 
 
+@needs_ref
 def test_battle80_512v512():
     ref, ora = RefEngine(80), OracleEngine(80)
     setup_pair([ref, ora], *c4_positions())
@@ -55,6 +59,7 @@ def test_battle80_512v512():
     assert st["deaths"] > 20, st
 
 
+@needs_ref
 def test_second_episode_keeps_rng_and_resets_ids():
     """reset() restarts ids at 0 but never reseeds the engine RNG (GridWorld.cc:76-124)."""
     ref, ora = RefEngine(40), OracleEngine(40)
@@ -63,6 +68,7 @@ def test_second_episode_keeps_rng_and_resets_ids():
         run_lockstep(ref, ora, steps=40, seed=10 + ep, stream="fight", check_obs_every=10)
 
 
+@needs_ref
 def test_set_seed_and_occupied_positions_are_skipped():
     ref, ora = RefEngine(40), OracleEngine(40)
     for e in (ref, ora):
@@ -75,6 +81,7 @@ def test_set_seed_and_occupied_positions_are_skipped():
     run_lockstep(ref, ora, steps=50, seed=7, stream="fight", check_obs_every=10)
 
 
+@needs_ref
 def test_inner_walls_and_observation_before_clear_dead():
     ref, ora = RefEngine(40), OracleEngine(40)
     walls = np.array([[20, y] for y in range(5, 35, 3)] + [[19, 20], [21, 20]], np.int32)
@@ -84,6 +91,7 @@ def test_inner_walls_and_observation_before_clear_dead():
     run_lockstep(ref, ora, steps=120, seed=11, stream="fight", skip_clear_every=4)
 
 
+@needs_ref
 def test_mean_info_matches():
     ref, ora = RefEngine(40), OracleEngine(40)
     setup_pair([ref, ora], *generate_map_positions(40))
@@ -95,6 +103,7 @@ def test_mean_info_matches():
     run_lockstep(ref, ora, steps=30, seed=2, stream="fight", check_obs_every=0, on_step=check)
 
 
+@needs_ref
 @pytest.mark.parametrize("size", [100, 104])
 def test_large_map_mode_moves_run_band_by_band(size):
     """W*H > 99*99 switches the reference to large_map_mode (GridWorld.cc:79-88): moves are filed into x-band
