@@ -104,6 +104,20 @@ int mfb_clear_dead(mfb_engine *eng, void *stream);
 int mfb_mean_action(const int32_t *d_actions /* [rows][cap] */, const int32_t *d_num /* [rows] */,
                     float *d_out /* [rows][n_action] */, int rows, int cap, int n_action, void *stream);
 
+/* K7: neighbourhood mean action per agent, the local form of the mean action of mean-field MARL:
+ * a_bar_i = 1/N_i sum_{j in N(i)} onehot(a_j).  For every listed slot i < num[e][g] (a dead agent still listed
+ * before clear_dead included), N(i) = the agents j != i of the SAME group, j < num[e][g], that are alive, have acted
+ * (last_action < n_action; it is n_action after a placement or an auto-reset) and stand at an offset
+ * pos_j - pos_i inside the disc CircleRange(radius, 0, 1) of Range.h:171-215 (radius cast to float, distances in
+ * double, no wrap-around).  out[b] = (float)count_b / (float)|N(i)| rounded to nearest; a row with |N(i)| = 0 is all
+ * zeros (the zero initial mean action of senario_battle.py:93), and so are rows >= num.  Called after
+ * mfb_step(..., clear_dead = 1) its rows line up with the next observation's rows.
+ *   radius    0 < radius <= view_radius (6 for battle); anything else, NaN included, is an error and launches nothing
+ *   d_outG    float[E][cap][n_action] per group, 16-byte aligned -- the row layout of mfb_observe_groups; NULL skips
+ *             that group
+ * Reads the engine state only (no RNG, no state change); a pending placement is committed first. */
+int mfb_local_mean_action(mfb_engine *eng, double radius, float *d_out0, float *d_out1, void *stream);
+
 /* state read-back into HOST buffers (synchronises `stream`): key in
  *   "num" int32[E][2], "dead_ct" int32[E][2], "pos" int32[E][2][cap][2], "hp" float[E][2][cap],
  *   "id" int32[E][2][cap], "alive" uint8[E][2][cap], "last_action" int32[E][2][cap],

@@ -178,6 +178,13 @@ int mfb_mean_action(const int32_t *d_actions, const int32_t *d_num, float *d_out
     MFB_END("mfb_mean_action")
 }
 
+int mfb_local_mean_action(mfb_engine *h, double radius, float *d_out0, float *d_out1, void *stream) {
+    MFB_BEGIN
+    float *out[kGroups] = {d_out0, d_out1};
+    E(h).local_mean_action(radius, out, (cudaStream_t)stream);
+    MFB_END("mfb_local_mean_action")
+}
+
 int mfb_get(mfb_engine *h, const char *key, void *host_buf, void *stream) {
     MFB_BEGIN
     Engine &e = E(h);

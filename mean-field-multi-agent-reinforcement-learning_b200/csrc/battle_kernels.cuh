@@ -5,6 +5,7 @@
 //                 (GridWorld.cc:430-496, 498-694, 696-728, 744-770; Map.cc:220-369;
 //                  RewardEngine.cc:216-240,373-443; senario_battle.py:141)
 //   k_mean_action (K5) standalone group mean action (senario_battle.py:141,255)
+//   k_local_mean_action (K7) per-agent neighbourhood mean action over a view-range disc (read-only)
 //   k_place       episode (re)initialisation from a placement template (GridWorld.cc:76-124,256-269)
 //
 // All arithmetic that reaches an output is ordered IEEE fp32 (compiled with -fmad=false, explicit
@@ -1062,6 +1063,89 @@ __global__ void k_mean_action(const int32_t *__restrict__ actions, const int32_t
         }
     }
     if (lane < n_action) out[(size_t)row * n_action + lane] = n > 0 ? __fdiv_rn((float)cnt, (float)n) : 0.0f;
+}
+
+// ----------------------------------------------------------------------------------------------
+// K7: neighbourhood mean action.  Observer i of (env e, group g) gets
+//   out[b] = #{j != i same group : alive_j, last_action_j = b < n_action, pos_j - pos_i in the disc} / (that count)
+// (0 when nobody counts), the disc being CircleRange(radius, 0, 1) (Range.h:171-215) with radius <= view_radius, so it
+// fits the kPad margin.  Rows >= num are zero.  Reads the engine state only.
+//
+// One CTA per (env, tile of observers, group).  The CTA builds a padded u8 grid of its group in shared memory (a cell
+// holds last_action + 1 of the alive agent that stands there and has acted, else 0); each thread then walks the disc
+// of one observer (no bounds tests), 8 probes in flight at a time, and counts the hits into its own column of a
+// [bin][thread] histogram (lanes never share a bank) with shared atomics whose result nobody waits for.  The centre is
+// skipped: a live observer stands there itself, while a listed dead one may have been stepped on, and then the agent
+// on its cell counts.  The histogram region is then reused for the rows, staged [thread][bin], and stored as one
+// contiguous block: cap and the tile are multiples of 4, so every tile is a whole number of 16-byte vectors.
+// ----------------------------------------------------------------------------------------------
+constexpr int kLocalBins = 32;   // n_action <= 32 (Engine checks move + attack <= 32)
+struct LocalMeanSmem { int grid, hist, total; };
+__host__ __device__ inline LocalMeanSmem local_mean_smem_layout(int W, int H, int tile, int n_action) {
+    LocalMeanSmem L; int o = 0;
+    L.grid = o;  o += ((W + 2 * kPad) * (H + 2 * kPad) + 15) & ~15;
+    L.hist = o;  o += 4 * n_action * tile;   // u32 [bin][thread], then f32 [thread][bin] rows
+    L.total = o;
+    return L;
+}
+
+__global__ void __launch_bounds__(kLocalMaxTile) k_local_mean_action(const __grid_constant__ LocalMeanIO io, const BattleState S) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const LocalMeanSmem L = local_mean_smem_layout(io.W, io.H, io.tile, io.n_action);
+    uint8_t *s_grid = smem_raw + L.grid;
+    uint32_t *s_hist = (uint32_t *)(smem_raw + L.hist);
+    float *s_stage = (float *)(smem_raw + L.hist);
+    const int tid = threadIdx.x, nt = blockDim.x;
+    const int e = blockIdx.x, first = blockIdx.y * nt, g = io.group[blockIdx.z];
+    const int cap = io.cap, n_action = io.n_action, PW = io.W + 2 * kPad;
+    const size_t base = ((size_t)e * kGroups + g) * cap;
+    const int n = S.num[e * kGroups + g];
+
+    for (int c = tid; c < (L.hist - L.grid) / 16; c += nt) ((uint4 *)s_grid)[c] = make_uint4(0u, 0u, 0u, 0u);
+    for (int b = 0; b < n_action; b++) s_hist[b * nt + tid] = 0u;
+    __syncthreads();
+    for (int s = tid; s < n; s += nt) {
+        const uint32_t st = S.state[base + s], a = st_act(st);
+        if (!st_dead(st) && a < (uint32_t)n_action) {
+            const int p = S.pos[base + s];
+            s_grid[(pos_y(p) + kPad) * PW + pos_x(p) + kPad] = (uint8_t)(a + 1);
+        }
+    }
+    __syncthreads();
+
+    const int i = first + tid;
+    uint32_t *h = s_hist + tid;                           // h[b * nt] = bin b of this thread
+    if (i < n) {
+        const int p = S.pos[base + i];
+        const uint8_t *c = s_grid + (pos_y(p) + kPad) * PW + pos_x(p) + kPad;
+        for (int k = 0; k < io.n_offsets; k += 8) {
+            uint32_t v[8];
+#pragma unroll
+            for (int u = 0; u < 8; u++) v[u] = k + u < io.n_offsets ? c[io.delta[k + u]] : 0u;
+#pragma unroll
+            for (int u = 0; u < 8; u++)
+                if (v[u]) atomicAdd(h + (v[u] - 1) * nt, 1u);
+        }
+        if (st_dead(S.state[base + i])) {
+            const uint32_t v = c[0];
+            if (v) atomicAdd(h + (v - 1) * nt, 1u);
+        }
+    }
+    uint32_t cnt[kLocalBins], total = 0;
+#pragma unroll
+    for (int b = 0; b < kLocalBins; b++) {
+        cnt[b] = b < n_action ? h[b * nt] : 0u;
+        total += cnt[b];
+    }
+    __syncthreads();                                      // every column is read: the region now takes the rows
+    float *row = s_stage + tid * n_action;                // (rows of threads past num are zeros: their counts are)
+#pragma unroll
+    for (int b = 0; b < kLocalBins; b++)
+        if (b < n_action) row[b] = cnt[b] ? __fdiv_rn((float)cnt[b], (float)total) : 0.0f;
+    __syncthreads();
+    const int rows = min(nt, cap - first);
+    float4 *dst = (float4 *)(io.out[g] + ((size_t)e * cap + first) * n_action);
+    for (int v = tid; v < rows * n_action / 4; v += nt) dst[v] = ((const float4 *)s_stage)[v];
 }
 
 // ----------------------------------------------------------------------------------------------

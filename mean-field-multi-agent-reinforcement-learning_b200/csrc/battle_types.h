@@ -124,4 +124,16 @@ struct ObsIO {
     int debug;       // only read by -DMF_PROFILE_BUILD binaries (profiling experiments): 1 = skip row composition
 };
 
+// K7 (k_local_mean_action): neighbourhood mean action.  Passed by value as a __grid_constant__ parameter; the disc
+// part (n_offsets, delta) is built on the host once per radius (Engine::local_mean_action).
+constexpr int kLocalMaxTile = 128;   // observers per CTA (= threads)
+struct LocalMeanIO {
+    float *out[kGroups];       // per group [E][cap][n_action]
+    int group[kGroups];        // blockIdx.z -> group (only the groups asked for are launched)
+    int W, H, cap, n_action;
+    int tile;                  // observers per CTA = blockDim.x, a multiple of 32
+    int n_offsets;             // cells of the disc other than the centre
+    int16_t delta[kViewCells]; // their offsets in the padded u8 grid (row pitch W + 2 * kPad)
+};
+
 }  // namespace mfmarl

@@ -594,4 +594,45 @@ void Engine::mean_action(const int32_t *d_actions, const int32_t *d_num, float *
     MF_CUDA(cudaGetLastError());
 }
 
+void Engine::local_mean_action(double radius, float *const out[kGroups], cudaStream_t st) {
+    const double view_radius = cfg_.type.view_radius;
+    if (!(radius > 0.0 && radius <= view_radius)) {   // also NaN
+        char msg[160];
+        snprintf(msg, sizeof(msg), "local_mean_action: radius %g outside (0, view_radius = %g]", radius, view_radius);
+        throw Fatal(msg);
+    }
+    int group_mask = 0;
+    for (int g = 0; g < kGroups; g++) {
+        if (!out[g]) continue;
+        if ((uintptr_t)out[g] & 15) throw Fatal("local_mean_action: output buffer must be 16-byte aligned");
+        group_mask |= 1 << g;
+    }
+    commit(st);
+    if (!group_mask) return;
+    const float r = (float)radius;                     // the engine's ranges are built from float radii
+    auto it = local_discs_.find(r);
+    if (it == local_discs_.end()) {
+        const CircleRange disc(r, 0.0f, 1);
+        if (disc.center > kPad) throw Fatal("local_mean_action: disc wider than the grid margin");
+        LocalMeanIO t{};
+        const int PW = P_.W + 2 * kPad;
+        for (int k = 0; k < disc.count; k++)
+            if (disc.dx[k] != 0 || disc.dy[k] != 0) t.delta[t.n_offsets++] = (int16_t)(disc.dy[k] * PW + disc.dx[k]);
+        it = local_discs_.emplace(r, t).first;
+    }
+    LocalMeanIO io = it->second;
+    io.W = P_.W; io.H = P_.H; io.cap = P_.cap; io.n_action = n_action();
+    io.tile = std::min(kLocalMaxTile, round_up(P_.cap, 32));
+    int ng = 0;
+    for (int g = 0; g < kGroups; g++) {
+        io.out[g] = out[g];
+        if ((group_mask >> g) & 1) io.group[ng++] = g;
+    }
+    const LocalMeanSmem L = local_mean_smem_layout(P_.W, P_.H, io.tile, io.n_action);
+    raise_dynamic_smem((const void *)k_local_mean_action, L.total, device_);
+    const dim3 grid((unsigned)P_.E, (unsigned)((P_.cap + io.tile - 1) / io.tile), (unsigned)ng);
+    k_local_mean_action<<<grid, io.tile, L.total, st>>>(io, S_);
+    MF_CUDA(cudaGetLastError());
+}
+
 }  // namespace mfmarl

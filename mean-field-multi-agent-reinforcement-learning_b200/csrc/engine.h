@@ -5,6 +5,7 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <map>
 #include <memory>
 #include <stdexcept>
 #include <string>
@@ -80,6 +81,9 @@ public:
     void step(const StepIO &io, cudaStream_t st);
     static void mean_action(const int32_t *d_actions, const int32_t *d_num, float *d_out, int rows,
                             int cap, int n_action, cudaStream_t st);
+    // K7: neighbourhood mean action of every listed agent (mfmarl_batched.h mfb_local_mean_action); out[g] is a
+    // 16-byte aligned float [E][cap][n_action] block or null (group skipped).  0 < radius <= view_radius.
+    void local_mean_action(double radius, float *const out[kGroups], cudaStream_t st);
 
     // E == 1: overwrite the agent records with a host copy (mapped pinned memory; runtime_api.cu rolls back a speculative
     // clear_dead with it).  Asynchronous on `st`.
@@ -135,6 +139,7 @@ private:
     int obs_ctas_per_sm_[2] = {2, 2};      // resident k_obs CTAs per SM at that size (occupancy query)
     int obs_grid_limit_ = 0;               // MFMARL_OBS_GRID: cap on k_obs CTAs (leaves SM slots to a concurrent k_step)
     int obs_debug_ = 0;                    // MFMARL_OBS_DEBUG at construction (profiling experiments only)
+    std::map<float, LocalMeanIO> local_discs_;   // K7 disc tables by radius (n_offsets, delta filled)
 
     // host-side placement template (what add_agents has built since the last reset)
     std::vector<unsigned char> h_walls_;          // [H*W]

@@ -64,7 +64,9 @@ class _Staging:
         self.key.index_copy_(0, dest, (env * id_span + ids[:n_rec].to(torch.int64)).reshape(-1))
         self.t.index_copy_(0, dest, torch.full((n_rec * cap,), self.step, dtype=torch.int64, device=dev))
         if self.use_mean:
-            self.prob.index_copy_(0, dest, prob[:n_rec, None, :].expand(n_rec, cap, prob.shape[-1]).reshape(n_rec * cap, -1))
+            # [E, act_n]: one mean action per env (the group mean); [E, cap, act_n]: one per agent (the local mean)
+            rows = prob[:n_rec] if prob.dim() == 3 else prob[:n_rec, None, :].expand(n_rec, cap, prob.shape[-1])
+            self.prob.index_copy_(0, dest, rows.reshape(n_rec * cap, -1))
         self.cursor += cnt.sum()
         self.upper += n_rec * cap
         self.step += 1
@@ -124,7 +126,8 @@ class DeviceMemoryGroup:
 
     def push(self, **kwargs):
         """state=(view [E, cap, 13, 13, 7], feature [E, cap, 34]), acts / rewards / alives / ids [E, cap],
-        prob [E, act_n] (the mean action every agent of the env saw), num [E], active [E] bool or None."""
+        prob [E, act_n] (the mean action every agent of the env saw) or [E, cap, act_n] (each agent's own), num [E],
+        active [E] bool or None."""
         view, feat = kwargs['state']
         if self._stage is None:
             self._stage = _Staging(self.stage_rows, self.obs_shape, self.feat_shape, self.act_n, self.use_mean,

@@ -48,6 +48,7 @@ class BatchedGridWorld:
         with torch.cuda.device(self.device):
             check(self.lib.mfb_create(ctypes.byref(cfg), ctypes.byref(self._h)))
         self.n_envs, self.map_size, self.rng = n_envs, map_size, rng
+        self.view_radius = float(cfg.view_radius)
         self._bufs = {}
         self._sizes = None
 
@@ -154,6 +155,27 @@ class BatchedGridWorld:
         with torch.cuda.device(self.device):
             fn = self.lib.mfb_observe_groups_bf16 if bf16 else self.lib.mfb_observe_groups
             check(fn(self._h, *ptrs, _stream()))
+        return out
+
+    def local_mean_action(self, groups=(0, 1), radius=None):
+        """Neighbourhood mean action of every listed agent (mfb_local_mean_action, kernel K7): per group a float32
+        [E, cap, n_action] tensor (None for a group not asked for).  Row i is the one-hot mean of the last actions of
+        agent i's living group-mates that have acted and stand inside the disc of `radius` around it (None = the
+        view radius, the largest allowed), or zeros when there are none; rows >= num are zero.  Called after step(),
+        its rows line up with the next observe_groups() rows.  The buffers belong to the engine and are reused by the
+        next call; nothing in the engine state changes."""
+        s = self.sizes
+        E, cap, n_action = self.n_envs, s["capacity"], s["n_action"]
+        radius = self.view_radius if radius is None else float(radius)
+        out, ptrs = [], []
+        for g in (0, 1):
+            if g in groups:
+                t = self._buf("local_mean_g%d" % g, (E, cap, n_action), torch.float32)
+                out.append(t); ptrs.append(_ptr(t))
+            else:
+                out.append(None); ptrs.append(None)
+        with torch.cuda.device(self.device):
+            check(self.lib.mfb_local_mean_action(self._h, radius, *ptrs, _stream()))
         return out
 
     def device_state(self, key):

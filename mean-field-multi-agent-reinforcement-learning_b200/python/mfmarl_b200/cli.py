@@ -28,7 +28,17 @@ def battle_parser(description, training):
         ap.add_argument("--rollout_bf16", action="store_true",
                         help="with --envs: the policies act on bf16 observation rows emitted by the engine (bf16 twins of "
                              "the networks; training stays fp32 on the fp32 rows)")
+        ap.add_argument("--mean_field", choices=("group", "local"), default="group",
+                        help="mean action of the mean-field learners: 'group' = over the whole group (the reference's), "
+                             "'local' = over each agent's group-mates within its view radius (needs --envs)")
     return ap
+
+
+def check_battle_args(ap, args):
+    """combinations argparse cannot express; exits with a usage error like argparse itself"""
+    if getattr(args, "mean_field", "group") == "local" and args.envs <= 0:
+        ap.error("--mean_field local needs the batched engine: pass --envs N (N > 0)")
+    return args
 
 
 def data_dirs(args, base_dir):

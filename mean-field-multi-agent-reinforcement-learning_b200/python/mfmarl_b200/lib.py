@@ -52,6 +52,7 @@ def load_library(path=None):
         "mfb_step": [vp, vp, vp, vp, vp, vp, vp, ci, vp],
         "mfb_clear_dead": [vp, vp],
         "mfb_mean_action": [vp, vp, vp, ci, ci, ci, vp],
+        "mfb_local_mean_action": [vp, ctypes.c_double, vp, vp, vp],
         "mfb_get": [vp, cp, vp, vp],
         "mfb_num_device_ptr": [vp, ctypes.POINTER(vp)],
         "mfb_step_host": [vp, vp, vp, vp, vp, vp, vp],

@@ -101,7 +101,7 @@ def battle(env, n_round, map_size, max_steps, handles, models, print_every, eps=
 # batched, device-resident form
 # ----------------------------------------------------------------------------------------------------------
 def play_batched(env, n_round, max_steps, models, eps=1.0, train=False, print_every=0, left_group=None,
-                 positions=None, obs_dtype=None, host_lag=None):
+                 positions=None, obs_dtype=None, host_lag=None, mean_field="group", mf_radius=None):
     """E episodes in lockstep on a `BatchedGridWorld` (one per environment), everything on the device.
 
     Per environment this is the loop of `play`: observe both groups -> models[g].act on the group's rows (with the
@@ -117,9 +117,17 @@ def play_batched(env, n_round, max_steps, models, eps=1.0, train=False, print_ev
     host_lag: how many steps the host may run ahead of the device before it looks at the "any environment still
     playing" flag (see below); None = 2 on a CUDA device, 0 = ask after every step.
 
+    mean_field: which mean action the policies see.  "group" (the reference's, senario_battle.py:141): every agent of
+    a group gets the one-hot mean of the whole group's previous actions.  "local": agent j gets the mean over its
+    group-mates inside the disc of radius `mf_radius` (None = the view radius) that acted last step
+    (`BatchedGridWorld.local_mean_action`), zeros before the first step; the replay then stores each agent's own row.
+
     Returns (max_nums [E, 2], nums [E, 2], mean_rewards [E, 2], total_rewards [E, 2]) as numpy arrays.
     """
     import torch
+    if mean_field not in ("group", "local"):
+        raise ValueError("mean_field must be 'group' or 'local', not %r" % (mean_field,))
+    local = mean_field == "local"
     E, cap = env.n_envs, env.capacity
     dev = env.device
     if positions is None:
@@ -130,6 +138,8 @@ def play_batched(env, n_round, max_steps, models, eps=1.0, train=False, print_ev
     env.add_agents(left_group, positions[0])
     env.add_agents(1 - left_group, positions[1])
     n_action = env.sizes["n_action"]
+    if local:
+        local_mean = env.local_mean_action(radius=mf_radius)    # nobody has acted yet: all rows zero
     live_num, live_id = env.device_state("num"), env.device_state("id")    # aliases of the engine's HBM state
     num = live_num.clone()                                                 # [E, 2] agents at observation time
     max_nums, final_nums = num.clone(), num.clone()
@@ -170,15 +180,22 @@ def play_batched(env, n_round, max_steps, models, eps=1.0, train=False, print_ev
         valid = (slot[None, None, :] < num[:, :, None]) & active[:, None, None]          # [E, 2, cap]
         for g in range(2):
             view, feat = act_obs[g]
-            prob = former[:, g, None, :].expand(E, cap, n_action).reshape(E * cap, n_action)
+            if local:
+                prob = local_mean[g].view(E * cap, n_action)
+            else:
+                prob = former[:, g, None, :].expand(E, cap, n_action).reshape(E * cap, n_action)
             a = models[g].act(state=[view.view((E * cap,) + tuple(view.shape[2:])), feat.view(E * cap, -1)],
                               prob=prob, eps=eps)
             actions[:, g] = a.reshape(E, cap)
         actions.masked_fill_(~valid, 0)
-        reward, alive, done, mean = env.step(actions)
+        reward, alive, done, mean = env.step(actions, want_mean_action=not local)
         if train:
             models[0].flush_buffer_batched(state=obs[0], acts=actions[:, 0], rewards=reward[:, 0], alives=alive[:, 0],
-                                           ids=ids[:, 0], prob=former[:, 0], num=num[:, 0], active=active)
+                                           ids=ids[:, 0], prob=local_mean[0] if local else former[:, 0], num=num[:, 0],
+                                           active=active)
+        if local:
+            # the next step's rows; enqueued after the flush above has read this step's on the same stream
+            local_mean = env.local_mean_action(radius=mf_radius)
         # statistics (senario_battle.py:146-152): nums still include the agents that died this step
         r = torch.where(valid, reward, torch.zeros_like(reward)).to(torch.float64).sum(dim=2)   # [E, 2]
         act_f = active[:, None].to(torch.float64)
@@ -188,7 +205,8 @@ def play_batched(env, n_round, max_steps, models, eps=1.0, train=False, print_ev
         # the reference reads get_num BEFORE the step's clear_dead (senario_battle.py:146): the agents that died in an
         # environment's last step still count, which is what Runner's `kill` statistic is built on
         final_nums = torch.where(active[:, None], num, final_nums)
-        former = torch.where(active[:, None, None], mean, former)
+        if not local:
+            former = torch.where(active[:, None, None], mean, former)
         active = active & (done == 0)
         if lag:
             flags[step_ct % lag].copy_(active.any().reshape(1), non_blocking=True)

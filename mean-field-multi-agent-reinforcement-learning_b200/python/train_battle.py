@@ -4,6 +4,8 @@ engine and the PyTorch learners.
     python train_battle.py --algo mfq                   one environment through the magent binding (reference loop)
     python train_battle.py --algo mfq --envs 1024       1024 lock-stepped environments on the GPU per round:
                                                          observations, mean actions and replay stay in HBM
+    python train_battle.py --algo mfq --envs 1024 --mean_field local
+                                                        the same with each agent's neighbourhood mean action
 """
 import os
 import sys
@@ -30,8 +32,8 @@ class BatchedEnvAdapter:
     """What Runner / spawn_ai ask of `env` (space queries) on top of a BatchedGridWorld, plus a `play` handle that
     reduces the per-environment statistics of play_batched to the scalars Runner logs (means over environments)."""
 
-    def __init__(self, benv, rollout_bf16=False):
-        self.benv, self.rollout_bf16 = benv, rollout_bf16
+    def __init__(self, benv, rollout_bf16=False, mean_field="group"):
+        self.benv, self.rollout_bf16, self.mean_field = benv, rollout_bf16, mean_field
 
     def get_view_space(self, handle):
         s = self.benv.sizes
@@ -51,7 +53,8 @@ class BatchedEnvAdapter:
         # every rank places the armies the same way round (the draw of senario_battle.py:14 comes from the round number)
         max_nums, nums, mean_r, total_r = play_batched(self.benv, n_round, max_steps, models, eps=eps, train=train,
                                                        print_every=print_every, left_group=n_round % 2,
-                                                       obs_dtype=torch.bfloat16 if self.rollout_bf16 else None)
+                                                       obs_dtype=torch.bfloat16 if self.rollout_bf16 else None,
+                                                       mean_field=self.mean_field)
         stats = np.stack([max_nums.mean(axis=0), nums.mean(axis=0), mean_r.mean(axis=0), total_r.mean(axis=0)])
         stats = all_ranks_mean(stats, self.benv.device)     # one decision (self-play update, win count) on every rank
         return tuple(list(row) for row in stats)
@@ -86,8 +89,9 @@ def init_distributed(device_arg):
 
 
 def main(argv=None):
-    from mfmarl_b200.cli import battle_parser, data_dirs
-    args = battle_parser("self-play training on the battle scenario", training=True).parse_args(argv)
+    from mfmarl_b200.cli import battle_parser, check_battle_args, data_dirs
+    ap = battle_parser("self-play training on the battle scenario", training=True)
+    args = check_battle_args(ap, ap.parse_args(argv))
     args.data_dir, render_dir = data_dirs(args, BASE_DIR)
 
     from mfmarl_b200.algo import spawn_ai, tools
@@ -103,7 +107,7 @@ def main(argv=None):
         cap = max(64, int(args.map_size * args.map_size * 0.04))
         benv = BatchedGridWorld(args.envs, map_size=args.map_size, capacity=cap, device=args.device, rng="philox",
                                 env_base=rank * args.envs)
-        env = BatchedEnvAdapter(benv, rollout_bf16=args.rollout_bf16)
+        env = BatchedEnvAdapter(benv, rollout_bf16=args.rollout_bf16, mean_field=args.mean_field)
         handles, play = [0, 1], env.play
     else:
         import magent
