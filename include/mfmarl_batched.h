@@ -147,6 +147,17 @@ int mfb_step_host_async(mfb_engine *eng, const int32_t *h_actions, float *h_rewa
                         float *h_mean_action, int32_t *h_done, void *stream, int *ticket);
 int mfb_host_wait(mfb_engine *eng, int ticket);
 
+/* Device memory for large, mostly-zero output blocks such as the observation rows.  Where the GPU supports generic
+ * compression (CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED) the block is a cuMemCreate allocation with
+ * CU_MEM_ALLOCATION_COMP_GENERIC: the L2 compresses its lines on the way to DRAM, losslessly and invisibly to loads and
+ * stores, so sparse rows cost fewer HBM bytes to write.  Elsewhere, or when the driver grants no compression, it is a
+ * plain cudaMalloc, and so is a block the driver has no compressible memory left for.  *compressed tells which
+ * (1 / 0).  The block is zeroed, and the call synchronises the device.  mfb_free_device synchronises the whole device
+ * before it releases a block, so it must not run while a stream is capturing a CUDA graph; it accepts NULL and nothing
+ * else that mfb_alloc_device did not return. */
+int mfb_alloc_device(unsigned long bytes, int device, void **ptr, int *compressed);
+int mfb_free_device(void *ptr);
+
 const char *mfb_last_error(void);
 
 /* ---- K6: Ising tabular mean-field Q-learning, one fused sweep over a batch of lattices -----------------

@@ -1,6 +1,10 @@
 // mfb_*: batched, device-resident C ABI (include/mfmarl_batched.h).
+#include <cudaTypedefs.h>
+
 #include <cstring>
+#include <map>
 #include <memory>
+#include <mutex>
 #include <vector>
 
 #include "../../include/mfmarl_batched.h"
@@ -47,6 +51,100 @@ int fail(const char *where, const std::exception &ex) {
 Engine &E(mfb_engine *h) {
     if (!h || !h->eng) throw Fatal("null engine handle");
     return *h->eng;
+}
+
+// Compressible device memory (mfb_alloc_device).  The driver's virtual-memory calls are looked up through the runtime,
+// so libmagent.so needs no libcuda at link or load time (the CPU-only tests load it on machines without a driver).
+struct DriverVmm {
+    PFN_cuDeviceGet get_device = nullptr;
+    PFN_cuDeviceGetAttribute get_attribute = nullptr;
+    PFN_cuMemGetAllocationGranularity granularity = nullptr;
+    PFN_cuMemAddressReserve reserve = nullptr;
+    PFN_cuMemAddressFree address_free = nullptr;
+    PFN_cuMemCreate create = nullptr;
+    PFN_cuMemGetAllocationPropertiesFromHandle properties = nullptr;
+    PFN_cuMemRelease release = nullptr;
+    PFN_cuMemMap map = nullptr;
+    PFN_cuMemUnmap unmap = nullptr;
+    PFN_cuMemSetAccess set_access = nullptr;
+};
+
+const DriverVmm &driver_vmm() {
+    static const DriverVmm d = [] {
+        DriverVmm v;
+        auto get = [](const char *sym, void **fn) {
+            cudaDriverEntryPointQueryResult q;
+            MF_CUDA(cudaGetDriverEntryPointByVersion(sym, fn, 12000, cudaEnableDefault, &q));
+            if (q != cudaDriverEntryPointSuccess || !*fn) throw Fatal(std::string("driver entry point missing: ") + sym);
+        };
+        get("cuDeviceGet", (void **)&v.get_device);
+        get("cuDeviceGetAttribute", (void **)&v.get_attribute);
+        get("cuMemGetAllocationGranularity", (void **)&v.granularity);
+        get("cuMemAddressReserve", (void **)&v.reserve);
+        get("cuMemAddressFree", (void **)&v.address_free);
+        get("cuMemCreate", (void **)&v.create);
+        get("cuMemGetAllocationPropertiesFromHandle", (void **)&v.properties);
+        get("cuMemRelease", (void **)&v.release);
+        get("cuMemMap", (void **)&v.map);
+        get("cuMemUnmap", (void **)&v.unmap);
+        get("cuMemSetAccess", (void **)&v.set_access);
+        return v;
+    }();
+    return d;
+}
+
+void cu_check(CUresult r, const char *what) {
+    if (r != CUDA_SUCCESS) throw Fatal(std::string(what) + " failed: CUresult " + std::to_string((int)r));
+}
+
+struct DeviceBlock { size_t size; CUmemGenericAllocationHandle handle; };   // size 0: a cudaMalloc fallback
+std::mutex g_blocks_mu;
+std::map<void *, DeviceBlock> g_blocks;
+
+// The caller's current device is restored when the allocator returns.
+struct DeviceGuard {
+    int prev = -1;
+    explicit DeviceGuard(int dev) { MF_CUDA(cudaGetDevice(&prev)); MF_CUDA(cudaSetDevice(dev)); }
+    ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
+};
+
+// Reserve + create + map + access, all or nothing.  Returns nullptr (and keeps nothing) when the driver hands back an
+// allocation without generic compression, or has no compressible memory left for it (the caller then falls back to
+// cudaMalloc, which reports a real out-of-memory itself).
+void *map_compressible(const DriverVmm &d, size_t bytes, int device, size_t *mapped, CUmemGenericAllocationHandle *h) {
+    CUmemAllocationProp prop = {};
+    prop.type = CU_MEM_ALLOCATION_TYPE_PINNED;
+    prop.location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+    prop.location.id = device;
+    prop.allocFlags.compressionType = CU_MEM_ALLOCATION_COMP_GENERIC;
+    size_t gran = 0;
+    cu_check(d.granularity(&gran, &prop, CU_MEM_ALLOC_GRANULARITY_MINIMUM), "cuMemGetAllocationGranularity");
+    const size_t size = (bytes + gran - 1) / gran * gran;
+    CUdeviceptr va = 0;
+    cu_check(d.reserve(&va, size, gran, 0, 0), "cuMemAddressReserve");
+    CUresult r = d.create(h, size, &prop, 0);
+    if (r != CUDA_SUCCESS) {
+        d.address_free(va, size);
+        if (r == CUDA_ERROR_OUT_OF_MEMORY) return nullptr;
+        cu_check(r, "cuMemCreate");
+    }
+    CUmemAllocationProp got = {};
+    r = d.properties(&got, *h);
+    if (r == CUDA_SUCCESS && got.allocFlags.compressionType != CU_MEM_ALLOCATION_COMP_GENERIC) {
+        d.release(*h); d.address_free(va, size);
+        return nullptr;
+    }
+    if (r == CUDA_SUCCESS) r = d.map(va, size, 0, *h, 0);
+    if (r == CUDA_SUCCESS) {
+        CUmemAccessDesc acc = {};
+        acc.location = prop.location;
+        acc.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+        r = d.set_access(va, size, &acc, 1);
+        if (r != CUDA_SUCCESS) d.unmap(va, size);
+    }
+    if (r != CUDA_SUCCESS) { d.release(*h); d.address_free(va, size); cu_check(r, "mapping compressible memory"); }
+    *mapped = size;
+    return (void *)va;
 }
 }  // namespace
 
@@ -333,6 +431,62 @@ int mfb_host_wait(mfb_engine *h, int ticket) {
     if (ticket < 0 || ticket > 1) throw Fatal("mfb_host_wait: bad ticket");
     if (h->slot[ticket].used) MF_CUDA(cudaEventSynchronize(h->slot[ticket].out_done));
     MFB_END("mfb_host_wait")
+}
+
+int mfb_alloc_device(unsigned long bytes, int device, void **ptr, int *compressed) {
+    MFB_BEGIN
+    if (!ptr || !compressed) throw Fatal("mfb_alloc_device: null output pointer");
+    if (bytes == 0) throw Fatal("mfb_alloc_device: zero bytes");
+    *ptr = nullptr; *compressed = 0;
+    DeviceGuard guard(device);
+    MF_CUDA(cudaFree(nullptr));                           // the device's primary context is current for the driver calls
+    const DriverVmm &d = driver_vmm();
+    CUdevice cu_dev;
+    int supported = 0;
+    cu_check(d.get_device(&cu_dev, device), "cuDeviceGet");
+    cu_check(d.get_attribute(&supported, CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, cu_dev), "cuDeviceGetAttribute");
+    DeviceBlock blk{0, 0};
+    void *p = supported ? map_compressible(d, bytes, device, &blk.size, &blk.handle) : nullptr;
+    if (!p) { MF_CUDA(cudaMalloc(&p, bytes)); blk.size = 0; }
+    // zeroed, as torch.zeros hands out a fresh buffer; synchronised because the caller's streams may not order
+    // themselves after the legacy default stream
+    cudaError_t err = cudaMemset(p, 0, bytes);
+    if (err == cudaSuccess) err = cudaDeviceSynchronize();
+    if (err != cudaSuccess) {
+        if (blk.size) { d.unmap((CUdeviceptr)p, blk.size); d.release(blk.handle); d.address_free((CUdeviceptr)p, blk.size); }
+        else cudaFree(p);
+        MF_CUDA(err);
+    }
+    {
+        std::lock_guard<std::mutex> lock(g_blocks_mu);
+        g_blocks[p] = blk;
+    }
+    *ptr = p;
+    *compressed = blk.size != 0;
+    MFB_END("mfb_alloc_device")
+}
+
+int mfb_free_device(void *ptr) {
+    MFB_BEGIN
+    if (!ptr) return 0;
+    DeviceBlock blk;
+    {
+        std::lock_guard<std::mutex> lock(g_blocks_mu);
+        auto it = g_blocks.find(ptr);
+        if (it == g_blocks.end()) throw Fatal("mfb_free_device: pointer not from mfb_alloc_device");
+        blk = it->second;
+        g_blocks.erase(it);
+    }
+    MF_CUDA(cudaDeviceSynchronize());                     // no queued kernel may still write the block
+    if (blk.size == 0) {
+        MF_CUDA(cudaFree(ptr));
+    } else {
+        const DriverVmm &d = driver_vmm();
+        cu_check(d.unmap((CUdeviceptr)ptr, blk.size), "cuMemUnmap");
+        cu_check(d.release(blk.handle), "cuMemRelease");
+        cu_check(d.address_free((CUdeviceptr)ptr, blk.size), "cuMemAddressFree");
+    }
+    MFB_END("mfb_free_device")
 }
 
 const char *mfb_last_error(void) { return last_error(); }

@@ -23,6 +23,39 @@ def _stream():
     return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
+class _DeviceBlock:
+    """One zeroed block from mfb_alloc_device (compressible memory where the GPU offers it), exposed through
+    __cuda_array_interface__ and freed when the last tensor made from it is gone: torch.as_tensor keeps this owner
+    alive, so a view tensor stays valid after its engine is dropped.  bfloat16 has no array-interface type string, so
+    a bf16 block is described as int16 and viewed as bfloat16 by tensor().
+
+    Freeing synchronises the whole device (no queued kernel may still write the block), at the moment the last
+    reference goes.  So do not drop the last reference to an observation block while a CUDA graph is being captured
+    (the synchronise would invalidate the capture), and expect every stream to stall when it happens.  The engines
+    reuse their blocks across calls, so this happens only when an engine is dropped or an output shape changes."""
+
+    _TYPESTR = {torch.float32: "<f4", torch.bfloat16: "<i2"}
+
+    def __init__(self, lib, shape, dtype, device):
+        nbytes = int(np.prod(shape)) * torch.empty((), dtype=dtype).element_size()
+        ptr, compressed = ctypes.c_void_p(), ctypes.c_int()
+        check(lib.mfb_alloc_device(nbytes, device.index or 0, ctypes.byref(ptr), ctypes.byref(compressed)))
+        self._lib, self._ptr = lib, ptr.value
+        self.compressed = bool(compressed.value)
+        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": self._TYPESTR[dtype],
+                                         "data": (ptr.value, False), "version": 2}
+        self._dtype, self._device = dtype, device
+
+    def tensor(self):
+        t = torch.as_tensor(self, device=self._device)
+        return t.view(self._dtype) if t.dtype != self._dtype else t
+
+    def __del__(self):
+        if getattr(self, "_ptr", None):
+            self._lib.mfb_free_device(ctypes.c_void_p(self._ptr))
+            self._ptr = None
+
+
 class BatchedGridWorld:
     def __init__(self, n_envs, map_size=40, capacity=64, device=None, rng="minstd", seed=0, env_base=0,
                  max_steps=0, auto_reset=False, step_threads=0, obs_tile_agents=0, obs_record=None, random_sides=False, concurrent_step_envs=0, **type_overrides):
@@ -50,6 +83,7 @@ class BatchedGridWorld:
         self.n_envs, self.map_size, self.rng = n_envs, map_size, rng
         self.view_radius = float(cfg.view_radius)
         self._bufs = {}
+        self._obs_compressed = None
         self._sizes = None
 
     def __del__(self):
@@ -112,20 +146,39 @@ class BatchedGridWorld:
     def capacity(self):
         return self.sizes["capacity"]
 
-    def _buf(self, name, shape, dtype):
+    def _buf(self, name, shape, dtype, obs=False):
+        """Engine-owned output buffer, reused by the next call.  obs=True: an observation block, in compressible
+        device memory where the GPU offers it (k_obs's rows are mostly zeros, so the L2 writes far fewer bytes to
+        HBM for them); every other buffer is a torch allocation."""
         t = self._bufs.get(name)
         if t is None or tuple(t.shape) != tuple(shape):
-            t = self._bufs[name] = torch.zeros(shape, dtype=dtype, device=self.device)
+            # drop the engine's references first, so that an old block nobody else holds is freed before its
+            # successor is allocated
+            self._bufs.pop(name, None)
+            t = None
+            if obs:
+                blk = _DeviceBlock(self.lib, shape, dtype, self.device)
+                self._obs_compressed = blk.compressed
+                t = blk.tensor()
+            else:
+                t = torch.zeros(shape, dtype=dtype, device=self.device)
+            self._bufs[name] = t
         return t
+
+    @property
+    def obs_compressed(self):
+        """Whether the engine-owned observation blocks are in compressible memory (None before the first one)."""
+        return self._obs_compressed
 
     # ------------------------------------------------------------ the two launches
     def observe(self, group_mask=3, out=None):
-        """-> (view float32[E, 2, cap, 13, 13, 7], feature float32[E, 2, cap, 34]); rows >= num are stale."""
+        """-> (view float32[E, 2, cap, 13, 13, 7], feature float32[E, 2, cap, 34]); rows >= num are stale.  Without
+        `out` the blocks belong to the engine (see obs_compressed) and are rewritten by the next call."""
         s = self.sizes
         E, cap, v = self.n_envs, s["capacity"], s["view_size"]
         if out is None:
-            view = self._buf("view", (E, 2, cap, v, v, s["n_channel"]), torch.float32)
-            feat = self._buf("feat", (E, 2, cap, s["feature_size"]), torch.float32)
+            view = self._buf("view", (E, 2, cap, v, v, s["n_channel"]), torch.float32, obs=True)
+            feat = self._buf("feat", (E, 2, cap, s["feature_size"]), torch.float32, obs=True)
         else:
             view, feat = out
         with torch.cuda.device(self.device):
@@ -147,8 +200,9 @@ class BatchedGridWorld:
         out, ptrs = [], []
         for g in (0, 1):
             if g in groups:
-                view = self._buf("view%s_g%d" % ("16" if bf16 else "", g), (E, cap, v, v, 8 if bf16 else s["n_channel"]), dtype)
-                feat = self._buf("feat_g%d" % g, (E, cap, s["feature_size"]), torch.float32)
+                view = self._buf("view%s_g%d" % ("16" if bf16 else "", g), (E, cap, v, v, 8 if bf16 else s["n_channel"]), dtype,
+                                 obs=True)
+                feat = self._buf("feat_g%d" % g, (E, cap, s["feature_size"]), torch.float32, obs=True)
                 out.append((view, feat)); ptrs += [_ptr(view), _ptr(feat)]
             else:
                 out.append(None); ptrs += [None, None]

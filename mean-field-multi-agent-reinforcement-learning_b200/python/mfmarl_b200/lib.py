@@ -58,6 +58,8 @@ def load_library(path=None):
         "mfb_step_host": [vp, vp, vp, vp, vp, vp, vp],
         "mfb_step_host_async": [vp, vp, vp, vp, vp, vp, vp, ctypes.POINTER(ci)],
         "mfb_host_wait": [vp, ci],
+        "mfb_alloc_device": [ctypes.c_ulong, ci, ctypes.POINTER(vp), ctypes.POINTER(ci)],
+        "mfb_free_device": [vp],
     }
     for name, argtypes in sig.items():
         fn = getattr(lib, name)
