@@ -199,6 +199,47 @@ int mfi_run(int dtype, int n_lattices, int side, int n_sweeps, int8_t *d_spins, 
             const void *d_temperatures, double lr, const void *d_uniforms, const uint8_t *d_update_mask, unsigned seed,
             unsigned lattice_base, unsigned step0, int32_t *d_n_up, void *d_reward_sum, void *stream);
 
+/* Per-lattice temperature schedules: mfi_step / mfi_run with one schedule per lattice, e.g. one batch holding every
+ * (temperature, replica) point of an order-parameter-against-temperature curve.  Lattice b draws sweep k at
+ * d_temperatures[k][b]; everything else (Philox keys, act groups, outputs, fp32 / fp64, the bits) is as above, so
+ * lattice b of a batch equals that lattice run alone with lattice_base + b and its own schedule.
+ *   mfi_step_lattices  d_temperatures  T [n_lattices]            device (K6)
+ *   mfi_run_lattices   d_temperatures  T [n_sweeps][n_lattices]  device (K6s at the fp32 sides 64 / 128 / 256 / 512,
+ *                                                                the generic K6r elsewhere and in fp64)
+ * The fp32 overrides that select a kernel without per-lattice tables -- MFMARL_ISING_PERSIST=1 (K6p), an
+ * MFMARL_ISING_RPT other than 0 or 8, and MFMARL_ISING_PERSIST=0 at sides 64 / 128 / 256 (the specialised K6r) unless
+ * MFMARL_ISING_RPT=0 -- make mfi_run_lattices return -1 with a message naming the variable, and nothing is launched
+ * (MFMARL_ISING_RPT=0 selects the generic K6r, which has the tables). */
+int mfi_step_lattices(int dtype, int n_lattices, int side, int8_t *d_spins, void *d_q, const void *d_temperatures,
+                      double lr, const void *d_uniforms, const uint8_t *d_update_mask, unsigned seed,
+                      unsigned lattice_base, unsigned step, int32_t *d_n_up, void *d_reward_sum, void *d_mse,
+                      void *stream);
+int mfi_run_lattices(int dtype, int n_lattices, int side, int n_sweeps, int8_t *d_spins, void *d_q,
+                     const void *d_temperatures, double lr, const void *d_uniforms, const uint8_t *d_update_mask,
+                     unsigned seed, unsigned lattice_base, unsigned step0, int32_t *d_n_up, void *d_reward_sum,
+                     void *stream);
+
+/* ---- K8: checkerboard single-spin-flip Metropolis on the same lattice model (the MCMC reference of the Ising curve)
+ * H = -1/2 sum_bonds sigma_i sigma_j = -1/2 sum_i r_i (sigma = 2 spin - 1, r_i = the environment's reward; coupling 1/2,
+ * Tc = 1 / ln(1 + sqrt 2) ~ 1.1346, MF-Q's temperature axis; flipping site i changes H by h below).  One sweep: every site with (x + y) even, then every site with (x + y) odd.  Site
+ * i flips when h = sigma_i sum_nbr sigma_j <= 0, and for h in {2, 4} when its Philox word r satisfies r < thr_h with
+ *   thr_h = min(floor(exp(-h / T) * 2^32), 2^32 - 1)   computed on the HOST in double with the C library's exp
+ * (Python's math.exp is the same function), so a CPU restatement reproduces every decision.
+ * Philox4x32-10: key (seed, lattice_base + lattice); site (x, y) of colour c = (x + y) & 1 in sweep step0 + k uses
+ * output word ((x & 31) >> 1) & 3 of counter ((y * ceil(side / 32) + x / 32) * 4 + (x & 31) / 8, step0 + k, c, 2)
+ * (the 2 keeps the stream apart from MF-Q's, which has 0 or 1 there).
+ *   side            even, 2 <= side <= 512
+ *   d_spins         int8 [n_lattices][side][side]   in/out, values {0, 1}
+ *   h_temperatures  double [n_sweeps][n_lattices]   HOST memory: every T finite and > 0 (the thresholds are computed
+ *                   from it on the host and uploaded with the launch)
+ *   d_n_up          int32[n_sweeps][n_lattices]     out or NULL: up spins after each sweep
+ *   d_bond_sum      int32[n_sweeps][n_lattices]     out or NULL: sum over the 2N bonds of sigma_i sigma_j after each sweep
+ *                   (= sum_i r_i, MF-Q's reward_sum; energy per site = -bond_sum / N)
+ * Bad input (odd side or out of range, T <= 0, inf or NaN) returns -1 before anything is launched. */
+int mfi_metropolis(int n_lattices, int side, int n_sweeps, int8_t *d_spins, const double *h_temperatures,
+                   unsigned seed, unsigned lattice_base, unsigned step0, int32_t *d_n_up, int32_t *d_bond_sum,
+                   void *stream);
+
 /* The Ising ENVIRONMENT interface (examples/ising_model/multiagent/environment.py:49-92 `_step` / `_reset`,
  * multiagent/core.py:99-125 `IsingWorld.step`, Ising.py:101-118 reward / observation) for callers that bring their
  * own policy, e.g. the unmodified main_MFQ_Ising.py over python/examples/ising_model (same package layout as the

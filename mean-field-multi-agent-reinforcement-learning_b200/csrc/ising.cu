@@ -103,8 +103,9 @@ __device__ __forceinline__ int bit_at(const uint32_t *rows, int wpr, int r, int 
     return (rows[r * wpr + (x >> 5)] >> (x & 31)) & 1;
 }
 
-template <typename T>
-__global__ void __launch_bounds__(sizeof(T) == 8 ? 512 : 1024) k_ising(const IsingArgs<T> A) {
+// PL: per-lattice temperatures, lattice b draws at temps[b] instead of A.temperature (mfi_step_lattices)
+template <typename T, bool PL>
+__device__ __forceinline__ void ising_sweep(const IsingArgs<T> A, const T *temps) {
     extern __shared__ __align__(16) uint32_t s_bits[];
     const int L = A.L, N = L * L, wpr = (L + 31) >> 5;
     uint32_t *s_old = s_bits, *s_new = s_bits + L * wpr;
@@ -129,7 +130,7 @@ __global__ void __launch_bounds__(sizeof(T) == 8 ? 512 : 1024) k_ising(const Isi
     }
     __syncthreads();
 
-    const T tparam = temperature_param(A.temperature);
+    const T tparam = temperature_param(PL ? temps[b] : A.temperature);
     T keep_q[kIsingRB]; int keep_sa[kIsingRB];     // this band: selected Q value, s | a << 3
     T prev_q = (T)0; int prev_sa = 0;              // last row of the previous band
     T row0_q = (T)0; int row0_sa = 0;              // row 0, finalised last (needs row L-1)
@@ -237,7 +238,15 @@ __global__ void __launch_bounds__(sizeof(T) == 8 ? 512 : 1024) k_ising(const Isi
 }
 
 template <typename T>
-static void launch_ising(const IsingArgs<T> &A, cudaStream_t st) {
+__global__ void __launch_bounds__(sizeof(T) == 8 ? 512 : 1024) k_ising(const IsingArgs<T> A) { ising_sweep<T, false>(A, nullptr); }
+template <typename T>
+__global__ void __launch_bounds__(sizeof(T) == 8 ? 512 : 1024) k_ising_lattices(const IsingArgs<T> A, const T *temps) {
+    ising_sweep<T, true>(A, temps);
+}
+
+// temps: null = A.temperature for every lattice, else T [B] device (one temperature per lattice)
+template <typename T>
+static void launch_ising(const IsingArgs<T> &A, cudaStream_t st, const T *temps = nullptr) {
     const int L = A.L, wpr = (L + 31) >> 5;
     if (L < 3 || L > 1024) throw Fatal("ising: lattice side must be in [3, 1024]");
     if ((size_t)2 * L * wpr * sizeof(uint32_t) > 200 * 1024) throw Fatal("ising: lattice too large for the shared-memory bit planes");
@@ -245,9 +254,15 @@ static void launch_ising(const IsingArgs<T> &A, cudaStream_t st) {
     if (sizeof(T) == 8 && L > 512) throw Fatal("ising: fp64 mode supports lattice sides up to 512");
     const int threads = wpr * 32;
     const size_t smem = (size_t)2 * L * wpr * sizeof(uint32_t);
-    if (smem > 48 * 1024)
-        MF_CUDA(cudaFuncSetAttribute(k_ising<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_ising<T><<<A.B, threads, smem, st>>>(A);
+    if (temps) {
+        if (smem > 48 * 1024)
+            MF_CUDA(cudaFuncSetAttribute(k_ising_lattices<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_ising_lattices<T><<<A.B, threads, smem, st>>>(A, temps);
+    } else {
+        if (smem > 48 * 1024)
+            MF_CUDA(cudaFuncSetAttribute(k_ising<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_ising<T><<<A.B, threads, smem, st>>>(A);
+    }
     MF_CUDA(cudaGetLastError());
 }
 
@@ -314,8 +329,9 @@ __device__ __forceinline__ void ising_uniforms(T (&uu)[kIsingRB], uint32_t x, ui
 }
 
 // FAST: L % 32 == 0 and rows % 4 == 0 -- every thread owns 4 live sites and a row's x-wrap is a word wrap.
-template <typename T, bool FAST>
-__global__ void __launch_bounds__(1024, 1) k_ising_resident(const IsingRunArgs<T> A) {
+// PL: A.temperatures is [K][B] (lattice b draws sweep k at row k, column b) instead of [K].
+template <typename T, bool FAST, bool PL>
+__device__ __forceinline__ void ising_resident_sweeps(const IsingRunArgs<T> A) {
     extern __shared__ __align__(16) unsigned char s_raw[];
     cg::cluster_group cluster = cg::this_cluster();
     const int C = (int)cluster.num_blocks(), rank = (int)cluster.block_rank();
@@ -440,7 +456,7 @@ __global__ void __launch_bounds__(1024, 1) k_ising_resident(const IsingRunArgs<T
         }
         if (k == A.K) break;
         // ---- draw sweep k: s = the count just computed, Boltzmann action, publish into buffer cur^1 ----
-        const T tparam = temperature_param(A.temperatures[k]);
+        const T tparam = temperature_param(PL ? A.temperatures[(size_t)k * A.B + b] : A.temperatures[k]);
         if (A.u != nullptr) {
 #pragma unroll
             for (int j = 0; j < kIsingRB; j++) {
@@ -493,6 +509,13 @@ __global__ void __launch_bounds__(1024, 1) k_ising_resident(const IsingRunArgs<T
         if (FAST || (r < rows && active)) A.spins[lbase + (size_t)(row0 + r) * L + x] = (int8_t)a_cur[j];
     }
     cluster.sync();       // nobody leaves while a neighbour's last remote store may still be in flight
+}
+
+template <typename T, bool FAST>
+__global__ void __launch_bounds__(1024, 1) k_ising_resident(const IsingRunArgs<T> A) { ising_resident_sweeps<T, FAST, false>(A); }
+template <typename T, bool FAST>
+__global__ void __launch_bounds__(1024, 1) k_ising_resident_lattices(const IsingRunArgs<T> A) {
+    ising_resident_sweeps<T, FAST, true>(A);
 }
 
 // ---- K6r specialised for fp32 and compile-time shapes (the bench shape 256 x 256 / 16 rows per CTA and the other
@@ -1007,7 +1030,8 @@ __device__ __forceinline__ uint32_t field_sum(uint32_t x) {            // sum of
     return (((x & 0x0F0F0F0Fu) + ((x >> 4) & 0x0F0F0F0Fu)) * 0x01010101u) >> 24;
 }
 
-template <int L, int RPT, bool MASK>
+// PL: A.temperatures is [K][B]; the log2e / T table is refilled from lattice b's column (prefetched during the previous lattice) when a slot takes lattice b up
+template <int L, int RPT, bool MASK, bool PL>
 __global__ void __launch_bounds__(2 * L, 512 / (2 * L) > 0 ? 512 / (2 * L) : 1) k_ising_persist_swar_f32(const IsingRunArgs<float> A, const int n_slots,
                                                                      unsigned long long *const halo) {
     static_assert(L % 32 == 0 && RPT % kIsingRB == 0 && RPT <= 8 && L % (2 * RPT) == 0, "shape");
@@ -1025,6 +1049,7 @@ __global__ void __launch_bounds__(2 * L, 512 / (2 * L) > 0 ? 512 / (2 * L) : 1) 
     unsigned long long *s_edge = s_inner + 2 * 2 * WPR;                             // [2 parity][2 band][WPR][2] {field word of lane 0 / 31, seq}
     int *s_wstat = (int *)(s_edge + 2 * 2 * WPR * 2);                               // [NW][32] packed statistics of up to 32 sweeps per warp
     float *s_tparam = (float *)(s_wstat + NW * 32);                                 // [K]
+    float *s_traw = s_tparam + A.K;                     // PL: [K] the raw temperatures of the slot's next lattice
     constexpr uint32_t INNER_BUF = 2u * WPR * 8u, EDGE_BUF = 2u * WPR * 2u * 8u;
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -1044,7 +1069,17 @@ __global__ void __launch_bounds__(2 * L, 512 / (2 * L) > 0 ? 512 / (2 * L) : 1) 
     const unsigned long long *const mb_in = halo + (((size_t)slot * C + rank) * 2 * 2 + (upper ? 0 : 1)) * WPR + w;
     unsigned long long *const mb_out = halo + (((size_t)slot * C + (upper ? up_rank : dn_rank)) * 2 * 2 + (upper ? 1 : 0)) * WPR + w;
 
-    for (int i = tid; i < A.K; i += NT) s_tparam[i] = temperature_param(A.temperatures[i]);
+    if (!PL) for (int i = tid; i < A.K; i += NT) s_tparam[i] = temperature_param(A.temperatures[i]);
+    // PL: lattice bb's column of the [K][B] table, copied into s_traw with cp.async while the slot still sweeps the
+    // lattice before it (a strided gather of K words: its latency would otherwise stall every hand-over).  Thread tid
+    // copies, and later converts, exactly the entries i = tid + j NT, so it only waits for its own copies.
+    auto prefetch_column = [&](int bb) {
+        for (int i = tid; i < A.K; i += NT)
+            asm volatile("cp.async.ca.shared.global [%0], [%1], 4;"
+                         :: "r"(smem_addr(s_traw + i)), "l"(A.temperatures + (size_t)i * A.B + bb) : "memory");
+        asm volatile("cp.async.commit_group;" ::: "memory");
+    };
+    if (PL && slot < A.B) prefetch_column(slot);
     for (int i = tid; i < 2 * 2 * WPR * 3; i += NT) s_inner[i] = 0ull;              // (s_inner and s_edge are contiguous) sequence numbers start at 1
 
     // everything a lattice needs, for the upper band (slot i = row i of the strip) or the lower one (slot i = row ROWS-1-i)
@@ -1222,6 +1257,11 @@ __global__ void __launch_bounds__(2 * L, 512 / (2 * L) > 0 ? 512 / (2 * L) : 1) 
     for (int b = slot; b < A.B; b += n_slots, state_no += (uint32_t)A.K + 1u) {
         const size_t lbase = (size_t)b * N;
         __syncthreads();                                        // the previous lattice's Q strip has been stored (first pass: the tables are set)
+        if (PL) {                                               // (every warp has left the previous lattice's last draw)
+            asm volatile("cp.async.wait_all;" ::: "memory");
+            for (int i = tid; i < A.K; i += NT) s_tparam[i] = temperature_param(s_traw[i]);
+            if (b + n_slots < A.B) prefetch_column(b + n_slots);
+        }
         for (int sp = 0; sp < 5; sp++) {
             const float4 *s4 = (const float4 *)(A.Q + (lbase * 5 + (size_t)sp * N + (size_t)row0 * L) * 2);
             float4 *d4 = (float4 *)(s_q + (size_t)sp * STRIP * 2);
@@ -1231,7 +1271,7 @@ __global__ void __launch_bounds__(2 * L, 512 / (2 * L) > 0 ? 512 / (2 * L) : 1) 
                 d4[i] = s4[(sr < RPT ? sr : ROWS - 1 - sr + RPT) * (L / 2) + c4];
             }
         }
-        __syncthreads();                                        // the strip is complete before anybody draws from it
+        __syncthreads();                                        // the strip and the table are complete before anybody draws
         if (upper) run_lattice(std::true_type{}, b, state_no);
         else run_lattice(std::false_type{}, b, state_no);
         for (int sp = 0; sp < 5; sp++) {
@@ -1245,6 +1285,7 @@ __global__ void __launch_bounds__(2 * L, 512 / (2 * L) > 0 ? 512 / (2 * L) : 1) 
         }
     }
 }
+
 
 template <typename T>
 static size_t resident_smem_bytes(int L, int rows) {
@@ -1282,9 +1323,11 @@ static void specialised_resident_kernel(const IsingRunArgs<float> &A, void (*&ke
 #undef MF_PICK
 }
 
-// K6p launcher (fp32, C > 1 strips per lattice): false = no persistent specialisation for this shape / switched off
-static bool launch_ising_persistent(const IsingRunArgs<double> &, cudaStream_t) { return false; }
-static bool launch_ising_persistent(const IsingRunArgs<float> &A, cudaStream_t st) {
+// K6p launcher (fp32, C > 1 strips per lattice): false = no persistent specialisation for this shape / switched off.
+// pl: per-lattice temperature table [K][B]; only K6s has such a variant (launch_ising_resident refuses the overrides
+// that would select K6p before it gets here)
+static bool launch_ising_persistent(const IsingRunArgs<double> &, cudaStream_t, bool) { return false; }
+static bool launch_ising_persistent(const IsingRunArgs<float> &A, cudaStream_t st, bool pl) {
     const char *env = getenv("MFMARL_ISING_PERSIST");
     const char *renv = getenv("MFMARL_ISING_RPT");
     if (A.L != 512) {                                               // (512: K6s is the only resident kernel, see below)
@@ -1299,7 +1342,7 @@ static bool launch_ising_persistent(const IsingRunArgs<float> &A, cudaStream_t s
         if (rpt == 8) { kern = A.mask ? k_ising_persist_f32<LL, RR, 8, true> : k_ising_persist_f32<LL, RR, 8, false>; threads = LL * (RR / 8); } \
         else { kern = A.mask ? k_ising_persist_f32<LL, RR, 4, true> : k_ising_persist_f32<LL, RR, 4, false>; threads = LL * (RR / 4); } \
     }
-    MF_PICK(256, 16) MF_PICK(128, 32)
+    if (!pl) { MF_PICK(256, 16) MF_PICK(128, 32) }
 #undef MF_PICK
     // K6s (SWAR neighbour counts): strips of two bands of 8 rows whatever K6r's cluster would be (no cluster here, so
     // the strip height is free); MFMARL_ISING_PERSIST=1 keeps K6p
@@ -1307,7 +1350,8 @@ static bool launch_ising_persistent(const IsingRunArgs<float> &A, cudaStream_t s
     bool swar = false;
     if (!(env && atoi(env) == 1) && rpt == 8) {
 #define MF_PICK(LL) \
-        if (A.L == LL) { kern = A.mask ? k_ising_persist_swar_f32<LL, 8, true> : k_ising_persist_swar_f32<LL, 8, false>; \
+        if (A.L == LL) { kern = pl ? (A.mask ? k_ising_persist_swar_f32<LL, 8, true, true> : k_ising_persist_swar_f32<LL, 8, false, true>) \
+                                   : (A.mask ? k_ising_persist_swar_f32<LL, 8, true, false> : k_ising_persist_swar_f32<LL, 8, false, false>); \
                          threads = 2 * LL; rows_per = 16; swar = true; }
         MF_PICK(256) MF_PICK(128) MF_PICK(64)
 #undef MF_PICK
@@ -1315,7 +1359,8 @@ static bool launch_ising_persistent(const IsingRunArgs<float> &A, cudaStream_t s
     // 512 x 512: a 16-row strip's Q (327 KB) does not fit, so strips of 8 rows with 4 rows per thread (1024 threads, 64
     // registers); no cluster kernel exists for this side, so neither MFMARL_ISING_PERSIST nor _RPT (other than 0) applies
     if (A.L == 512) {
-        kern = A.mask ? k_ising_persist_swar_f32<512, 4, true> : k_ising_persist_swar_f32<512, 4, false>;
+        kern = pl ? (A.mask ? k_ising_persist_swar_f32<512, 4, true, true> : k_ising_persist_swar_f32<512, 4, false, true>)
+                  : (A.mask ? k_ising_persist_swar_f32<512, 4, true, false> : k_ising_persist_swar_f32<512, 4, false, false>);
         threads = 1024; rows_per = 8; swar = true;
     }
     if (!kern) return false;
@@ -1325,18 +1370,18 @@ static bool launch_ising_persistent(const IsingRunArgs<float> &A, cudaStream_t s
         for (int k0 = 0; k0 < A.K; k0 += kMaxSweeps) {
             IsingRunArgs<float> part = A;
             part.K = std::min(kMaxSweeps, A.K - k0);
-            part.temperatures = A.temperatures + k0; part.step0 = A.step0 + (uint32_t)k0;
+            part.temperatures = A.temperatures + (size_t)k0 * (pl ? A.B : 1); part.step0 = A.step0 + (uint32_t)k0;
             if (A.u) part.u = A.u + (size_t)k0 * A.B * A.L * A.L;
             if (A.mask) part.mask = A.mask + (size_t)k0 * A.B * A.L * A.L;
             part.n_up = A.n_up + (size_t)k0 * A.B;
             if (A.reward_sum) part.reward_sum = A.reward_sum + (size_t)k0 * A.B;
-            if (!launch_ising_persistent(part, st)) return false;
+            if (!launch_ising_persistent(part, st, pl)) return false;
         }
         return true;
     }
     // K6p: bit buffers + statistics; K6s: message slots [2][2][wpr] x (1 + 2) of 8 bytes + [warps][32] statistics
     const size_t smem = (swar ? (size_t)5 * rows_per * A.L * 8 + (size_t)2 * 2 * wpr * 3 * 8 + (size_t)(threads / 32) * 32 * 4
-                              : resident_smem_bytes<float>(A.L, rows_per)) + (size_t)A.K * sizeof(float);
+                              : resident_smem_bytes<float>(A.L, rows_per)) + (size_t)A.K * sizeof(float) * (pl ? 2 : 1);
     MF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int dev = 0, n_sm = 0, per_sm = 0;
     MF_CUDA(cudaGetDevice(&dev));
@@ -1380,20 +1425,37 @@ static bool launch_ising_persistent(const IsingRunArgs<float> &A, cudaStream_t s
     return true;
 }
 
+// The environment overrides that select a kernel without per-lattice temperature tables (K6p, the specialised K6r)
+// refuse a per-lattice call instead of running another kernel.  They only ever apply to fp32 below side 512.
+static void refuse_per_lattice_overrides(int L) {
+    const char *penv = getenv("MFMARL_ISING_PERSIST"), *renv = getenv("MFMARL_ISING_RPT");
+    if (L == 512) return;
+    if (penv && atoi(penv) == 1)
+        throw Fatal("MFMARL_ISING_PERSIST=1 selects K6p, which has no per-lattice temperature tables");
+    if (renv && atoi(renv) != 0 && atoi(renv) != 8)
+        throw Fatal(std::string("MFMARL_ISING_RPT=") + renv + " selects a specialised kernel without per-lattice temperature tables");
+    if (penv && atoi(penv) == 0 && !(renv && atoi(renv) == 0) && (L == 64 || L == 128 || L == 256))
+        throw Fatal("MFMARL_ISING_PERSIST=0 selects the specialised cluster kernel k_ising_resident_f32, which has no per-lattice "
+                    "temperature tables (MFMARL_ISING_RPT=0 selects the generic one)");
+}
+
+// pl: A.temperatures is [K][B] (per-lattice schedules, mfi_run_lattices) instead of [K]
 template <typename T>
-static void launch_ising_resident(const IsingRunArgs<T> &A0, cudaStream_t st) {
+static void launch_ising_resident(const IsingRunArgs<T> &A0, cudaStream_t st, bool pl = false) {
     IsingRunArgs<T> A = A0;
     const int L = A.L, wpr = (L + 31) >> 5, LP = wpr * 32;
     const int C = resident_cluster_size<T>(L);
     A.rows_per = C > 0 ? L / C : 0;
-    if (launch_ising_persistent(A, st)) return;                     // (declines shapes it has no specialisation for)
+    if (pl && sizeof(T) == 4) refuse_per_lattice_overrides(L);
+    if (launch_ising_persistent(A, st, pl)) return;                 // (declines shapes it has no specialisation for)
     if (C == 0) throw Fatal("ising resident kernel: lattice side " + std::to_string(L) + " not supported (use mfi_step)");
     const int bands = (A.rows_per + kIsingRB - 1) / kIsingRB;
     const size_t smem = resident_smem_bytes<T>(L, A.rows_per);
     const bool fast = (L % 32 == 0) && (A.rows_per % kIsingRB == 0);
-    void (*kern)(const IsingRunArgs<T>) = fast ? k_ising_resident<T, true> : k_ising_resident<T, false>;
+    void (*kern)(const IsingRunArgs<T>) = pl ? (fast ? k_ising_resident_lattices<T, true> : k_ising_resident_lattices<T, false>)
+                                             : (fast ? k_ising_resident<T, true> : k_ising_resident<T, false>);
     unsigned threads = (unsigned)(LP * bands);
-    specialised_resident_kernel(A, kern, threads);
+    if (!pl) specialised_resident_kernel(A, kern, threads);
     MF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (C > 8) MF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
     cudaLaunchConfig_t cfg{};
@@ -1501,6 +1563,30 @@ extern "C" int mfi_step(int dtype, int n_lattices, int side, int8_t *d_spins, vo
     return 0;
 }
 
+extern "C" int mfi_step_lattices(int dtype, int n_lattices, int side, int8_t *d_spins, void *d_q,
+                                 const void *d_temperatures, double lr, const void *d_uniforms,
+                                 const uint8_t *d_update_mask, unsigned seed, unsigned lattice_base, unsigned step,
+                                 int32_t *d_n_up, void *d_reward_sum, void *d_mse, void *stream) {
+    try {
+        if (!d_temperatures) throw Fatal("need a device temperature table [n_lattices]");
+        if (dtype == 0) {
+            IsingArgs<float> A{n_lattices, side, d_spins, (float *)d_q, 0.0f, (float)lr,
+                               (const float *)d_uniforms, d_update_mask, seed, lattice_base, step, d_n_up,
+                               (float *)d_reward_sum, (float *)d_mse};
+            launch_ising(A, (cudaStream_t)stream, (const float *)d_temperatures);
+        } else if (dtype == 1) {
+            IsingArgs<double> A{n_lattices, side, d_spins, (double *)d_q, 0.0, lr,
+                                (const double *)d_uniforms, d_update_mask, seed, lattice_base, step, d_n_up,
+                                (double *)d_reward_sum, (double *)d_mse};
+            launch_ising(A, (cudaStream_t)stream, (const double *)d_temperatures);
+        } else throw Fatal("dtype must be 0 (f32) or 1 (f64)");
+    } catch (const std::exception &ex) {
+        set_last_error(std::string("mfi_step_lattices: ") + ex.what());
+        return -1;
+    }
+    return 0;
+}
+
 extern "C" int mfi_resident_cluster_size(int dtype, int side) {
     if (dtype != 1 && side == 512) return 64;          // K6s only: 64 strips of 8 rows (no cluster kernel at this side)
     return dtype == 1 ? resident_cluster_size<double>(side) : resident_cluster_size<float>(side);
@@ -1525,6 +1611,31 @@ extern "C" int mfi_run(int dtype, int n_lattices, int side, int n_sweeps, int8_t
         } else throw Fatal("mfi_run: dtype must be 0 (f32) or 1 (f64)");
     } catch (const std::exception &ex) {
         set_last_error(std::string("mfi_run: ") + ex.what());
+        return -1;
+    }
+    return 0;
+}
+
+extern "C" int mfi_run_lattices(int dtype, int n_lattices, int side, int n_sweeps, int8_t *d_spins, void *d_q,
+                                const void *d_temperatures, double lr, const void *d_uniforms,
+                                const uint8_t *d_update_mask, unsigned seed, unsigned lattice_base, unsigned step0,
+                                int32_t *d_n_up, void *d_reward_sum, void *stream) {
+    try {
+        if (n_sweeps < 1 || n_lattices < 1) throw Fatal("need at least one sweep and one lattice");
+        if (!d_temperatures) throw Fatal("need a device temperature table [n_sweeps][n_lattices]");
+        if (dtype == 0) {
+            IsingRunArgs<float> A{n_lattices, side, n_sweeps, 0, d_spins, (float *)d_q, (const float *)d_temperatures,
+                                  (float)lr, (const float *)d_uniforms, d_update_mask, seed, lattice_base, step0, d_n_up,
+                                  (float *)d_reward_sum};
+            launch_ising_resident(A, (cudaStream_t)stream, true);
+        } else if (dtype == 1) {
+            IsingRunArgs<double> A{n_lattices, side, n_sweeps, 0, d_spins, (double *)d_q, (const double *)d_temperatures,
+                                   lr, (const double *)d_uniforms, d_update_mask, seed, lattice_base, step0, d_n_up,
+                                   (double *)d_reward_sum};
+            launch_ising_resident(A, (cudaStream_t)stream, true);
+        } else throw Fatal("dtype must be 0 (f32) or 1 (f64)");
+    } catch (const std::exception &ex) {
+        set_last_error(std::string("mfi_run_lattices: ") + ex.what());
         return -1;
     }
     return 0;

@@ -57,18 +57,32 @@ class IsingMFQ:
         self.mse = torch.zeros((n_lattices,), dtype=dtype, device=self.device)
 
     def step(self, temperature, uniforms=None, update_mask=None, stats=True):
-        """One fused sweep.  uniforms [B, N] (same dtype) injects the Boltzmann draws (test hook);
+        """One fused sweep.  temperature: a number, or a [B] tensor with one temperature per lattice;
+        uniforms [B, N] (same dtype) injects the Boltzmann draws (test hook);
         update_mask uint8 [B, N] restricts the Q update to the act group (act_rate < 1)."""
         if uniforms is not None:
             assert uniforms.dtype == self.dtype and uniforms.is_cuda and uniforms.is_contiguous()
         if update_mask is not None:
             assert update_mask.dtype == torch.uint8 and update_mask.is_cuda and update_mask.is_contiguous()
+        # a one-element tensor stays the shared temperature it always was
+        per_lattice = isinstance(temperature, torch.Tensor) and temperature.dim() == 1 and temperature.numel() > 1
+        if per_lattice:
+            assert tuple(temperature.shape) == (self.B,), "per-lattice temperatures must be [n_lattices]"
+            temps = temperature.to(device=self.device, dtype=self.dtype).contiguous()
         with torch.cuda.device(self.device):
-            check(self.lib.mfi_step(_DTYPES[self.dtype], self.B, self.L, _ptr(self.spins), _ptr(self.Q),
-                                    float(temperature), float(self.lr), _ptr(uniforms), _ptr(update_mask),
-                                    self.seed, self.lattice_base, self.t, _ptr(self.n_up),
-                                    _ptr(self.reward_sum) if stats else None, _ptr(self.mse) if stats else None,
-                                    ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+            stream = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
+            if per_lattice:
+                check(self.lib.mfi_step_lattices(_DTYPES[self.dtype], self.B, self.L, _ptr(self.spins), _ptr(self.Q),
+                                                 _ptr(temps), float(self.lr), _ptr(uniforms), _ptr(update_mask),
+                                                 self.seed, self.lattice_base, self.t, _ptr(self.n_up),
+                                                 _ptr(self.reward_sum) if stats else None,
+                                                 _ptr(self.mse) if stats else None, stream))
+            else:
+                check(self.lib.mfi_step(_DTYPES[self.dtype], self.B, self.L, _ptr(self.spins), _ptr(self.Q),
+                                        float(temperature), float(self.lr), _ptr(uniforms), _ptr(update_mask),
+                                        self.seed, self.lattice_base, self.t, _ptr(self.n_up),
+                                        _ptr(self.reward_sum) if stats else None, _ptr(self.mse) if stats else None,
+                                        stream))
         self.t += 1
         return self.n_up, self.reward_sum, self.mse
 
@@ -80,10 +94,14 @@ class IsingMFQ:
     def run(self, temperatures, uniforms=None, resident=None, update_mask=None):
         """len(temperatures) sweeps.  With the resident kernel (default when the shape allows) they run in ONE
         launch with Q in shared memory; otherwise one streaming launch per sweep.  Both give the same bits.
+        temperatures: a [K] schedule shared by every lattice, or a [K, B] tensor (column b = lattice b's schedule).
         update_mask uint8 [K, B, N]: the act group of every sweep (act_rate < 1).
         Returns (n_up int32 [K, B], reward_sum [K, B])."""
         temps = torch.as_tensor(temperatures, dtype=self.dtype, device=self.device).contiguous()
-        K = int(temps.numel())
+        per_lattice = temps.dim() == 2 and temps.shape[1] > 1          # ([K, 1] stays a shared schedule, as before)
+        if per_lattice:
+            assert temps.shape[1] == self.B, "per-lattice temperatures must be [n_sweeps, n_lattices]"
+        K = int(temps.shape[0]) if per_lattice else int(temps.numel())
         if resident is None:
             resident = self.resident_cluster > 0
         n_up = torch.zeros((K, self.B), dtype=torch.int32, device=self.device)
@@ -95,16 +113,17 @@ class IsingMFQ:
             assert update_mask.dtype == torch.uint8 and update_mask.is_cuda and update_mask.is_contiguous()
             assert tuple(update_mask.shape) == (K, self.B, self.N)
         if resident:
+            run = self.lib.mfi_run_lattices if per_lattice else self.lib.mfi_run
             with torch.cuda.device(self.device):
-                check(self.lib.mfi_run(_DTYPES[self.dtype], self.B, self.L, K, _ptr(self.spins), _ptr(self.Q),
-                                       _ptr(temps), float(self.lr), _ptr(uniforms), _ptr(update_mask), self.seed,
-                                       self.lattice_base,
-                                       self.t, _ptr(n_up), _ptr(rsum),
-                                       ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+                check(run(_DTYPES[self.dtype], self.B, self.L, K, _ptr(self.spins), _ptr(self.Q),
+                          _ptr(temps), float(self.lr), _ptr(uniforms), _ptr(update_mask), self.seed,
+                          self.lattice_base,
+                          self.t, _ptr(n_up), _ptr(rsum),
+                          ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
             self.t += K
             self.n_up.copy_(n_up[-1])
         else:
-            host_t = temps.cpu().tolist()
+            host_t = temps if per_lattice else temps.cpu().tolist()
             for k in range(K):
                 self.step(host_t[k], uniforms=None if uniforms is None else uniforms[k],
                           update_mask=None if update_mask is None else update_mask[k])
@@ -121,6 +140,55 @@ class IsingMFQ:
     def q_table(self):
         """Q as the reference lays it out: [B, N, 5, 2]."""
         return self.Q.permute(0, 2, 1, 3).contiguous()
+
+
+class IsingMetropolis:
+    """Checkerboard single-spin-flip Metropolis chains (kernel K8, C ABI `mfi_metropolis`) on B independent L x L tori
+    of the model MF-Q learns on: H = -1/2 sum_i sigma_i sum_nbr sigma_j, the same temperature axis (Tc ~ 1.1346).
+    The MCMC reference of the order-parameter-against-temperature curve.  L even, 2 <= L <= 512."""
+
+    def __init__(self, n_lattices, side, seed=13, lattice_base=0, spins=None, device=None):
+        if not torch.cuda.is_available():
+            raise RuntimeError("IsingMetropolis needs a CUDA device: there is no CPU fallback")
+        self.lib = load_library()
+        self.device = torch.device(device if device is not None else "cuda:%d" % torch.cuda.current_device())
+        self.B, self.L, self.N = n_lattices, side, side * side
+        self.seed, self.lattice_base = seed, lattice_base
+        self.t = 0
+        if spins is None:   # Bernoulli(0.5) spins, as IsingMFQ
+            gen = torch.Generator(device=self.device)
+            gen.manual_seed(seed + 7919 * lattice_base)
+            spins = torch.randint(0, 2, (n_lattices, side, side), generator=gen, device=self.device,
+                                  dtype=torch.int8)
+        self.spins = torch.as_tensor(spins, dtype=torch.int8, device=self.device).contiguous().clone()
+        assert tuple(self.spins.shape) == (n_lattices, side, side)
+        self.n_up = (self.spins != 0).sum(dim=(1, 2)).to(torch.int32)
+
+    def run(self, temperatures):
+        """K sweeps in one launch.  temperatures: [K] shared by every lattice, or [K, B] (column b = lattice b's).
+        Returns (n_up int32 [K, B], bond_sum int32 [K, B]): up spins and sum over the 2N bonds of sigma_i sigma_j
+        after every sweep (bond_sum = MF-Q's reward_sum; energy per site = -bond_sum / N)."""
+        temps = np.asarray(temperatures.cpu() if isinstance(temperatures, torch.Tensor) else temperatures,
+                           dtype=np.float64)
+        if temps.ndim == 1:
+            temps = np.repeat(temps[:, None], self.B, axis=1)
+        assert temps.ndim == 2 and temps.shape[1] == self.B, "temperatures must be [K] or [K, n_lattices]"
+        temps = np.ascontiguousarray(temps)
+        K = temps.shape[0]
+        n_up = torch.empty((K, self.B), dtype=torch.int32, device=self.device)
+        bond_sum = torch.empty((K, self.B), dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            check(self.lib.mfi_metropolis(self.B, self.L, K, _ptr(self.spins), temps.ctypes.data_as(ctypes.c_void_p),
+                                          self.seed, self.lattice_base, self.t, _ptr(n_up), _ptr(bond_sum),
+                                          ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+        self.t += K
+        self.n_up.copy_(n_up[-1])
+        return n_up, bond_sum
+
+    def order_param(self):
+        """|n_up - n_down| / N per lattice after the last sweep"""
+        up = self.n_up.to(torch.float64)
+        return (2 * up - self.N).abs() / torch.full_like(up, float(self.N))
 
 
 def temperature_schedule(t0, n, decay_rate, decay_gap, floor, start=0.3):

@@ -60,6 +60,11 @@ def load_library(path=None):
         "mfb_host_wait": [vp, ci],
         "mfb_alloc_device": [ctypes.c_ulong, ci, ctypes.POINTER(vp), ctypes.POINTER(ci)],
         "mfb_free_device": [vp],
+        "mfi_step_lattices": [ci, ci, ci, vp, vp, vp, ctypes.c_double, vp, vp, ctypes.c_uint, ctypes.c_uint,
+                              ctypes.c_uint, vp, vp, vp, vp],
+        "mfi_run_lattices": [ci, ci, ci, ci, vp, vp, vp, ctypes.c_double, vp, vp, ctypes.c_uint, ctypes.c_uint,
+                             ctypes.c_uint, vp, vp, vp],
+        "mfi_metropolis": [ci, ci, ci, vp, vp, ctypes.c_uint, ctypes.c_uint, ctypes.c_uint, vp, vp, vp],
     }
     for name, argtypes in sig.items():
         fn = getattr(lib, name)
