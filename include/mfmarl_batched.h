@@ -170,7 +170,10 @@ const char *mfb_last_error(void);
  *   d_q            T    [n_lattices][5][side*side][2]  in/out, entry (s, a) of site i at ((s*N + i)*2 + a)
  *   d_uniforms     T    [n_lattices][side*side] or NULL: injected uniforms (test hook; a = [u >= p0]);
  *                  NULL = Philox4x32-10, key (seed, lattice_base + lattice), counter (column, row / 4, step, 0);
- *                  output word row % 4 is the site's draw, u = that word (rounded toward zero to 24 bits) / 2^32
+ *                  fp32: output word row % 4 is the site's draw, u = that word (rounded toward zero to 24 bits) / 2^32;
+ *                  fp64: two calls, counter word 3 = 0 for rows 4j, 4j+1 and 1 for rows 4j+2, 4j+3, each call serving
+ *                  two rows: (hi, lo) = output words (0, 1) for the even row and (2, 3) for the odd one, and
+ *                  u = ((hi >> 5) * 2^26 + (lo >> 6)) / 2^53 (53 bits, in [0, 1))
  *   d_update_mask  uint8[n_lattices][side*side] or NULL: the act group (act_rate < 1); NULL = all sites
  *   d_n_up         int32[n_lattices]  out: up spins after the sweep (order parameter = |2 up - N| / N)
  *   d_reward_sum,
