@@ -243,6 +243,30 @@ int mfi_metropolis(int n_lattices, int side, int n_sweeps, int8_t *d_spins, cons
                    unsigned seed, unsigned lattice_base, unsigned step0, int32_t *d_n_up, int32_t *d_bond_sum,
                    void *stream);
 
+/* ---- K9: Swendsen-Wang cluster updates on the same lattice model (the MCMC reference near Tc and at odd sides)
+ * H = -1/2 sum_bonds sigma_i sigma_j as for K8.  Site i = y * side + x owns its right bond to ((x + 1) mod side, y) and
+ * its down bond to (x, (y + 1) mod side): 2N bonds (at side 2 the two bonds between a pair of sites are distinct).
+ * One sweep:
+ *   1. a bond is active iff its two spins are aligned and its Philox word r satisfies r < thr with
+ *        thr = min(floor((1 - exp(-1 / T)) * 2^32), 2^32 - 1)   computed on the HOST in double with the C library's exp
+ *      (T = 1e-3 clamps to 2^32 - 1; T = 1e20 gives 0, no bonds);
+ *   2. clusters are the connected components of the active bonds; a cluster's canonical label is its SMALLEST flat site
+ *      index (the kernel's result depends on this label only, never on the order in which its threads merge);
+ *   3. the cluster with root r flips as a whole iff r's flip word has its top bit set (word >= 2^31);
+ *   4. d_n_up / d_bond_sum as for K8, of the final spins of the sweep.
+ * Philox4x32-10: key (seed, lattice_base + lattice); in sweep step0 + k
+ *   bond words of site i: counter (i >> 1, step0 + k, 0, 3), output word 2 (i & 1) = its right bond,
+ *                         2 (i & 1) + 1 = its down bond
+ *   flip word of root r:  output word r & 3 of counter (r >> 2, step0 + k, 1, 3)
+ * (the 3 keeps the stream apart from MF-Q's 0 / 1 and K8's 2).
+ *   side            2 <= side <= 256, odd or even (the uint16 cluster labels of a lattice live in shared memory)
+ *   other arguments as for mfi_metropolis
+ * Bad input (side out of range, T <= 0, inf or NaN, null spins or temperatures, fewer than one lattice or one sweep)
+ * returns -1 with a message prefixed "mfi_swendsen_wang: " before anything is launched or written. */
+int mfi_swendsen_wang(int n_lattices, int side, int n_sweeps, int8_t *d_spins, const double *h_temperatures,
+                      unsigned seed, unsigned lattice_base, unsigned step0, int32_t *d_n_up, int32_t *d_bond_sum,
+                      void *stream);
+
 /* The Ising ENVIRONMENT interface (examples/ising_model/multiagent/environment.py:49-92 `_step` / `_reset`,
  * multiagent/core.py:99-125 `IsingWorld.step`, Ising.py:101-118 reward / observation) for callers that bring their
  * own policy, e.g. the unmodified main_MFQ_Ising.py over python/examples/ising_model (same package layout as the

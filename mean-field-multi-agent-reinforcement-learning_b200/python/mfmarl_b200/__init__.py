@@ -5,6 +5,7 @@ buffers (device memory, streams); the engine never runs on the CPU.
 """
 from .lib import load_library, LIB_PATH
 from .battle import BatchedGridWorld, mean_action
-from .ising import IsingMFQ, IsingMetropolis
+from .ising import IsingMFQ, IsingMetropolis, IsingSwendsenWang
 
-__all__ = ["load_library", "LIB_PATH", "BatchedGridWorld", "mean_action", "IsingMFQ", "IsingMetropolis"]
+__all__ = ["load_library", "LIB_PATH", "BatchedGridWorld", "mean_action", "IsingMFQ", "IsingMetropolis",
+           "IsingSwendsenWang"]

@@ -5,6 +5,9 @@ advances all of them by one fused step per call: Boltzmann action per site, spin
 -- the loop body of the reference's main_MFQ_Ising.py:105-134.  `run` re-expresses that script's outer loop
 (temperature schedule :108-112, order-parameter stagnation stop :149-156) over the fused step, with the
 same command-line flags (:13-26).
+
+The MCMC references of the same model: `IsingMetropolis` (checkerboard single-spin flips, kernel K8, `mfi_metropolis`)
+and `IsingSwendsenWang` (cluster updates, kernel K9, `mfi_swendsen_wang`).
 """
 import argparse
 import ctypes
@@ -142,14 +145,15 @@ class IsingMFQ:
         return self.Q.permute(0, 2, 1, 3).contiguous()
 
 
-class IsingMetropolis:
-    """Checkerboard single-spin-flip Metropolis chains (kernel K8, C ABI `mfi_metropolis`) on B independent L x L tori
-    of the model MF-Q learns on: H = -1/2 sum_i sigma_i sum_nbr sigma_j, the same temperature axis (Tc ~ 1.1346).
-    The MCMC reference of the order-parameter-against-temperature curve.  L even, 2 <= L <= 512."""
+class _IsingChain:
+    """B independent L x L tori of the model MF-Q learns on, H = -1/2 sum_bonds sigma_i sigma_j, on the same temperature
+    axis (Tc ~ 1.1346), advanced by the MCMC kernel behind the C entry point `_entry` (which takes mfi_metropolis's
+    arguments)."""
+    _entry = None
 
     def __init__(self, n_lattices, side, seed=13, lattice_base=0, spins=None, device=None):
         if not torch.cuda.is_available():
-            raise RuntimeError("IsingMetropolis needs a CUDA device: there is no CPU fallback")
+            raise RuntimeError("%s needs a CUDA device: there is no CPU fallback" % type(self).__name__)
         self.lib = load_library()
         self.device = torch.device(device if device is not None else "cuda:%d" % torch.cuda.current_device())
         self.B, self.L, self.N = n_lattices, side, side * side
@@ -178,9 +182,10 @@ class IsingMetropolis:
         n_up = torch.empty((K, self.B), dtype=torch.int32, device=self.device)
         bond_sum = torch.empty((K, self.B), dtype=torch.int32, device=self.device)
         with torch.cuda.device(self.device):
-            check(self.lib.mfi_metropolis(self.B, self.L, K, _ptr(self.spins), temps.ctypes.data_as(ctypes.c_void_p),
-                                          self.seed, self.lattice_base, self.t, _ptr(n_up), _ptr(bond_sum),
-                                          ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+            check(getattr(self.lib, self._entry)(self.B, self.L, K, _ptr(self.spins),
+                                                 temps.ctypes.data_as(ctypes.c_void_p), self.seed, self.lattice_base,
+                                                 self.t, _ptr(n_up), _ptr(bond_sum),
+                                                 ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
         self.t += K
         self.n_up.copy_(n_up[-1])
         return n_up, bond_sum
@@ -189,6 +194,20 @@ class IsingMetropolis:
         """|n_up - n_down| / N per lattice after the last sweep"""
         up = self.n_up.to(torch.float64)
         return (2 * up - self.N).abs() / torch.full_like(up, float(self.N))
+
+
+class IsingMetropolis(_IsingChain):
+    """Checkerboard single-spin-flip Metropolis chains (kernel K8, C ABI `mfi_metropolis`) on B independent L x L tori
+    of the model MF-Q learns on: H = -1/2 sum_i sigma_i sum_nbr sigma_j, the same temperature axis (Tc ~ 1.1346).
+    The MCMC reference of the order-parameter-against-temperature curve.  L even, 2 <= L <= 512."""
+    _entry = "mfi_metropolis"
+
+
+class IsingSwendsenWang(_IsingChain):
+    """Swendsen-Wang cluster chains (kernel K9, C ABI `mfi_swendsen_wang`) on B independent L x L tori of the same model
+    and temperature axis as IsingMetropolis.  Its autocorrelation time near Tc is a few sweeps at any side, so it is
+    the MCMC reference where single-spin flips decorrelate slowly; it needs no colouring.  2 <= L <= 256, odd or even."""
+    _entry = "mfi_swendsen_wang"
 
 
 def temperature_schedule(t0, n, decay_rate, decay_gap, floor, start=0.3):

@@ -1,9 +1,13 @@
 """`python -m mfmarl_b200.ising_sweep`: the Ising curve -- order parameter and bond energy against temperature -- for
-MF-Q and for a Metropolis chain of the same model, every (temperature, replica) lattice of a method in ONE batch.
+MF-Q and for MCMC chains of the same model, every (temperature, replica) lattice of a method in ONE batch.
 
 MF-Q: lattice (j, r) follows main_MFQ_Ising.py's schedule (T from 0.3, times --decay_rate every --decay_gap sweeps)
 with the floor T_j (that script's -t flag), through the per-lattice temperature tables of `mfi_run_lattices`.
-MCMC: checkerboard Metropolis (K8, `mfi_metropolis`) at T_j for every sweep.
+MCMC (`--method mcmc`, CSV label mcmc): checkerboard Metropolis (K8, `mfi_metropolis`) at T_j for every sweep; even
+sides only.
+SW (`--method sw`, CSV label sw): Swendsen-Wang cluster updates (K9, `mfi_swendsen_wang`) at T_j for every sweep; any
+side up to 256.  Near Tc its autocorrelation time is a few sweeps at any side, where Metropolis needs ~L^2 sweeps.
+`--method both` is MF-Q and Metropolis.
 Per temperature: mean and standard error over the replicas of each lattice's average, over the final --window sweeps,
 of |2 up - N| / N and of the bond energy per site -sum_bonds sigma_i sigma_j / N (-2 when ordered; the energy of the
 model, H = -1/2 sum_bonds sigma_i sigma_j, is half of it).  Lattice (j, r) is lattice j * replicas + r of the batch and
@@ -15,7 +19,7 @@ import csv
 import numpy as np
 import torch
 
-from .ising import IsingMetropolis, IsingMFQ, temperature_schedule
+from .ising import IsingMetropolis, IsingMFQ, IsingSwendsenWang, temperature_schedule
 
 COLUMNS = ["temperature", "order_mean", "order_sem", "energy_mean", "energy_sem"]
 
@@ -58,11 +62,12 @@ def run_mfq(temps, replicas, side, sweeps, seed=13, lr=0.1, decay_rate=0.99, dec
     return torch.cat(ups), torch.cat(rsums)
 
 
-def run_mcmc(temps, replicas, side, sweeps, seed=13, start="up", chunk=1000):
-    """all lattices in one IsingMetropolis -> (n_up int32 [K, B], bond_sum int32 [K, B])"""
+def run_mcmc(temps, replicas, side, sweeps, seed=13, start="up", chunk=1000, chain_class=IsingMetropolis):
+    """all lattices in one chain_class (IsingMetropolis or IsingSwendsenWang)
+    -> (n_up int32 [K, B], bond_sum int32 [K, B])"""
     B = len(temps) * replicas
     spins = torch.ones((B, side, side), dtype=torch.int8) if start == "up" else None
-    chain = IsingMetropolis(B, side, seed=seed, spins=spins)
+    chain = chain_class(B, side, seed=seed, spins=spins)
     table = np.repeat(np.asarray(temps, np.float64), replicas)[None, :]
     ups, bonds = [], []
     for k0 in range(0, sweeps, chunk):
@@ -79,13 +84,14 @@ def sweep(argv=None):
     ap.add_argument("--side", default=20, type=int, help="lattice side (the paper's 20 x 20 by default)")
     ap.add_argument("--sweeps", default=5000, type=int)
     ap.add_argument("--window", default=1000, type=int, help="final sweeps the averages are taken over")
-    ap.add_argument("--method", default="both", choices=["mfq", "mcmc", "both"])
+    ap.add_argument("--method", default="both", choices=["mfq", "mcmc", "sw", "both"],
+                    help="mcmc: Metropolis (even sides); sw: Swendsen-Wang (any side <= 256); both: mfq and mcmc")
     ap.add_argument("--seed", default=13, type=int)
     ap.add_argument("-lr", "--learning_rate", default=0.1, type=float)
     ap.add_argument("-dr", "--decay_rate", default=0.99, type=float)
     ap.add_argument("-dg", "--decay_gap", default=2000, type=int)
     ap.add_argument("--mcmc_start", default="up", choices=["up", "random"],
-                    help="Metropolis start: all up (reaches either phase fast) or Bernoulli(0.5)")
+                    help="start of the mcmc and sw chains: all up (reaches either phase fast) or Bernoulli(0.5)")
     ap.add_argument("--out", default=None, help="CSV file of the table (one row per method and temperature)")
     args = ap.parse_args(argv)
     temps = parse_grid(args.temperatures)
@@ -97,7 +103,8 @@ def sweep(argv=None):
             n_up, rsum = run_mfq(temps, args.replicas, args.side, args.sweeps, seed=args.seed, lr=args.learning_rate,
                                  decay_rate=args.decay_rate, decay_gap=args.decay_gap)
         else:
-            n_up, rsum = run_mcmc(temps, args.replicas, args.side, args.sweeps, seed=args.seed, start=args.mcmc_start)
+            n_up, rsum = run_mcmc(temps, args.replicas, args.side, args.sweeps, seed=args.seed, start=args.mcmc_start,
+                                  chain_class=IsingSwendsenWang if method == "sw" else IsingMetropolis)
         tables[method] = summarise(temps, args.replicas, args.side, n_up, rsum, args.window)
     for j, T in enumerate(temps):
         print("T = %.4f  " % T + "  ".join("%s |m| = %.4f +- %.4f  e = %.4f +- %.4f" % ((m,) + tuple(tables[m][j, 1:]))

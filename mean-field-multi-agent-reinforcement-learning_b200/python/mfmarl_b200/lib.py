@@ -65,6 +65,7 @@ def load_library(path=None):
         "mfi_run_lattices": [ci, ci, ci, ci, vp, vp, vp, ctypes.c_double, vp, vp, ctypes.c_uint, ctypes.c_uint,
                              ctypes.c_uint, vp, vp, vp],
         "mfi_metropolis": [ci, ci, ci, vp, vp, ctypes.c_uint, ctypes.c_uint, ctypes.c_uint, vp, vp, vp],
+        "mfi_swendsen_wang": [ci, ci, ci, vp, vp, ctypes.c_uint, ctypes.c_uint, ctypes.c_uint, vp, vp, vp],
     }
     for name, argtypes in sig.items():
         fn = getattr(lib, name)
