@@ -37,7 +37,8 @@ typedef struct mfb_config {
     int step_threads;      /* 0 = auto                                                               */
     int obs_tile_agents;   /* agents per observation CTA, 0 = auto: clamp(capacity, 64, 256)         */
     int obs_record;        /* per-env observation record kept by k_step for k_obs: -1 = auto (on for
-                              capacity >= 256), 0 = off, 1 = on; same observations either way          */
+                              capacity >= 256, and wherever the kernels run from HBM), 0 = off (refused
+                              where they run from HBM), 1 = on; same observations either way             */
     int concurrent_step_envs; /* pipelined use: envs of a sibling engine whose mfb_step runs on another stream while
                               this engine's mfb_observe streams; the observation kernel then leaves SM slots free
                               where a step CTA does not fit beside it (0 = not pipelined)                     */
@@ -67,7 +68,9 @@ int mfb_add_agents(mfb_engine *eng, int group, int n, const int *xs, const int *
 int mfb_add_agents_per_env(mfb_engine *eng, int group, int n, const int *xs, const int *ys, int *n_added);
 int mfb_set_seed(mfb_engine *eng, unsigned long seed);
 
-/* sizes: key in {"capacity","n_envs","n_action","view_size","n_channel","feature_size","attack_base"} */
+/* sizes: key in {"capacity","n_envs","n_action","view_size","n_channel","feature_size","attack_base"}.
+ * "hbm_kernels": the kernels that run from HBM at the engine's geometry (map, capacity after the pending placement)
+ * because their shared-memory layout exceeds a CTA's: bit 0 k_step, 1 k_obs, 2 k_obs_record, 3 k_local_mean_action. */
 int mfb_query(mfb_engine *eng, const char *key, int *out);
 
 /* K1.  d_view float[E][2][cap][13][13][7], d_feature float[E][2][cap][feature_size]; rows >= num are

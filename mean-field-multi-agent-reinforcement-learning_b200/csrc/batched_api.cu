@@ -219,6 +219,7 @@ int mfb_query(mfb_engine *h, const char *key, int *out) {
     else if (k == "n_channel") *out = 7;
     else if (k == "feature_size") *out = e.params().feature_size;
     else if (k == "attack_base") *out = e.params().n_move;
+    else if (k == "hbm_kernels") *out = e.hbm_kernels();   // 1 k_step, 2 k_obs, 4 k_obs_record, 8 k_local_mean_action
     else throw Fatal("mfb_query: unknown key " + k);
     MFB_END("mfb_query")
 }

@@ -122,6 +122,39 @@ __device__ __forceinline__ void build_obs_record(const BattleParams &P, const Ba
     }
 }
 
+// The same record for maps whose padded grid does not fit in shared memory: the grid is built in place in the env's
+// record in HBM (walls from the template, then the alive agents).  Only the minimap counts stay in shared memory
+// (s_cnt: 2*169 ints).
+__device__ __forceinline__ void build_obs_record_hbm(const BattleParams &P, const BattleState &S, int e, int *s_cnt) {
+    const int tid = threadIdx.x, nt = blockDim.x, W = P.W, cap = P.cap, PW = W + 2 * kPad;
+    const ObsRecord R = obs_record_layout(P.W, P.H, cap);
+    unsigned char *rec = S.obs_record + (size_t)e * R.total;
+    uint16_t *grid = (uint16_t *)rec;
+    const size_t ebase = (size_t)e * 2 * cap;
+    for (int c = tid; c < R.hp10 / 16; c += nt) ((uint4 *)rec)[c] = ((const uint4 *)S.grid_template)[c];
+    for (int c = tid; c < 2 * kViewCells; c += nt) s_cnt[c] = 0;
+    const int n0 = S.num[e * 2], n1 = S.num[e * 2 + 1];
+    __syncthreads();
+    const uint8_t *lut = S.mini_lut;
+    float *hp10 = (float *)(rec + R.hp10);
+    for (int s = tid; s < 2 * cap; s += nt) {
+        const int gg = s >= cap, i = s - gg * cap;
+        if (i >= (gg ? n1 : n0)) continue;
+        const int p = S.pos[ebase + s], x = pos_x(p), y = pos_y(p);
+        atomicAdd(&s_cnt[gg * kViewCells + lut[W + y] + lut[x]], 1);
+        if (!st_dead(S.state[ebase + s])) {
+            grid[(y + kPad) * PW + x + kPad] = (uint16_t)(((2 + gg) << 14) | s);
+            hp10[s] = __fdiv_rn(S.hp[ebase + s], P.hp);
+        }
+    }
+    __syncthreads();
+    float *mini = (float *)(rec + R.mini);
+    for (int c = tid; c < 2 * kViewCells; c += nt) {
+        const int tot = c >= kViewCells ? n1 : n0;
+        mini[c] = tot > 0 ? __fdiv_rn((float)s_cnt[c], (float)tot) : 0.0f;
+    }
+}
+
 // Episode start from the placement template of env e (k_place at commit, k_step's auto-reset).  `side` = 1 swaps the
 // armies: group g takes the other block's positions AND ids -- generate_map adds the left block first, so the ids
 // follow the side, not the group (senario_battle.py:14-37).
@@ -146,12 +179,14 @@ __device__ __forceinline__ void place_from_template(const BattleParams &P, const
 
 // minstd_rand0 after n steps from state s: s * 16807^n mod (2^31 - 1), square and multiply over a table of
 // 16807^(2^b) -- the reference's sequential chain (GridWorld.cc:510-515 draws one number per attack) without the chain.
+// 14 bits: n <= 2 * 8191, one draw per attack of a step (tests/test_minstd_jump_table.py checks the table).
 __device__ __forceinline__ uint32_t minstd_jump(uint32_t s, uint32_t n) {
-    const uint32_t pw[12] = {16807u, 282475249u, 984943658u, 1457850878u, 1137522503u, 1636807826u,
-                             685118024u, 515204530u, 897054849u, 2038299453u, 1836275591u, 349037107u};
+    const uint32_t pw[14] = {16807u, 282475249u, 984943658u, 1457850878u, 1137522503u, 1636807826u,
+                             685118024u, 515204530u, 897054849u, 2038299453u, 1836275591u, 349037107u,
+                             149796865u, 1186652285u};
     uint64_t acc = s;
 #pragma unroll
-    for (int b = 0; b < 12; b++)
+    for (int b = 0; b < 14; b++)
         if ((n >> b) & 1u) acc = (acc * pw[b]) % 2147483647ull;
     return (uint32_t)acc;
 }
@@ -196,24 +231,41 @@ enum { MISC_WARP = 0, MISC_N = 32, MISC_DEAD = 34, MISC_FLAG = 40, MISC_HIST = 6
 // mover results while the move phase runs
 enum : int { MV_FAIL = 0, MV_OK = 1, MV_WAIT = 2 };
 
+// Dynamic shared memory of k_step<true>: s_misc, then the minimap counts of build_obs_record_hbm.
+constexpr int kStepHbmSmem = 4 * 128 + 4 * 2 * kViewCells;
+// k_step<true>'s workspace: [E][step_smem_layout().total], right after the E observation records
+__host__ __device__ inline unsigned char *step_workspace(const BattleParams &P, const BattleState &S) {
+    return S.obs_record + (size_t)P.E * obs_record_layout(P.W, P.H, P.cap).total;
+}
+
+// HBM = false: the working set lives in dynamic shared memory (step_smem_layout(...).total bytes).  HBM = true, for
+// geometries whose layout exceeds a CTA's shared memory: the same layout in HBM, in the env's slice of the workspace
+// that follows the observation records (always kept at such geometries) in their allocation -- the shared atomics
+// become global atomics on the env's own lines, served by L2.  Only s_misc and the minimap counts stay in shared
+// memory (kStepHbmSmem bytes), and the observation record is built in place.
+template <bool HBM>
 __global__ void k_step(const __grid_constant__ BattleParams P, const BattleState S, const StepIO io) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const StepSmem L = step_smem_layout(P.W, P.H, P.cap, P.obs_cached);
-    int *s_pos = (int *)(smem_raw + L.pos);
-    float *s_hp = (float *)(smem_raw + L.hp);
-    float *s_nr = (float *)(smem_raw + L.nr);
-    uint32_t *s_state = (uint32_t *)(smem_raw + L.state);
-    uint32_t *s_att = (uint32_t *)(smem_raw + L.att);
-    int *s_aux = (int *)(smem_raw + L.aux);
-    uint32_t *s_mv = (uint32_t *)(smem_raw + L.mv);
-    int *s_mvt = (int *)(smem_raw + L.mvt);
-    int *s_scr0 = (int *)(smem_raw + L.scr0);
-    int *s_scr1 = (int *)(smem_raw + L.scr1);
-    uint16_t *s_tag_a = (uint16_t *)(smem_raw + L.tag_a);
-    uint16_t *s_tag_v = (uint16_t *)(smem_raw + L.tag_v);
-    uint16_t *s_mvidx = (uint16_t *)(smem_raw + L.mvidx);
+    unsigned char *const ws = HBM ? step_workspace(P, S) + (size_t)blockIdx.x * L.total : nullptr;
+#define STEP_AT(off) (HBM ? ws + (off) : smem_raw + (off))
+    int *s_pos = (int *)STEP_AT(L.pos);
+    float *s_hp = (float *)STEP_AT(L.hp);
+    float *s_nr = (float *)STEP_AT(L.nr);
+    uint32_t *s_state = (uint32_t *)STEP_AT(L.state);
+    uint32_t *s_att = (uint32_t *)STEP_AT(L.att);
+    int *s_aux = (int *)STEP_AT(L.aux);
+    uint32_t *s_mv = (uint32_t *)STEP_AT(L.mv);
+    int *s_mvt = (int *)STEP_AT(L.mvt);
+    int *s_scr0 = (int *)STEP_AT(L.scr0);
+    int *s_scr1 = (int *)STEP_AT(L.scr1);
+    uint16_t *s_tag_a = (uint16_t *)STEP_AT(L.tag_a);
+    uint16_t *s_tag_v = (uint16_t *)STEP_AT(L.tag_v);
+    uint16_t *s_mvidx = (uint16_t *)STEP_AT(L.mvidx);
     int *s_misc = (int *)(smem_raw + L.misc);
-    uint32_t *s_grid = (uint32_t *)(smem_raw + L.grid);
+    if constexpr (HBM) s_misc = (int *)smem_raw;
+    uint32_t *s_grid = (uint32_t *)STEP_AT(L.grid);
+#undef STEP_AT
     constexpr uint32_t kNoClaim = 0xFFFF0000u;
 
     const int e = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
@@ -650,15 +702,23 @@ __global__ void k_step(const __grid_constant__ BattleParams P, const BattleState
     }
     if (P.obs_cached && (phases & (PH_STEP | PH_CLEAR))) {        // positions / alive flags / slot indices changed
         __syncthreads();                                          // the write-back above is visible to the whole CTA
-        build_obs_record(P, S, e, (uint16_t *)(smem_raw + L.grid),
-                         (int *)(smem_raw + L.grid + obs_record_layout(P.W, P.H, P.cap).hp10));
+        if constexpr (HBM)
+            build_obs_record_hbm(P, S, e, (int *)(smem_raw + 4 * 128));
+        else
+            build_obs_record(P, S, e, (uint16_t *)(smem_raw + L.grid),
+                             (int *)(smem_raw + L.grid + obs_record_layout(P.W, P.H, P.cap).hp10));
     }
 }
 
-// the observation record of every env after a placement (commit / late add); one CTA per env
+// the observation record of every env after a placement (commit / late add); one CTA per env.  HBM = true: the padded
+// grid is built in place in the record (shared memory: the 2*169 minimap counts only)
+template <bool HBM>
 __global__ void k_obs_record(const __grid_constant__ BattleParams P, const BattleState S) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    build_obs_record(P, S, blockIdx.x, (uint16_t *)smem_raw, (int *)(smem_raw + obs_record_layout(P.W, P.H, P.cap).hp10));
+    if constexpr (HBM)
+        build_obs_record_hbm(P, S, blockIdx.x, (int *)smem_raw);
+    else
+        build_obs_record(P, S, blockIdx.x, (uint16_t *)smem_raw, (int *)(smem_raw + obs_record_layout(P.W, P.H, P.cap).hp10));
 }
 
 // ----------------------------------------------------------------------------------------------
@@ -708,7 +768,11 @@ __host__ __device__ inline ObsSmem obs_smem_layout(int W, int H, int cap, int ca
     L.stage1 = o; o += stage_bytes;
     L.rec = o;    o += 16 * kObsMaxTile;                              // (pos, id, state, last_rew) of the tile's agents
     L.record = L.cnt = L.tmpl = 0;
-    if (cached) {                                                     // the env's observation record, as one bulk copy lands it
+    if (cached == 2) {                                                // the record is read where it is, in HBM / L2
+        L.code = L.hp10 = L.mini = 0;
+        L.fxy = o;    o += 4 * (W + H);
+        o = (o + 15) & ~15;
+    } else if (cached) {                                              // the env's observation record, as one bulk copy lands it
         const ObsRecord R = obs_record_layout(W, H, cap);
         L.record = o; L.code = o + R.grid; L.hp10 = o + R.hp10; L.mini = o + R.mini; o += R.total;   // (16-byte pieces)
         L.fxy = o;    o += 4 * (W + H);
@@ -752,11 +816,14 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {     // rou
     return r;
 }
 
-template <bool CACHED, bool BF16>
+// REC_HBM (CACHED only, for records too large for shared memory): the view look-ups, hp / 10 and the minimaps are read
+// from the env's record in HBM / L2 instead of a shared-memory copy; everything after the look-ups is unchanged.
+template <bool CACHED, bool BF16, bool REC_HBM = false>
 __global__ void __launch_bounds__(kObsThreads, BF16 ? kObsCtasPerSm + 1 : kObsCtasPerSm)   // bf16 rows: smaller staging, 3 CTAs fit
 k_obs(const __grid_constant__ BattleParams P, const BattleState S, const ObsIO io) {
+    static_assert(CACHED || !REC_HBM, "the HBM record mode reads the observation record");
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    const ObsSmem L = obs_smem_layout(P.W, P.H, P.cap, CACHED, BF16);
+    const ObsSmem L = obs_smem_layout(P.W, P.H, P.cap, REC_HBM ? 2 : (int)CACHED, BF16);
     constexpr int kRowBytes = BF16 ? kViewRowBf16Bytes : kViewRow * 4;
     constexpr int kStageBytes = kObsChunk * kRowBytes;
     float *const s_stage0 = (float *)(smem_raw + L.stage0), *const s_stage1 = (float *)(smem_raw + L.stage1);
@@ -831,7 +898,11 @@ k_obs(const __grid_constant__ BattleParams P, const BattleState S, const ObsIO i
             // cp.async (LDGSTS), 16 bytes per thread and instruction, NOT a bulk copy: a bulk load is queued in the SM's
             // TMA unit behind this CTA's (and its neighbour's) 38 KB bulk stores still draining -- ncu showed 24 % of
             // the samples waiting on that load's mbarrier with 32-agent tiles; the LSU path only pays the L2 latency.
-            {
+            if constexpr (REC_HBM) {
+                unsigned char *rec = S.obs_record + (size_t)e * rec_bytes;
+                const ObsRecord R = obs_record_layout(P.W, P.H, P.cap);
+                s_code = (uint16_t *)rec; s_hp10 = (float *)(rec + R.hp10); s_mini = (float *)(rec + R.mini);
+            } else {
                 const unsigned char *src = S.obs_record + (size_t)e * rec_bytes;
                 const uint32_t dst = (uint32_t)__cvta_generic_to_shared(smem_raw + L.record);
                 for (uint32_t c = (uint32_t)tid * 16u; c < rec_bytes; c += kObsThreads * 16u)
@@ -847,7 +918,7 @@ k_obs(const __grid_constant__ BattleParams P, const BattleState S, const ObsIO i
             ng = g ? n1 : n0;
             a_end = min(ng, a_begin + io.tile_agents);
             if (tid < a_end - a_begin) s_rec[tid] = my_rec;
-            asm volatile("cp.async.wait_all;" ::: "memory");   // this thread's pieces have landed; the barrier at the top of
+            if constexpr (!REC_HBM) asm volatile("cp.async.wait_all;" ::: "memory");   // this thread's pieces have landed; the barrier at the top of
             if (a_begin >= ng) {                               // the first chunk (or of the next item) publishes everybody's
                 if (tid == 0) s_next = next_ticket;
                 continue;
@@ -1081,17 +1152,22 @@ __global__ void k_mean_action(const int32_t *__restrict__ actions, const int32_t
 // ----------------------------------------------------------------------------------------------
 constexpr int kLocalBins = 32;   // n_action <= 32 (Engine checks move + attack <= 32)
 struct LocalMeanSmem { int grid, hist, total; };
-__host__ __device__ inline LocalMeanSmem local_mean_smem_layout(int W, int H, int tile, int n_action) {
+__host__ __device__ inline LocalMeanSmem local_mean_smem_layout(int W, int H, int tile, int n_action, bool grid = true) {
     LocalMeanSmem L; int o = 0;
-    L.grid = o;  o += ((W + 2 * kPad) * (H + 2 * kPad) + 15) & ~15;
+    L.grid = o;  if (grid) o += ((W + 2 * kPad) * (H + 2 * kPad) + 15) & ~15;
     L.hist = o;  o += 4 * n_action * tile;   // u32 [bin][thread], then f32 [thread][bin] rows
     L.total = o;
     return L;
 }
 
+//
+// REC_HBM (maps whose u8 grid does not fit beside the histogram): no grid is built.  The observation record's padded
+// grid already holds every alive listed agent as kind << 14 | slot (kind 2 + group); a probe counts a cell when the
+// kind is the observer's group and the agent there has acted, its last action read from the state arrays.
+template <bool REC_HBM>
 __global__ void __launch_bounds__(kLocalMaxTile) k_local_mean_action(const __grid_constant__ LocalMeanIO io, const BattleState S) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    const LocalMeanSmem L = local_mean_smem_layout(io.W, io.H, io.tile, io.n_action);
+    const LocalMeanSmem L = local_mean_smem_layout(io.W, io.H, io.tile, io.n_action, !REC_HBM);
     uint8_t *s_grid = smem_raw + L.grid;
     uint32_t *s_hist = (uint32_t *)(smem_raw + L.hist);
     float *s_stage = (float *)(smem_raw + L.hist);
@@ -1101,14 +1177,17 @@ __global__ void __launch_bounds__(kLocalMaxTile) k_local_mean_action(const __gri
     const size_t base = ((size_t)e * kGroups + g) * cap;
     const int n = S.num[e * kGroups + g];
 
-    for (int c = tid; c < (L.hist - L.grid) / 16; c += nt) ((uint4 *)s_grid)[c] = make_uint4(0u, 0u, 0u, 0u);
+    if constexpr (!REC_HBM)
+        for (int c = tid; c < (L.hist - L.grid) / 16; c += nt) ((uint4 *)s_grid)[c] = make_uint4(0u, 0u, 0u, 0u);
     for (int b = 0; b < n_action; b++) s_hist[b * nt + tid] = 0u;
-    __syncthreads();
-    for (int s = tid; s < n; s += nt) {
-        const uint32_t st = S.state[base + s], a = st_act(st);
-        if (!st_dead(st) && a < (uint32_t)n_action) {
-            const int p = S.pos[base + s];
-            s_grid[(pos_y(p) + kPad) * PW + pos_x(p) + kPad] = (uint8_t)(a + 1);
+    if constexpr (!REC_HBM) {
+        __syncthreads();
+        for (int s = tid; s < n; s += nt) {
+            const uint32_t st = S.state[base + s], a = st_act(st);
+            if (!st_dead(st) && a < (uint32_t)n_action) {
+                const int p = S.pos[base + s];
+                s_grid[(pos_y(p) + kPad) * PW + pos_x(p) + kPad] = (uint8_t)(a + 1);
+            }
         }
     }
     __syncthreads();
@@ -1117,6 +1196,31 @@ __global__ void __launch_bounds__(kLocalMaxTile) k_local_mean_action(const __gri
     uint32_t *h = s_hist + tid;                           // h[b * nt] = bin b of this thread
     if (i < n) {
         const int p = S.pos[base + i];
+        if constexpr (REC_HBM) {
+            const ObsRecord R = obs_record_layout(io.W, io.H, cap);
+            const uint16_t *c = (const uint16_t *)(S.obs_record + (size_t)e * R.total) + (pos_y(p) + kPad) * PW + pos_x(p) + kPad;
+            const uint32_t kind = 2u + (uint32_t)g;
+            const uint32_t *st_env = S.state + (size_t)e * kGroups * cap;   // record slots index [2][cap]
+            auto bin = [&](uint32_t code) -> uint32_t {   // last action + 1 of a same-group agent that acted, else 0
+                if ((code >> 14) != kind) return 0u;
+                const uint32_t a = st_act(st_env[code & 0x3FFFu]);
+                return a < (uint32_t)n_action ? a + 1 : 0u;
+            };
+            for (int k = 0; k < io.n_offsets; k += 8) {
+                uint32_t v[8];
+#pragma unroll
+                for (int u = 0; u < 8; u++) v[u] = k + u < io.n_offsets ? __ldg(c + io.delta[k + u]) : 0u;
+#pragma unroll
+                for (int u = 0; u < 8; u++) v[u] = bin(v[u]);
+#pragma unroll
+                for (int u = 0; u < 8; u++)
+                    if (v[u]) atomicAdd(h + (v[u] - 1) * nt, 1u);
+            }
+            if (st_dead(S.state[base + i])) {
+                const uint32_t v = bin(__ldg(c));
+                if (v) atomicAdd(h + (v - 1) * nt, 1u);
+            }
+        } else {
         const uint8_t *c = s_grid + (pos_y(p) + kPad) * PW + pos_x(p) + kPad;
         for (int k = 0; k < io.n_offsets; k += 8) {
             uint32_t v[8];
@@ -1129,6 +1233,7 @@ __global__ void __launch_bounds__(kLocalMaxTile) k_local_mean_action(const __gri
         if (st_dead(S.state[base + i])) {
             const uint32_t v = c[0];
             if (v) atomicAdd(h + (v - 1) * nt, 1u);
+        }
         }
     }
     uint32_t cnt[kLocalBins], total = 0;

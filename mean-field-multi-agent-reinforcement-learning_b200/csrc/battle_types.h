@@ -17,7 +17,8 @@
 //
 // The occupancy grid (Map::slots / channel_ids, Map.h:72-74) is NOT stored: every kernel rebuilds it
 // in shared memory from walls + the alive agents, so there is a single source of truth and
-// clear_dead never has to patch a map.
+// clear_dead never has to patch a map.  (Geometries whose working set exceeds a CTA's shared memory
+// rebuild it in a per-env HBM workspace instead: Engine::hbm_kernels.)
 #pragma once
 #include <stdint.h>
 
@@ -63,7 +64,8 @@ struct BattleParams {
     int tmpl_stride;        // 0: one placement template for every env; 4*cap: a template per env (add_agents_per_env)
     int random_sides;       // auto-reset: each env draws (Philox, keyed by env and episode) whether the two armies swap
                             // their starting blocks, as generate_map does per round (senario_battle.py:14)
-    int obs_cached;         // k_obs starts an item from the per-env observation record (large groups) instead of the agent arrays
+    int obs_cached;         // k_obs starts an item from the per-env observation record (large groups, and every geometry
+                            // whose kernels run from HBM) instead of the agent arrays
     int move_bands;         // 0, or the reference's NUM_SEP_BUFFER when W*H > 99*99 ("large map mode", GridWorld.cc:79-88):
     int band_width;         //   moves run x-band by x-band, then the band-boundary buffer (GridWorld.cc:443-463,662-672)
     uint32_t seed;
@@ -83,7 +85,8 @@ struct BattleState {   // device pointers
     uint8_t *walls;
     uint16_t *grid_template;           // [(H+12)*(W+12)] padded occupancy grid holding only the walls (kind << 14)
     uint8_t *mini_lut;                 // [W] x / scale_w, then [H] (y / scale_h) * view: minimap cell of a position
-    unsigned char *obs_record;         // [E][obs_record_layout().total] when obs_cached (battle_kernels.cuh)
+    unsigned char *obs_record;         // [E][obs_record_layout().total] when obs_cached (battle_kernels.cuh), followed by
+                                       // k_step's workspace [E][step_smem_layout().total] when k_step runs from HBM
     unsigned long long *agent_steps;   // [E] running count of agents taken through a step (statistic)
     int32_t *obs_ticket;               // [2] of this launch (ring of kObsTicketRing pairs): next item, CTAs finished (rewound by the last CTA)
     // episode template for auto-reset

@@ -97,6 +97,10 @@ struct Engine::LateRecords {
 // ---------------------------------------------------------------------------------------------
 static int round_up(int v, int m) { return (v + m - 1) / m * m; }
 
+// dynamic shared memory a CTA may use; a kernel whose layout for the engine's geometry needs more runs from HBM
+constexpr int kSmemLimit = 227 * 1024;
+static int local_mean_tile(int cap) { return std::min(kLocalMaxTile, round_up(cap, 32)); }
+
 // cudaFuncAttributeMaxDynamicSharedMemorySize is a per-function, per-device setting shared by every engine of the
 // process: it is only ever RAISED, so that an engine of a small geometry cannot pull it below what a larger engine
 // (created earlier, launching later) still needs.
@@ -106,7 +110,7 @@ static void raise_dynamic_smem(const void *func, int bytes, int device) {
     std::lock_guard<std::mutex> lock(mu);
     int &cur = granted[std::make_pair(func, device)];
     if (bytes <= cur) return;
-    if (bytes > 227 * 1024)
+    if (bytes > kSmemLimit)
         throw Fatal("geometry needs " + std::to_string(bytes) + " B of shared memory per CTA (limit 232448): map or capacity too large");
     MF_CUDA(cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
     // the same L1 / shared-memory split for k_obs and k_step: the two kernels alternate every step (and overlap on two
@@ -152,6 +156,7 @@ Engine::Engine(const EngineConfig &cfg) : cfg_(cfg) {
         const char *env = getenv("MFMARL_OBS_CACHED");
         const int want = cfg.obs_cached >= 0 ? cfg.obs_cached : (env ? atoi(env) : -1);
         P_.obs_cached = want >= 0 ? (want != 0) : (round_up(cfg.capacity, 4) >= 256);
+        obs_cached_off_ = want == 0;
     }
     P_.move_bands = 0; P_.band_width = cfg.width;
     if (cfg.width * cfg.height > 99 * 99) {                       // GridWorld.cc:79-88 "large_map_mode"
@@ -188,6 +193,8 @@ Engine::Engine(const EngineConfig &cfg) : cfg_(cfg) {
             P_.obs_cell[slot] = (uint8_t)c;
         }
     }
+
+    require_obs_record(std::max(4, round_up(cfg.capacity, 4)));   // (refuses before anything is allocated)
 
     // cap-independent per-env arrays
     const size_t E = (size_t)P_.E;
@@ -242,8 +249,36 @@ size_t Engine::grid_template_bytes() const {
     return (cells * 2 + 15) / 16 * 16;
 }
 
+// A geometry at which k_step or k_obs cannot keep its grid in shared memory runs them from HBM, and those variants read
+// (k_obs) or build (k_step) the observation record: switch it on, or refuse an explicit "off".
+void Engine::require_obs_record(int cap) {
+    if (P_.obs_cached) return;
+    const int W = P_.W, H = P_.H;
+    const bool big = step_smem_layout(W, H, cap, 0).total > kSmemLimit || obs_smem_layout(W, H, cap, 0).total > kSmemLimit ||
+                     local_mean_smem_layout(W, H, local_mean_tile(cap), n_action()).total > kSmemLimit;
+    if (!big) return;
+    if (obs_cached_off_)
+        throw Fatal("observation record switched off (obs_record = 0 or MFMARL_OBS_CACHED=0), but a " + std::to_string(W) +
+                    "x" + std::to_string(H) + " map with capacity " + std::to_string(cap) +
+                    " does not fit in shared memory: its kernels run from HBM and read the observation record there; "
+                    "leave obs_record at -1 (auto) or 1");
+    P_.obs_cached = 1;
+}
+
+int Engine::hbm_kernels() const {
+    const int W = P_.W, H = P_.H, cap = P_.cap;
+    int m = 0;
+    if (step_smem_layout(W, H, cap, P_.obs_cached).total > kSmemLimit) m |= HBM_STEP;
+    // (one choice for fp32 and bf16 rows: the fp32 layout is the larger)
+    if (P_.obs_cached && obs_smem_layout(W, H, cap, 1).total > kSmemLimit) m |= HBM_OBS;
+    if (P_.obs_cached && obs_record_layout(W, H, cap).hp10 + 4 * 2 * kViewCells > kSmemLimit) m |= HBM_RECORD;
+    if (local_mean_smem_layout(W, H, local_mean_tile(cap), n_action()).total > kSmemLimit) m |= HBM_LOCAL_MEAN;
+    return m;
+}
+
 void Engine::alloc_state(int cap) {
     if (2 * cap > 0x3FFF) throw Fatal("capacity too large for the 14-bit slot field of the occupancy grid");
+    require_obs_record(cap);
     P_.cap = cap;
     const size_t n = slots();
     MF_CUDA(cudaMalloc(&S_.pos, n * 4)); MF_CUDA(cudaMalloc(&S_.hp, n * 4));
@@ -251,9 +286,10 @@ void Engine::alloc_state(int cap) {
     MF_CUDA(cudaMalloc(&S_.next_rew, n * 4)); MF_CUDA(cudaMalloc(&S_.last_rew, n * 4));
     MF_CUDA(cudaMalloc(&S_.init_pos, (size_t)P_.E * 4 * cap * 4));     // room for a template per env
     S_.obs_record = nullptr;
-    if (P_.obs_cached) {
+    if (P_.obs_cached) {   // (hbm_kernels() & HBM_STEP implies obs_cached: require_obs_record)
         const size_t bytes = (size_t)P_.E * obs_record_layout(P_.W, P_.H, cap).total;
-        MF_CUDA(cudaMalloc(&S_.obs_record, bytes));
+        const size_t ws = (hbm_kernels() & HBM_STEP) ? (size_t)P_.E * step_smem_layout(P_.W, P_.H, cap, 1).total : 0;
+        MF_CUDA(cudaMalloc(&S_.obs_record, bytes + ws));
         MF_CUDA(cudaMemset(S_.obs_record, 0, bytes));
     }
     MF_CUDA(cudaMemset(S_.pos, 0, n * 4)); MF_CUDA(cudaMemset(S_.hp, 0, n * 4));
@@ -420,9 +456,13 @@ void Engine::restore_state(const int32_t *pos, const int32_t *id, const uint32_t
 
 void Engine::rebuild_obs_records(cudaStream_t st) {
     if (!P_.obs_cached) return;
-    const int smem = obs_record_layout(P_.W, P_.H, P_.cap).hp10 + 4 * 2 * kViewCells;
-    raise_dynamic_smem((const void *)k_obs_record, smem, device_);
-    k_obs_record<<<P_.E, 256, smem, st>>>(P_, S_);
+    if (hbm_kernels() & HBM_RECORD) {
+        k_obs_record<true><<<P_.E, 256, 4 * 2 * kViewCells, st>>>(P_, S_);
+    } else {
+        const int smem = obs_record_layout(P_.W, P_.H, P_.cap).hp10 + 4 * 2 * kViewCells;
+        raise_dynamic_smem((const void *)k_obs_record<false>, smem, device_);
+        k_obs_record<false><<<P_.E, 256, smem, st>>>(P_, S_);
+    }
     MF_CUDA(cudaGetLastError());
 }
 
@@ -519,8 +559,11 @@ void Engine::observe_groups(float *const d_view[kGroups], float *const d_feature
     }
     io.env_stride = env_stride; io.group_mask = group_mask;
     io.debug = obs_debug_;
-    const ObsSmem L = obs_smem_layout(P_.W, P_.H, P_.cap, P_.obs_cached, bf16);
+    const int hbm = hbm_kernels();
+    const bool rec_hbm = hbm & HBM_OBS;
+    const ObsSmem L = obs_smem_layout(P_.W, P_.H, P_.cap, rec_hbm ? 2 : P_.obs_cached, bf16);
     void (*kern)(const BattleParams, const BattleState, const ObsIO) =
+        rec_hbm ? (bf16 ? k_obs<true, true, true> : k_obs<true, false, true>) :
         P_.obs_cached ? (bf16 ? k_obs<true, true> : k_obs<true, false>) : (bf16 ? k_obs<false, true> : k_obs<false, false>);
     raise_dynamic_smem((const void *)kern, L.total, device_);
     int &ctas_per_sm = obs_ctas_per_sm_[bf16 ? 1 : 0];
@@ -535,7 +578,7 @@ void Engine::observe_groups(float *const d_view[kGroups], float *const d_feature
     // k_obs CTA to EXIT -- and persistent CTAs all exit at the end.  Leaving one k_obs slot free per expected k_step CTA
     // lets the two kernels really overlap: C4 on two streams 1.07e9 -> 1.16e9 agent-steps/s (profiles/r02).
     if (cfg_.concurrent_step_envs > 0) {
-        const int step_smem = step_smem_layout(P_.W, P_.H, P_.cap, P_.obs_cached).total + 1024;
+        const int step_smem = ((hbm & HBM_STEP) ? kStepHbmSmem : step_smem_layout(P_.W, P_.H, P_.cap, P_.obs_cached).total) + 1024;
         const int sm_smem = 227 * 1024, obs_smem = L.total + 1024;
         const int fit_beside_full = (sm_smem - ctas_per_sm * obs_smem) / step_smem;
         if (fit_beside_full < 1 && ctas_per_sm > 1) {
@@ -574,13 +617,18 @@ void Engine::observe_groups(float *const d_view[kGroups], float *const d_feature
 
 void Engine::step(const StepIO &io, cudaStream_t st) {
     commit(st);
+    const bool hbm = hbm_kernels() & HBM_STEP;
     const StepSmem L = step_smem_layout(P_.W, P_.H, P_.cap, P_.obs_cached);
-    raise_dynamic_smem((const void *)k_step, L.total, device_);
+    if (!hbm) raise_dynamic_smem((const void *)k_step<false>, L.total, device_);
     int threads = cfg_.step_threads > 0 ? cfg_.step_threads : std::min(1024, std::max(64, P_.cap));
     // a few environments cannot fill the GPU anyway: wider CTAs shorten the parallel phases (grid load, lists, scans)
     if (cfg_.step_threads <= 0 && P_.E <= n_sm_ / 2) threads = std::max(threads, 256);
     threads = round_up(threads, 32);
-    k_step<<<P_.E, threads, L.total, st>>>(P_, S_, io);
+    if (hbm) {
+        k_step<true><<<P_.E, threads, kStepHbmSmem, st>>>(P_, S_, io);
+    } else {
+        k_step<false><<<P_.E, threads, L.total, st>>>(P_, S_, io);
+    }
     MF_CUDA(cudaGetLastError());
     if (io.phases & (PH_STEP | PH_CLEAR | PH_SETACT)) stepped_ = true;
 }
@@ -622,16 +670,21 @@ void Engine::local_mean_action(double radius, float *const out[kGroups], cudaStr
     }
     LocalMeanIO io = it->second;
     io.W = P_.W; io.H = P_.H; io.cap = P_.cap; io.n_action = n_action();
-    io.tile = std::min(kLocalMaxTile, round_up(P_.cap, 32));
+    io.tile = local_mean_tile(P_.cap);
     int ng = 0;
     for (int g = 0; g < kGroups; g++) {
         io.out[g] = out[g];
         if ((group_mask >> g) & 1) io.group[ng++] = g;
     }
-    const LocalMeanSmem L = local_mean_smem_layout(P_.W, P_.H, io.tile, io.n_action);
-    raise_dynamic_smem((const void *)k_local_mean_action, L.total, device_);
     const dim3 grid((unsigned)P_.E, (unsigned)((P_.cap + io.tile - 1) / io.tile), (unsigned)ng);
-    k_local_mean_action<<<grid, io.tile, L.total, st>>>(io, S_);
+    if (hbm_kernels() & HBM_LOCAL_MEAN) {   // probes the observation record's grid (always kept at such geometries)
+        if (!P_.obs_cached) throw Fatal("local_mean_action: a map this large needs the observation record");
+        k_local_mean_action<true><<<grid, io.tile, local_mean_smem_layout(P_.W, P_.H, io.tile, io.n_action, false).total, st>>>(io, S_);
+    } else {
+        const LocalMeanSmem L = local_mean_smem_layout(P_.W, P_.H, io.tile, io.n_action);
+        raise_dynamic_smem((const void *)k_local_mean_action<false>, L.total, device_);
+        k_local_mean_action<false><<<grid, io.tile, L.total, st>>>(io, S_);
+    }
     MF_CUDA(cudaGetLastError());
 }
 

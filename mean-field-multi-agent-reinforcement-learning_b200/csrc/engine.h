@@ -49,7 +49,8 @@ struct EngineConfig {
     int concurrent_step_envs = 0 /* envs of a sibling engine whose k_step runs (on another stream) while this engine's
                                     k_obs streams: k_obs then leaves SM slots free for it where the two do not fit together */;
     int random_sides = 0 /* auto-reset draws per env and episode whether the armies swap their starting blocks */;
-    int obs_cached = -1 /* observation record: -1 auto (capacity >= 256, or MFMARL_OBS_CACHED), 0 off, 1 on */;
+    int obs_cached = -1 /* observation record: -1 auto (capacity >= 256, or MFMARL_OBS_CACHED), 0 off, 1 on; always on
+                           where the kernels run from HBM (0 is refused there) */;
     unsigned seed = 0;
     AgentTypeParams type;
     float attack_bonus[kGroups] = {0.2f, 0.2f};
@@ -115,6 +116,10 @@ public:
     const CircleRange &view_range() const { return view_; }
     const CircleRange &attack_range() const { return attack_; }
     const CircleRange &move_range() const { return move_; }
+    // kernels whose shared-memory layout for the current geometry (map, capacity) exceeds a CTA's shared memory, so
+    // they run from HBM instead: a mask of HBM_* (mfb_query "hbm_kernels")
+    enum { HBM_STEP = 1, HBM_OBS = 2, HBM_RECORD = 4, HBM_LOCAL_MEAN = 8 };
+    int hbm_kernels() const;
 
 private:
     void alloc_state(int cap);
@@ -124,6 +129,7 @@ private:
     void late_add_sync_down();   // E == 1 only: device state -> host records
     void late_add_sync_up();
     void rebuild_obs_records(cudaStream_t st);   // observation records of every env from the state arrays (obs_cached)
+    void require_obs_record(int cap);            // geometries that run from HBM: record on, or refuse a forced "off"
 
     struct LateRecords;                    // scratch of one late add_agents call (E == 1)
     std::unique_ptr<LateRecords> late_;
@@ -140,6 +146,7 @@ private:
     int obs_grid_limit_ = 0;               // MFMARL_OBS_GRID: cap on k_obs CTAs (leaves SM slots to a concurrent k_step)
     int obs_debug_ = 0;                    // MFMARL_OBS_DEBUG at construction (profiling experiments only)
     std::map<float, LocalMeanIO> local_discs_;   // K7 disc tables by radius (n_offsets, delta filled)
+    bool obs_cached_off_ = false;          // the record was switched off explicitly (config or MFMARL_OBS_CACHED=0)
 
     // host-side placement template (what add_agents has built since the last reset)
     std::vector<unsigned char> h_walls_;          // [H*W]
