@@ -69,6 +69,7 @@ int mfb_add_agents_per_env(mfb_engine *eng, int group, int n, const int *xs, con
 int mfb_set_seed(mfb_engine *eng, unsigned long seed);
 
 /* sizes: key in {"capacity","n_envs","n_action","view_size","n_channel","feature_size","attack_base"}.
+ * "state_bytes": R, the size of one env's state record (mfb_save_envs; depends on the capacity only).
  * "hbm_kernels": the kernels that run from HBM at the engine's geometry (map, capacity after the pending placement)
  * because their shared-memory layout exceeds a CTA's: bit 0 k_step, 1 k_obs, 2 k_obs_record, 3 k_local_mean_action. */
 int mfb_query(mfb_engine *eng, const char *key, int *out);
@@ -125,7 +126,8 @@ int mfb_local_mean_action(mfb_engine *eng, double radius, float *d_out0, float *
  *   "num" int32[E][2], "dead_ct" int32[E][2], "pos" int32[E][2][cap][2], "hp" float[E][2][cap],
  *   "id" int32[E][2][cap], "alive" uint8[E][2][cap], "last_action" int32[E][2][cap],
  *   "step_ct" int32[E], "rng" uint32[E], "agent_steps" uint64[E] (agents stepped since creation),
- *   "side" int32[E] (1 = armies swapped this episode, random_sides), "episode" int32[E]              */
+ *   "side" int32[E] (1 = armies swapped this episode, random_sides), "episode" int32[E],
+ *   "walls" uint8[H][W] (1 = obstacle: the border ring and add_walls; the engine's, not per env)     */
 int mfb_get(mfb_engine *eng, const char *key, void *host_buf, void *stream);
 /* device pointer to the live int32[E][2] agent counts (for masking on the device) */
 int mfb_num_device_ptr(mfb_engine *eng, const int32_t **out);
@@ -135,6 +137,47 @@ int mfb_num_device_ptr(mfb_engine *eng, const int32_t **out);
  * mfb_get): "num" int32[E][2], "id" int32[E][2][cap], "pos" int32[E][2][cap] (x | y << 16),
  * "hp" float[E][2][cap], "step_ct" int32[E] */
 int mfb_state_device_ptr(mfb_engine *eng, const char *key, const void **out);
+
+/* ---- Save, restore and fork environments ------------------------------------------------------------------
+ * Each env is saved as one record of R bytes (mfb_query "state_bytes"; R = 96 + 64 * cap, a multiple of 16), all
+ * 32-bit words little-endian:
+ *   bytes  0..31   magic 0x5342464D ("MFBS"), format version 1, W, H, cap, n_action, embedding_size, 0
+ *   bytes 32..39   uint64 FNV-1a hash of the engine's H*W wall bytes ("walls"), taken when the placement is committed
+ *   bytes 40..95   num[2], dead_ct[2], rng (minstd state), step_ct, id_counter, side, episode, init_num[2], 0, 0, 0
+ *   bytes 96..     eight [2][cap] slices, raw (rows at or past num included, so a record round-trips byte for byte):
+ *                  pos (x | y << 16), hp (f32), id, state (dead | last_op << 8 | last_action << 16), next_rew (f32),
+ *                  last_rew (f32), then the env's placement template: pos, id (the shared template where the engine
+ *                  has one) -- what auto-reset re-places the env from
+ * Not in a record: agent_steps (an engine statistic), the observation record and k_step's HBM workspace (derived from
+ * the state, rebuilt on load), the walls (the engine's; identified by the hash) and the engine config (agent type,
+ * rewards, seed, rng_mode, env_base, max_steps, random_sides).  An exact continuation needs an engine created with the
+ * same config.
+ *   envs   HOST int32[n] env indices, or NULL = all n_envs in order (then n must equal n_envs)
+ *   d_out / d_in   DEVICE [n][R], 16-byte aligned
+ * mfb_save_envs commits a pending placement first (as mfb_get does), then is asynchronous on `stream`; repeated indices
+ * are allowed.  A save or load with an index list copies it to an engine-owned device buffer; that copy is ordered on
+ * `stream` after the previous call that used the buffer, on whatever stream (the host does not wait).
+ * mfb_load_envs validates before it writes anything.  On the host: n in [1, n_envs], indices in range and not repeated,
+ * buffers not NULL.  On the device, k_state_check checks every record: magic and version; W, H, cap, n_action equal
+ * to the engine's (a record of another capacity needs an engine created with that capacity); the wall hash; num,
+ * dead_ct and init_num in [0, cap]; every listed agent position (slots < num) and template position (< init_num) on
+ * the map; last_action <= n_action.  Reading its verdicts back is the one synchronisation of a load (of `stream`).  A
+ * bad record returns -1 with "mfb_load_envs: record k: <reason>" and leaves the engine unchanged; otherwise
+ * k_load_envs writes the envs.  After a load:
+ *   - an engine with one shared template whose template differs from a loaded one's moves to one template per env
+ *     (as mfb_add_agents_per_env does), so auto-reset re-places every loaded env from its record's template;
+ *   - the engine counts as stepped: mfb_add_agents follows the after-step rules, mfb_reset discards everything;
+ *   - the observation record is rebuilt where the engine keeps one.
+ * RNG: the random_sides draw at auto-reset is Philox keyed by the global env id env_base + e in EVERY rng_mode.
+ *   - MFB_RNG_MINSTD: the attack shuffle's stream state travels in the record.  Without random_sides a loaded env
+ *     continues exactly as its source would have, at any index.  With random_sides it does so at any index only up to
+ *     its next auto-reset; from there on, at another global id, it draws its own side.
+ *   - MFB_RNG_PHILOX: the attack shuffle is keyed by env_base + e too, so at another global id a loaded env draws its
+ *     own attack orders from the first step.
+ * At the source's global id a loaded env reproduces its source exactly in both modes (create the engine with a
+ * matching env_base to replay any env). */
+int mfb_save_envs(mfb_engine *eng, int n, const int32_t *envs, void *d_out /* device [n][R] */, void *stream);
+int mfb_load_envs(mfb_engine *eng, int n, const int32_t *envs, const void *d_in /* device [n][R] */, void *stream);
 
 /* Host-buffer convenience used for the end-to-end measurement: pinned-host actions in, results out.
  * Copies h_actions -> device, runs mfb_step (clear_dead = 1), copies the results back, synchronises. */

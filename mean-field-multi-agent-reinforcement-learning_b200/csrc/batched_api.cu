@@ -220,6 +220,7 @@ int mfb_query(mfb_engine *h, const char *key, int *out) {
     else if (k == "feature_size") *out = e.params().feature_size;
     else if (k == "attack_base") *out = e.params().n_move;
     else if (k == "hbm_kernels") *out = e.hbm_kernels();   // 1 k_step, 2 k_obs, 4 k_obs_record, 8 k_local_mean_action
+    else if (k == "state_bytes") *out = (int)e.state_bytes();
     else throw Fatal("mfb_query: unknown key " + k);
     MFB_END("mfb_query")
 }
@@ -305,6 +306,7 @@ int mfb_get(mfb_engine *h, const char *key, void *host_buf, void *stream) {
     else if (k == "episode") copy(S.episode, ne * 4);
     else if (k == "rng") copy(S.rng, ne * 4);
     else if (k == "agent_steps") copy(S.agent_steps, ne * 8);
+    else if (k == "walls") memcpy(host_buf, e.host_walls().data(), e.host_walls().size());
     else if (k == "pos" || k == "alive" || k == "last_action") {
         std::vector<int32_t> tmp(n);
         MF_CUDA(cudaMemcpyAsync(tmp.data(), k == "pos" ? (const void *)S.pos : (const void *)S.state, n * 4,
@@ -322,6 +324,18 @@ int mfb_get(mfb_engine *h, const char *key, void *host_buf, void *stream) {
         }
     } else throw Fatal("mfb_get: unknown key " + k);
     MFB_END("mfb_get")
+}
+
+int mfb_save_envs(mfb_engine *h, int n, const int32_t *envs, void *d_out, void *stream) {
+    MFB_BEGIN
+    E(h).save_envs(n, envs, d_out, (cudaStream_t)stream);
+    MFB_END("mfb_save_envs")
+}
+
+int mfb_load_envs(mfb_engine *h, int n, const int32_t *envs, const void *d_in, void *stream) {
+    MFB_BEGIN
+    E(h).load_envs(n, envs, d_in, (cudaStream_t)stream);
+    MFB_END("mfb_load_envs")
 }
 
 int mfb_num_device_ptr(mfb_engine *h, const int32_t **out) {

@@ -242,6 +242,8 @@ Engine::~Engine() {
     cudaFree(S_.num); cudaFree(S_.dead_ct); cudaFree(S_.rng); cudaFree(S_.step_ct);
     cudaFree(S_.id_counter); cudaFree(S_.walls); cudaFree(S_.init_num); cudaFree(S_.agent_steps); cudaFree(S_.obs_ticket); cudaFree(S_.mini_lut); cudaFree(S_.grid_template);
     cudaFree(S_.side); cudaFree(S_.episode);
+    cudaFree(d_state_io_);
+    if (state_io_done_) cudaEventDestroy(state_io_done_);
 }
 
 size_t Engine::grid_template_bytes() const {
@@ -513,6 +515,8 @@ void Engine::commit(cudaStream_t st) {
     MF_CUDA(cudaMemcpyAsync(S_.init_pos, tmpl.data(), tmpl.size() * 4, cudaMemcpyHostToDevice, st));
     MF_CUDA(cudaMemcpyAsync(S_.init_num, num.data(), num.size() * 4, cudaMemcpyHostToDevice, st));
     MF_CUDA(cudaMemcpyAsync(S_.walls, h_walls_.data(), h_walls_.size(), cudaMemcpyHostToDevice, st));
+    wall_hash_ = 14695981039346656037ull;   // FNV-1a 64
+    for (unsigned char b : h_walls_) wall_hash_ = (wall_hash_ ^ b) * 1099511628211ull;
     // the observation kernel's shared-memory grid starts from this image: walls only, 6-cell empty margin
     std::vector<uint16_t> gtmpl(grid_template_bytes() / 2, 0);
     const int PW = P_.W + 2 * (kView / 2);

@@ -91,6 +91,12 @@ public:
     void restore_state(const int32_t *pos, const int32_t *id, const uint32_t *state, const float *hp, const float *next_rew,
                        const float *last_rew, const int32_t *num, const int32_t *dead_ct, cudaStream_t st);
 
+    // ---- per-env state records (mfmarl_batched.h mfb_save_envs / mfb_load_envs; engine_state.cu) ----
+    size_t state_bytes() const;                  // R: bytes of one env's record at the current capacity
+    // envs: host int32[n] env indices, or null = every env in order (n = E); d_out / d_in: device [n][R], 16-byte aligned
+    void save_envs(int n, const int32_t *envs, void *d_out, cudaStream_t st);   // asynchronous; repeated indices allowed
+    void load_envs(int n, const int32_t *envs, const void *d_in, cudaStream_t st);   // validates every record first (syncs)
+
     // ---- state access ----
     void commit(cudaStream_t st);                // upload a pending placement
     void download_num(cudaStream_t st);          // refresh h_num from the device (syncs)
@@ -130,6 +136,7 @@ private:
     void late_add_sync_up();
     void rebuild_obs_records(cudaStream_t st);   // observation records of every env from the state arrays (obs_cached)
     void require_obs_record(int cap);            // geometries that run from HBM: record on, or refuse a forced "off"
+    const int32_t *upload_targets(int n, const int32_t *envs, const void *buf, bool load, cudaStream_t st);
 
     struct LateRecords;                    // scratch of one late add_agents call (E == 1)
     std::unique_ptr<LateRecords> late_;
@@ -160,6 +167,10 @@ private:
     bool placement_dirty_ = true;
     bool stepped_ = false;                        // a step has run since the last placement upload
     std::vector<int> h_num_;                      // [E][2] mirror, refreshed by download_num
+    unsigned long long wall_hash_ = 0;            // FNV-1a 64 of h_walls_ as last committed (identifies the walls of a record)
+    int32_t *d_state_io_ = nullptr;               // save / load scratch: env indices, then the check kernel's verdicts
+    size_t state_io_words_ = 0;
+    cudaEvent_t state_io_done_ = nullptr;         // the last save / load launch that reads the scratch
 };
 
 // error reporting shared by the two C ABIs

@@ -4,8 +4,8 @@ Thin ctypes layer over build/libmagent.so (C ABI: include/mfmarl_batched.h).  Py
 buffers (device memory, streams); the engine never runs on the CPU.
 """
 from .lib import load_library, LIB_PATH
-from .battle import BatchedGridWorld, mean_action
+from .battle import BatchedGridWorld, decode_env_state, mean_action
 from .ising import IsingMFQ, IsingMetropolis, IsingSwendsenWang
 
-__all__ = ["load_library", "LIB_PATH", "BatchedGridWorld", "mean_action", "IsingMFQ", "IsingMetropolis",
+__all__ = ["load_library", "LIB_PATH", "BatchedGridWorld", "decode_env_state", "mean_action", "IsingMFQ", "IsingMetropolis",
            "IsingSwendsenWang"]

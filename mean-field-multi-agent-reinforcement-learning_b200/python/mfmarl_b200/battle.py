@@ -295,7 +295,8 @@ class BatchedGridWorld:
             "side": ("i4", lambda E, c: (E,)), "episode": ("i4", lambda E, c: (E,))}
 
     def get(self, key):
-        dtype, shape = self._GET[key]
+        """mfb_get: the keys of _GET as numpy arrays, and "walls" uint8[H, W] (1 = obstacle)."""
+        dtype, shape = ("u1", lambda E, c: (self.map_size, self.map_size)) if key == "walls" else self._GET[key]
         buf = np.empty(shape(self.n_envs, self.capacity), dtype=dtype)
         with torch.cuda.device(self.device):
             check(self.lib.mfb_get(self._h, key.encode(), buf.ctypes.data, _stream()))
@@ -303,6 +304,95 @@ class BatchedGridWorld:
 
     def get_num(self):
         return self.get("num")
+
+    # ------------------------------------------------------------ save / restore / fork
+    def _targets(self, envs):
+        if envs is None:
+            return self.n_envs, None
+        envs = np.ascontiguousarray(np.asarray(envs, dtype=np.int32).reshape(-1))
+        return len(envs), envs
+
+    def save_envs(self, envs=None):
+        """-> uint8[n, R] on the engine's device, one state record per listed env (None = every env in order; repeated
+        indices are allowed).  The caller owns the tensor.  Record layout: include/mfmarl_batched.h, decode_env_state."""
+        n, idx = self._targets(envs)
+        out = torch.empty((n, self.query("state_bytes")), dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            check(self.lib.mfb_save_envs(self._h, n, None if idx is None else idx.ctypes.data, _ptr(out), _stream()))
+        return out
+
+    def load_envs(self, states, envs=None):
+        """Writes records (uint8[n, R], on the device or on the CPU, then copied over) into the listed envs (None =
+        every env in order; no index twice).  Every record is validated first: a malformed one raises, and then
+        nothing in the engine has changed.  The engine counts as stepped afterwards."""
+        n, idx = self._targets(envs)
+        states = states.to(self.device).contiguous()
+        assert states.dtype == torch.uint8 and states.dim() == 2, (states.dtype, tuple(states.shape))
+        if states.shape[0] != n:
+            raise ValueError("%d records for %d target envs" % (states.shape[0], n))
+        if states.shape[1] != self.query("state_bytes"):
+            raise ValueError("records of %d bytes; this engine's are %d (capacity %d): create the engine with the "
+                             "records' capacity" % (states.shape[1], self.query("state_bytes"), self.capacity))
+        with torch.cuda.device(self.device):
+            check(self.lib.mfb_load_envs(self._h, n, None if idx is None else idx.ctypes.data, _ptr(states), _stream()))
+
+    def state_dict(self):
+        """Every env's record and the wall map, as CPU tensors (torch.save-able).  Resuming needs an engine created
+        with the same config: see load_state_dict."""
+        records = self.save_envs().cpu()
+        return {"map_size": self.map_size, "capacity": self.capacity, "n_envs": self.n_envs,
+                "walls": torch.from_numpy(self.get("walls")), "records": records}
+
+    def load_state_dict(self, d):
+        """On an engine created with the config of the one that made `d`: reset(), the saved walls, then every
+        env's record.  With the same config, steps continue exactly as the saved engine's would have.  A dict of
+        another geometry raises before anything in the engine changes."""
+        want = (self.map_size, self.capacity, self.n_envs)
+        got = (d["map_size"], d["capacity"], d["n_envs"])
+        if got != want or tuple(d["walls"].shape) != (self.map_size, self.map_size) \
+                or tuple(d["records"].shape) != (self.n_envs, self.query("state_bytes")):
+            raise ValueError("state of a %dx%d map, capacity %d, %d envs: this engine has %dx%d, capacity %d, %d envs "
+                             "(create it with the saved geometry)" % (got[0], got[0], got[1], got[2],
+                                                                      want[0], want[0], want[1], want[2]))
+        self.reset()
+        walls = d["walls"].numpy()
+        ys, xs = np.nonzero(walls)
+        if len(xs):
+            self.add_walls(np.stack([xs, ys], axis=1))
+        self.load_envs(d["records"])
+
+
+_STATE_HEAD = 96                        # bytes before the [2][cap] slices (include/mfmarl_batched.h)
+_STATE_SLICES = ("pos", "hp", "id", "state", "next_rew", "last_rew", "init_pos", "init_id")
+
+
+def decode_env_state(record, cap):
+    """One env's state record (uint8[R], a tensor or an array) -> dict of numpy arrays, named like the mfb_get keys
+    where one exists: header (magic, version, W, H, cap, n_action, embedding_size, wall_hash), num[2], dead_ct[2],
+    rng, step_ct, id_counter, side, episode, init_num[2]; [2, cap] slices hp, id, state (raw), alive, last_action,
+    next_rew, last_rew, init_id; and pos / init_pos as [2, cap, 2] (x, y)."""
+    raw = record.cpu().numpy() if isinstance(record, torch.Tensor) else np.asarray(record)
+    raw = np.ascontiguousarray(raw, dtype=np.uint8).reshape(-1)
+    if len(raw) != _STATE_HEAD + len(_STATE_SLICES) * 8 * cap:
+        raise ValueError("a record of capacity %d has %d bytes, not %d" % (cap, _STATE_HEAD + 64 * cap, len(raw)))
+    w = raw[:_STATE_HEAD].view(np.int32)
+    u = raw[:_STATE_HEAD].view(np.uint32)
+    out = {"magic": u[0], "version": u[1], "W": w[2], "H": w[3], "cap": w[4], "n_action": w[5], "embedding_size": w[6],
+           "wall_hash": raw[32:40].view(np.uint64)[0], "num": w[10:12].copy(), "dead_ct": w[12:14].copy(),
+           "rng": u[14], "step_ct": w[15], "id_counter": w[16], "side": w[17], "episode": w[18],
+           "init_num": w[19:21].copy()}
+    body = raw[_STATE_HEAD:].view(np.int32).reshape(len(_STATE_SLICES), 2, cap)
+    for j, name in enumerate(_STATE_SLICES):
+        out[name] = body[j].copy()
+    for name in ("hp", "next_rew", "last_rew"):
+        out[name] = out[name].view(np.float32)
+    out["state"] = out["state"].view(np.uint32)
+    out["alive"] = (1 - (out["state"] & 1)).astype(np.uint8)
+    out["last_action"] = ((out["state"] >> 16) & 0xFF).astype(np.int32)
+    for name in ("pos", "init_pos"):
+        p = out[name]
+        out[name] = np.stack([p & 0xFFFF, (p >> 16) & 0xFFFF], axis=-1).astype(np.int32)
+    return out
 
 
 def mean_action(actions, num, n_action=21):

@@ -55,6 +55,8 @@ def load_library(path=None):
         "mfb_local_mean_action": [vp, ctypes.c_double, vp, vp, vp],
         "mfb_get": [vp, cp, vp, vp],
         "mfb_num_device_ptr": [vp, ctypes.POINTER(vp)],
+        "mfb_save_envs": [vp, ci, vp, vp, vp],
+        "mfb_load_envs": [vp, ci, vp, vp, vp],
         "mfb_step_host": [vp, vp, vp, vp, vp, vp, vp],
         "mfb_step_host_async": [vp, vp, vp, vp, vp, vp, vp, ctypes.POINTER(ci)],
         "mfb_host_wait": [vp, ci],
