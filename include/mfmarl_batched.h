@@ -179,6 +179,27 @@ int mfb_state_device_ptr(mfb_engine *eng, const char *key, const void **out);
 int mfb_save_envs(mfb_engine *eng, int n, const int32_t *envs, void *d_out /* device [n][R] */, void *stream);
 int mfb_load_envs(mfb_engine *eng, int n, const int32_t *envs, const void *d_in /* device [n][R] */, void *stream);
 
+/* Observation rows rendered from state records (kernel k_render_obs), e.g. for a replay that stores one record per
+ * (env, step) instead of every agent's row.  Row k of the output is bit for bit what mfb_observe_groups writes for slot
+ * `slot` of group `group` when an env of this engine holds record `record`, with the engine's walls: the view disc,
+ * both minimaps (count / num over every listed agent, dead or not; 0 / 0 = 0) with the "+1" self marker, id bits, the
+ * one-hot last action, last_rew, x / W, y / H -- rows of dead but still listed agents included.
+ *   d_records   DEVICE [n_records][R] state records (mfb_save_envs), 16-byte aligned
+ *   d_rows      DEVICE int32[n_rows][3]: (record index, group, slot), 16-byte aligned
+ *   d_view      DEVICE float[n_rows][13][13][7], d_feature float[n_rows][feature_size], 16-byte aligned; exactly these
+ *               rows are written, nothing past row n_rows - 1
+ *   d_bad_rows  DEVICE int32 or NULL: set to the number of rows zeroed by the rules below (no synchronisation)
+ * Input from outside never makes the kernel read or write outside these buffers.  A row comes out all zeros (view and
+ * features) when its record index is not in [0, n_records), its group is not 0 or 1, its slot is not in [0, cap), its
+ * slot is at or past the record's num[group], its own position is off the map, or its record's header does not match
+ * this engine (magic, version, W, H, cap, n_action, wall hash).  Inside a record num is clamped to [0, cap], and listed
+ * agents whose position is off the map are neither drawn nor counted in the minimaps.
+ * A pending placement is committed first (as mfb_save_envs does); then the call is asynchronous on `stream` and changes
+ * no engine state.  Returns -1 ("mfb_render_observations: ...") for n_rows < 0, n_records < 1 with n_rows > 0, a NULL
+ * buffer or one that is not 16-byte aligned, before anything is launched. */
+int mfb_render_observations(mfb_engine *eng, int n_records, const void *d_records, int n_rows, const int32_t *d_rows,
+                            float *d_view, float *d_feature, int32_t *d_bad_rows /* may be NULL */, void *stream);
+
 /* Host-buffer convenience used for the end-to-end measurement: pinned-host actions in, results out.
  * Copies h_actions -> device, runs mfb_step (clear_dead = 1), copies the results back, synchronises. */
 int mfb_step_host(mfb_engine *eng, const int32_t *h_actions, float *h_reward, uint8_t *h_alive,

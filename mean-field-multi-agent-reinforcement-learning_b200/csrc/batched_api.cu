@@ -332,6 +332,13 @@ int mfb_save_envs(mfb_engine *h, int n, const int32_t *envs, void *d_out, void *
     MFB_END("mfb_save_envs")
 }
 
+int mfb_render_observations(mfb_engine *h, int n_records, const void *d_records, int n_rows, const int32_t *d_rows,
+                            float *d_view, float *d_feature, int32_t *d_bad_rows, void *stream) {
+    MFB_BEGIN
+    E(h).render_observations(n_records, d_records, n_rows, d_rows, d_view, d_feature, d_bad_rows, (cudaStream_t)stream);
+    MFB_END("mfb_render_observations")
+}
+
 int mfb_load_envs(mfb_engine *h, int n, const int32_t *envs, const void *d_in, void *stream) {
     MFB_BEGIN
     E(h).load_envs(n, envs, d_in, (cudaStream_t)stream);

@@ -96,6 +96,10 @@ public:
     // envs: host int32[n] env indices, or null = every env in order (n = E); d_out / d_in: device [n][R], 16-byte aligned
     void save_envs(int n, const int32_t *envs, void *d_out, cudaStream_t st);   // asynchronous; repeated indices allowed
     void load_envs(int n, const int32_t *envs, const void *d_in, cudaStream_t st);   // validates every record first (syncs)
+    // observation rows of listed (record, group, slot) triples, as k_obs would write them for an env holding the record
+    // (mfb_render_observations); asynchronous, changes no engine state.  d_bad_rows (may be null) receives the rows zeroed
+    void render_observations(int n_records, const void *d_records, int n_rows, const int32_t *d_rows, float *d_view,
+                             float *d_feature, int32_t *d_bad_rows, cudaStream_t st);
 
     // ---- state access ----
     void commit(cudaStream_t st);                // upload a pending placement

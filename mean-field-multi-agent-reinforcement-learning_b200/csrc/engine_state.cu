@@ -3,6 +3,7 @@
 //   k_state_check  validates records before anything is written (one CTA per record)
 //   k_save_envs    gathers listed envs into records                (one CTA per record)
 //   k_load_envs    scatters validated records into listed envs     (one CTA per record)
+//   k_render_obs   observation rows of (record, group, slot) triples (one warp per row; mfb_render_observations)
 //
 // Record of R = 96 + 64 * cap bytes (the layout is documented in include/mfmarl_batched.h):
 //   words 0..23   header and per-env scalars (StateWord below)
@@ -192,6 +193,133 @@ k_load_envs(const __grid_constant__ BattleParams P, const BattleState S, const i
     }
 }
 
+// ---- k_render_obs: observation rows rendered again from state records (mfb_render_observations) ----
+// One warp per output row.  A sampled batch almost never has two rows of one record, so nothing is built per record:
+// the warp scans its record's <= 2 * cap listed agents once, counting the minimaps and drawing the alive ones that fall
+// in its 13 x 13 window into per-warp shared memory, composes the row there one cell per lane, and drains it with
+// 16-byte stores (rows are 4732 B, so row k starts 12 k mod 16 bytes past a 16-byte boundary: a 0-3 float head and
+// tail go out as scalars -- nothing is written past row k, since a gather output has no padding behind its last row).
+// The formulas are k_obs's (battle_kernels.cuh): walls from the engine's padded grid_template, hp / max_hp with
+// __fdiv_rn, count / num with 0 / 0 = 0, the "+1" self marker in both minimap channels, the features of
+// GridWorld.cc:411-421.
+constexpr int kRenderWarps = 4, kRenderThreads = 32 * kRenderWarps;
+constexpr int kRenderStage = kViewRow + 5;   // floats of a warp's staged row: up to 3 of alignment shift, 16-byte multiple
+constexpr int kRenderPad = kView / 2;   // the 6-cell empty margin of grid_template
+
+__global__ void __launch_bounds__(kRenderThreads)
+k_render_obs(const __grid_constant__ BattleParams P, const uint16_t *__restrict__ grid_template,
+             const uint8_t *__restrict__ mini_lut, const unsigned char *__restrict__ records, int n_records,
+             const int32_t *__restrict__ rows, int n_rows, float *__restrict__ view, float *__restrict__ feature,
+             int32_t *__restrict__ bad_rows, unsigned long long wall_hash) {
+    __shared__ __align__(16) float s_row[kRenderWarps][kRenderStage];   // the row, shifted to row k's 16-byte phase
+    __shared__ int s_cnt[kRenderWarps][2 * kViewCells];     // minimap counts, then (in place) count / num as floats
+    __shared__ uint8_t s_kind[kRenderWarps][kViewCells + 7];   // window cell: 0 empty, 1 wall, 2 + group of an alive agent
+    __shared__ float s_hp[kRenderWarps][kViewCells];         // hp / max_hp of that agent
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const size_t k = (size_t)blockIdx.x * kRenderWarps + w;
+    if (k >= (size_t)n_rows) return;                         // (warp-uniform)
+    const int cap = P.cap, W = P.W, H = P.H, FS = P.feature_size, emb = P.embedding_size;
+    const int n_action = P.n_move + P.n_attack;
+    float *const vrow = view + k * kViewRow;
+    float *const frow = feature + k * FS;
+    const int r = rows[3 * k], g = rows[3 * k + 1], slot = rows[3 * k + 2];
+
+    bool ok = (unsigned)r < (unsigned)n_records && (unsigned)g < (unsigned)kGroups && (unsigned)slot < (unsigned)cap;
+    const unsigned char *rec = records + (ok ? (size_t)r * state_record_bytes(cap) : 0);
+    int n0 = 0, n1 = 0;                                      // (scalars: a dynamically indexed array would go to local memory)
+    if (ok) {
+        const uint32_t *h = (const uint32_t *)rec;
+        const unsigned long long hash = (unsigned long long)h[W_HASH_HI] << 32 | h[W_HASH_LO];
+        ok = h[W_MAGIC] == kStateMagic && h[W_VERSION] == kStateVersion && (int)h[W_W] == W && (int)h[W_H] == H &&
+             (int)h[W_CAP] == cap && (int)h[W_NACT] == n_action && hash == wall_hash;
+        n0 = min(max((int)h[W_NUM], 0), cap);
+        n1 = min(max((int)h[W_NUM + 1], 0), cap);
+    }
+    const int32_t *pos = (const int32_t *)(rec + kStateHead);   // slices [2][cap]: 0 pos, 1 hp, 2 id, 3 state, 5 last_rew
+    const float *hp = (const float *)(pos + 2 * cap);
+    const int32_t *id = pos + 4 * cap;
+    const uint32_t *state = (const uint32_t *)(pos + 6 * cap);
+    const float *last_rew = (const float *)(pos + 10 * cap);
+    const int s_self = g * cap + slot;
+    ok = ok && slot < (g ? n1 : n0);
+    const uint32_t p_self = ok ? (uint32_t)pos[s_self] : 0u;
+    ok = ok && on_map(P, p_self);
+    if (!ok) {
+        for (int i = lane; i < kViewRow; i += 32) vrow[i] = 0.0f;
+        for (int i = lane; i < FS; i += 32) frow[i] = 0.0f;
+        if (lane == 0 && bad_rows) atomicAdd(bad_rows, 1);
+        return;
+    }
+    const int ax = (int)(p_self & 0xFFFFu), ay = (int)(p_self >> 16), PW = W + 2 * kRenderPad;
+    int *const cnt = s_cnt[w];
+    uint8_t *const kind = s_kind[w];
+    float *const hpc = s_hp[w];
+    for (int c = lane; c < kViewCells; c += 32) {
+        const int vy = c / kView, vx = c - vy * kView;
+        kind[c] = (uint8_t)(grid_template[(size_t)(ay + vy) * PW + ax + vx] >> 14);   // window corner (ax - 6, ay - 6)
+    }
+    for (int c = lane; c < 2 * kViewCells; c += 32) cnt[c] = 0;
+    __syncwarp();
+    for (int gg = 0; gg < kGroups; gg++) {
+        for (int i = lane; i < (gg ? n1 : n0); i += 32) {
+            const int s = gg * cap + i;
+            const uint32_t q = (uint32_t)pos[s];
+            if (!on_map(P, q)) continue;                          // (only a record from outside: neither drawn nor counted)
+            const int x = (int)(q & 0xFFFFu), y = (int)(q >> 16);
+            atomicAdd(&cnt[gg * kViewCells + mini_lut[W + y] + mini_lut[x]], 1);   // dead or not (GridWorld.cc:359-370)
+            const int dx = x - ax + kRenderPad, dy = y - ay + kRenderPad;
+            if ((unsigned)dx < (unsigned)kView && (unsigned)dy < (unsigned)kView && !(state[s] & 1u)) {
+                kind[dy * kView + dx] = (uint8_t)(2 + gg);
+                hpc[dy * kView + dx] = __fdiv_rn(hp[s], P.hp);   // Map.cc:208
+            }
+        }
+    }
+    __syncwarp();
+    float *const mini = (float *)cnt;
+    for (int c = lane; c < 2 * kViewCells; c += 32) {
+        const int tot = c >= kViewCells ? n1 : n0;
+        mini[c] = tot > 0 ? __fdiv_rn((float)cnt[c], (float)tot) : 0.0f;   // GridWorld.cc:372-377; 0/0 defined as 0
+    }
+    __syncwarp();
+    const float *mini_own = mini + g * kViewCells, *mini_oth = mini + (1 - g) * kViewCells;
+    const uint32_t kind_own = 2u + (uint32_t)g, kind_oth = 3u - (uint32_t)g;
+    const int self_c = mini_lut[W + ay] + mini_lut[ax];
+    // row float j sits at s_row[w][shift + j]: shift + j is a multiple of 4 exactly where vrow + j is 16-byte aligned
+    const int head = (int)((4 - (k * 3) % 4) % 4);            // floats before row k's first 16-byte boundary
+    const int shift = (4 - head) % 4;
+    float *const row = s_row[w] + shift;
+    for (int c = lane; c < kViewCells; c += 32) {              // one cell per lane: stride-7 words, no bank conflicts
+        const uint32_t kd = (P.disc[c >> 5] >> (c & 31)) & 1u ? kind[c] : 0u;   // occupancy only inside the view disc
+        const float h = hpc[c], self = c == self_c ? 1.0f : 0.0f;
+        float *o = row + c * kChan;
+        o[0] = kd == 1u ? 1.0f : 0.0f;
+        o[1] = kd == kind_own ? 1.0f : 0.0f;
+        o[2] = kd == kind_own ? h : 0.0f;
+        o[3] = self != 0.0f ? mini_own[c] + self : mini_own[c];   // self marker in both minimaps (GridWorld.cc:396-408)
+        o[4] = kd == kind_oth ? 1.0f : 0.0f;
+        o[5] = kd == kind_oth ? h : 0.0f;
+        o[6] = self != 0.0f ? mini_oth[c] + self : mini_oth[c];
+    }
+    __syncwarp();
+    if (lane < head) vrow[lane] = row[lane];
+    const int n4 = (kViewRow - head) >> 2;
+    const float4 *src4 = (const float4 *)(row + head);
+    float4 *dst4 = (float4 *)(vrow + head);
+    for (int q = lane; q < n4; q += 32) dst4[q] = src4[q];
+    const int tail = head + 4 * n4;
+    if (lane < kViewRow - tail) vrow[tail + lane] = row[tail + lane];
+    // features (GridWorld.cc:411-421): id bits LSB first, one-hot last action, last reward, x / W, y / H
+    const int my_id = id[s_self], act = (int)((state[s_self] >> 16) & 0xFFu);
+    const float rew = last_rew[s_self];
+    for (int j = lane; j < FS; j += 32) {
+        float v = (j < emb) ? (float)((my_id >> j) & 1) : ((j - emb == act) ? 1.0f : 0.0f);
+        v = j == emb + n_action ? rew : v;
+        v = j == emb + n_action + 1 ? __fdiv_rn((float)ax, (float)W) : v;
+        v = j == emb + n_action + 2 ? __fdiv_rn((float)ay, (float)H) : v;
+        frow[j] = v;
+    }
+}
+
 namespace {
 const char *check_reason(int code) {
     switch (code) {
@@ -251,6 +379,26 @@ void Engine::save_envs(int n, const int32_t *envs, void *d_out, cudaStream_t st)
     k_save_envs<<<n, kStateThreads, 0, st>>>(P_, S_, d_envs, (unsigned char *)d_out, wall_hash_, n_action());
     MF_CUDA(cudaGetLastError());
     if (d_envs) MF_CUDA(cudaEventRecord(state_io_done_, st));
+}
+
+void Engine::render_observations(int n_records, const void *d_records, int n_rows, const int32_t *d_rows, float *d_view,
+                                 float *d_feature, int32_t *d_bad_rows, cudaStream_t st) {
+    if (n_rows < 0) throw Fatal("n_rows = " + std::to_string(n_rows) + " < 0");
+    if (n_rows > 0 && n_records < 1) throw Fatal("n_records = " + std::to_string(n_records) + " < 1 with rows to render");
+    const std::pair<const void *, const char *> bufs[] = {{d_records, "records"}, {d_rows, "rows"}, {d_view, "view"},
+                                                          {d_feature, "feature"}};
+    for (const auto &b : bufs) {
+        if (!b.first) throw Fatal(std::string("null ") + b.second + " buffer");
+        if ((uintptr_t)b.first & 15) throw Fatal(std::string(b.second) + " buffer must be 16-byte aligned");
+    }
+    if ((uintptr_t)d_bad_rows & 3) throw Fatal("bad_rows counter must be 4-byte aligned");
+    commit(st);
+    if (d_bad_rows) MF_CUDA(cudaMemsetAsync(d_bad_rows, 0, 4, st));
+    if (n_rows == 0) return;
+    const unsigned blocks = (unsigned)(((size_t)n_rows + kRenderWarps - 1) / kRenderWarps);
+    k_render_obs<<<blocks, kRenderThreads, 0, st>>>(P_, S_.grid_template, S_.mini_lut, (const unsigned char *)d_records,
+                                                     n_records, d_rows, n_rows, d_view, d_feature, d_bad_rows, wall_hash_);
+    MF_CUDA(cudaGetLastError());
 }
 
 void Engine::load_envs(int n, const int32_t *envs, const void *d_in, cudaStream_t st) {

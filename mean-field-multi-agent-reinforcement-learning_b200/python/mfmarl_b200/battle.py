@@ -312,11 +312,18 @@ class BatchedGridWorld:
         envs = np.ascontiguousarray(np.asarray(envs, dtype=np.int32).reshape(-1))
         return len(envs), envs
 
-    def save_envs(self, envs=None):
+    def save_envs(self, envs=None, out=None):
         """-> uint8[n, R] on the engine's device, one state record per listed env (None = every env in order; repeated
-        indices are allowed).  The caller owns the tensor.  Record layout: include/mfmarl_batched.h, decode_env_state."""
+        indices are allowed).  The caller owns the tensor.  Record layout: include/mfmarl_batched.h, decode_env_state.
+        out: a contiguous, 16-byte aligned uint8[n, R] device tensor to write into (e.g. a slice of a replay's record
+        arena) instead of a new one."""
         n, idx = self._targets(envs)
-        out = torch.empty((n, self.query("state_bytes")), dtype=torch.uint8, device=self.device)
+        R = self.query("state_bytes")
+        if out is None:
+            out = torch.empty((n, R), dtype=torch.uint8, device=self.device)
+        elif out.dtype != torch.uint8 or tuple(out.shape) != (n, R) or not out.is_contiguous() or out.device != self.device:
+            raise ValueError("out must be a contiguous uint8[%d, %d] tensor on %s, not %s[%s] on %s"
+                             % (n, R, self.device, out.dtype, ", ".join(map(str, out.shape)), out.device))
         with torch.cuda.device(self.device):
             check(self.lib.mfb_save_envs(self._h, n, None if idx is None else idx.ctypes.data, _ptr(out), _stream()))
         return out
@@ -335,6 +342,33 @@ class BatchedGridWorld:
                              "records' capacity" % (states.shape[1], self.query("state_bytes"), self.capacity))
         with torch.cuda.device(self.device):
             check(self.lib.mfb_load_envs(self._h, n, None if idx is None else idx.ctypes.data, _ptr(states), _stream()))
+
+    def render_observations(self, records, rows, out=None, bad_rows=None):
+        """Observation rows rendered from state records (mfb_render_observations, kernel k_render_obs).
+        records uint8[n_records, R] and rows int32[n, 3] = (record index, group, slot), both on the engine's device
+        -> (view float32[n, 13, 13, 7], feature float32[n, 34]).  Row k is bit for bit what observe_groups() gives for
+        that slot when an env holds record rows[k, 0].  A row whose reference or record is not valid for this engine
+        comes out all zeros; bad_rows (an int32[1] device tensor, optional) is set to how many did, without a
+        synchronisation.  out: (view, feature) tensors of those shapes to write into.  Asynchronous on the current
+        stream; nothing in the engine changes."""
+        s = self.sizes
+        assert records.dtype == torch.uint8 and records.dim() == 2 and records.is_contiguous(), (records.dtype, records.shape)
+        assert rows.dtype == torch.int32 and rows.dim() == 2 and rows.shape[1] == 3 and rows.is_contiguous(), (rows.dtype, rows.shape)
+        n, v = rows.shape[0], s["view_size"]
+        if out is None:
+            view = torch.empty((n, v, v, s["n_channel"]), dtype=torch.float32, device=self.device)
+            feat = torch.empty((n, s["feature_size"]), dtype=torch.float32, device=self.device)
+        else:
+            view, feat = out
+            assert view.is_contiguous() and feat.is_contiguous() and view.shape[0] >= n and feat.shape[0] >= n
+        if n == 0:
+            if bad_rows is not None:
+                bad_rows.zero_()
+            return view, feat
+        with torch.cuda.device(self.device):
+            check(self.lib.mfb_render_observations(self._h, records.shape[0], _ptr(records), n, _ptr(rows), _ptr(view),
+                                                   _ptr(feat), _ptr(bad_rows), _stream()))
+        return view, feat
 
     def state_dict(self):
         """Every env's record and the wall map, as CPU tensors (torch.save-able).  Resuming needs an engine created

@@ -31,6 +31,10 @@ def battle_parser(description, training):
         ap.add_argument("--mean_field", choices=("group", "local"), default="group",
                         help="mean action of the mean-field learners: 'group' = over the whole group (the reference's), "
                              "'local' = over each agent's group-mates within its view radius (needs --envs)")
+        ap.add_argument("--replay", choices=("rows", "states"), default="rows",
+                        help="with --envs, the Q learners' device replay: 'rows' stores every observation row (4.9 KB "
+                             "each, so only the first envs fit), 'states' stores one env state record per recorded env "
+                             "and step and renders the rows when a batch is sampled (~100 B per row: every env fits)")
     return ap
 
 
@@ -38,6 +42,11 @@ def check_battle_args(ap, args):
     """combinations argparse cannot express; exits with a usage error like argparse itself"""
     if getattr(args, "mean_field", "group") == "local" and args.envs <= 0:
         ap.error("--mean_field local needs the batched engine: pass --envs N (N > 0)")
+    if getattr(args, "replay", "rows") == "states":
+        if args.envs <= 0:
+            ap.error("--replay states needs the batched engine: pass --envs N (N > 0)")
+        if args.algo not in ("mfq", "il"):
+            ap.error("--replay states is for the Q learners (mfq, il); %s keeps whole episodes of rows" % args.algo)
     return args
 
 

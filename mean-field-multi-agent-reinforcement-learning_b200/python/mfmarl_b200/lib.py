@@ -57,6 +57,7 @@ def load_library(path=None):
         "mfb_num_device_ptr": [vp, ctypes.POINTER(vp)],
         "mfb_save_envs": [vp, ci, vp, vp, vp],
         "mfb_load_envs": [vp, ci, vp, vp, vp],
+        "mfb_render_observations": [vp, ci, vp, ci, vp, vp, vp, vp, vp],
         "mfb_step_host": [vp, vp, vp, vp, vp, vp, vp],
         "mfb_step_host_async": [vp, vp, vp, vp, vp, vp, vp, ctypes.POINTER(ci)],
         "mfb_host_wait": [vp, ci],

@@ -112,7 +112,8 @@ def play_batched(env, n_round, max_steps, models, eps=1.0, train=False, print_ev
 
     obs_dtype=torch.bfloat16: the policies act on the engine's bf16 NHWC-8 observation rows (no cast, no padding pass,
     bf16 tensor cores; see algo.base.bf16_rollout_copy); the fp32 rows are still produced for the replay buffer when
-    train=True.
+    train=True, unless the main model's replay keeps state records (replay_kind "states"): then the recorded envs are
+    saved after each observation (`models[0].record_slice`) and their rows are rendered only when sampled.
 
     host_lag: how many steps the host may run ahead of the device before it looks at the "any environment still
     playing" flag (see below); None = 2 on a CUDA device, 0 = ask after every step.
@@ -128,6 +129,7 @@ def play_batched(env, n_round, max_steps, models, eps=1.0, train=False, print_ev
     if mean_field not in ("group", "local"):
         raise ValueError("mean_field must be 'group' or 'local', not %r" % (mean_field,))
     local = mean_field == "local"
+    states = train and getattr(models[0], "replay_kind", "rows") == "states"
     E, cap = env.n_envs, env.capacity
     dev = env.device
     if positions is None:
@@ -172,9 +174,12 @@ def play_batched(env, n_round, max_steps, models, eps=1.0, train=False, print_ev
     while step_ct < max_steps and still_playing():
         if obs_dtype is not None and obs_dtype != torch.float32:
             act_obs = env.observe_groups(dtype=obs_dtype)  # bf16 [E, cap, 13, 13, 8] rows for the policies
-            obs = env.observe_groups(groups=(0,)) if train else act_obs
+            obs = env.observe_groups(groups=(0,)) if train and not states else act_obs
         else:
             obs = act_obs = env.observe_groups()           # per group: view [E, cap, 13, 13, 7], feature [E, cap, 34]
+        if states:                                         # the state k_obs just saw, straight into the replay's arena
+            records = models[0].record_slice(env)
+            env.save_envs(None if records.shape[0] == E else range(records.shape[0]), out=records)
         num.copy_(live_num)
         ids = live_id.clone()                              # rows of this step, before clear_dead compacts them
         valid = (slot[None, None, :] < num[:, :, None]) & active[:, None, None]          # [E, 2, cap]
@@ -190,9 +195,10 @@ def play_batched(env, n_round, max_steps, models, eps=1.0, train=False, print_ev
         actions.masked_fill_(~valid, 0)
         reward, alive, done, mean = env.step(actions, want_mean_action=not local)
         if train:
-            models[0].flush_buffer_batched(state=obs[0], acts=actions[:, 0], rewards=reward[:, 0], alives=alive[:, 0],
-                                           ids=ids[:, 0], prob=local_mean[0] if local else former[:, 0], num=num[:, 0],
-                                           active=active)
+            rows = {"records": records} if states else {"state": obs[0]}
+            models[0].flush_buffer_batched(acts=actions[:, 0], rewards=reward[:, 0], alives=alive[:, 0], ids=ids[:, 0],
+                                           prob=local_mean[0] if local else former[:, 0], num=num[:, 0], active=active,
+                                           **rows)
         if local:
             # the next step's rows; enqueued after the flush above has read this step's on the same stream
             local_mean = env.local_mean_action(radius=mf_radius)

@@ -6,6 +6,9 @@ engine and the PyTorch learners.
                                                          observations, mean actions and replay stay in HBM
     python train_battle.py --algo mfq --envs 1024 --mean_field local
                                                         the same with each agent's neighbourhood mean action
+    python train_battle.py --algo mfq --envs 1024 --replay states
+                                                        the replay keeps env state records and renders the rows it
+                                                         samples: every environment's transitions are recorded
 """
 import os
 import sys
@@ -115,13 +118,15 @@ def main(argv=None):
         env = magent.GridWorld('battle', map_size=args.map_size)
         env.set_render_dir(render_dir)
         handles = env.get_handles()
-    # batched rounds produce envs x agents x steps rows: give the device replay room for up to 2^20 of them (5 GB)
-    device_rows = min(1 << 20, args.envs * cap * args.max_steps) if args.envs > 0 else None
+    # batched rounds produce envs x agents x steps rows: give the device replay room for up to 2^20 of them (5 GB), or
+    # 2^25 where a row is a reference to a state record (~100 B a row, plus the records)
+    max_rows = 1 << 25 if args.replay == "states" else 1 << 20
+    device_rows = min(max_rows, args.envs * cap * args.max_steps) if args.envs > 0 else None
     # ... and scale the Q learners' minibatch with the number of recorded environments, so that a round keeps the
     # reference's number of gradient steps (new rows * 2 / batch, tools.py:352-360) instead of multiplying it
     rec_envs = max(1, min(args.envs, device_rows // (cap * args.max_steps))) if args.envs > 0 else 1
     models = [spawn_ai(args.algo, env, handles[0], args.algo + '-me', args.max_steps, device=args.device,
-                       device_rows=device_rows, batch_size=64 * rec_envs),
+                       device_rows=device_rows, batch_size=64 * rec_envs, replay=args.replay),
               spawn_ai(args.algo, env, handles[1], args.algo + '-opponent', args.max_steps, device=args.device)]
     for m in models:
         m.grad_sync = world > 1
