@@ -34,7 +34,8 @@ typedef struct mfb_config {
     int max_steps;         /* with auto_reset: episode horizon (0 = none)                            */
     int auto_reset;        /* re-place the armies when an episode ends (done or horizon)             */
     int device;            /* CUDA device ordinal, -1 = current                                      */
-    int step_threads;      /* 0 = auto                                                               */
+    int step_threads;      /* threads per k_step CTA: <= 0 = auto; 33..1024, rounded up to a multiple of 32;
+                              1..32 and > 1024 make mfb_create fail with a message naming the value           */
     int obs_tile_agents;   /* agents per observation CTA, 0 = auto: clamp(capacity, 64, 256)         */
     int obs_record;        /* per-env observation record kept by k_step for k_obs: -1 = auto (on for
                               capacity >= 256, and wherever the kernels run from HBM), 0 = off (refused
@@ -71,7 +72,10 @@ int mfb_set_seed(mfb_engine *eng, unsigned long seed);
 /* sizes: key in {"capacity","n_envs","n_action","view_size","n_channel","feature_size","attack_base"}.
  * "state_bytes": R, the size of one env's state record (mfb_save_envs; depends on the capacity only).
  * "hbm_kernels": the kernels that run from HBM at the engine's geometry (map, capacity after the pending placement)
- * because their shared-memory layout exceeds a CTA's: bit 0 k_step, 1 k_obs, 2 k_obs_record, 3 k_local_mean_action. */
+ * because their shared-memory layout exceeds a CTA's: bit 0 k_step, 1 k_obs, 2 k_obs_record, 3 k_local_mean_action.
+ * Launch shape: "step_threads" the CTA width k_step launches with (after the auto rules); "obs_record" 1 if the engine
+ * keeps the observation record, else 0; "obs_tile" and "obs_grid" the agents per work item and the CTAs of the engine's
+ * last observation launch (0 before the first one). */
 int mfb_query(mfb_engine *eng, const char *key, int *out);
 
 /* K1.  d_view float[E][2][cap][13][13][7], d_feature float[E][2][cap][feature_size]; rows >= num are

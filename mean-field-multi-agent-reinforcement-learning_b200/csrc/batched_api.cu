@@ -220,6 +220,10 @@ int mfb_query(mfb_engine *h, const char *key, int *out) {
     else if (k == "feature_size") *out = e.params().feature_size;
     else if (k == "attack_base") *out = e.params().n_move;
     else if (k == "hbm_kernels") *out = e.hbm_kernels();   // 1 k_step, 2 k_obs, 4 k_obs_record, 8 k_local_mean_action
+    else if (k == "step_threads") *out = e.step_threads();   // k_step's CTA width
+    else if (k == "obs_record") *out = e.params().obs_cached;
+    else if (k == "obs_tile") *out = e.last_obs_tile();       // k_obs's tile_agents and grid at the last observe
+    else if (k == "obs_grid") *out = e.last_obs_grid();
     else if (k == "state_bytes") *out = (int)e.state_bytes();
     else throw Fatal("mfb_query: unknown key " + k);
     MFB_END("mfb_query")

@@ -131,6 +131,11 @@ Engine::Engine(const EngineConfig &cfg) : cfg_(cfg) {
 
     if (cfg.n_envs < 1 || cfg.width < 3 || cfg.height < 3 || cfg.width > 4096 || cfg.height > 4096)
         throw Fatal("invalid engine config (n_envs / map size)");
+    // k_step's mean-action export zeroes and writes its [2][32] histogram with threads 0..63: a one-warp CTA would
+    // leave group 1's bins unset; 1024 is the CUDA limit on threads per block
+    if (cfg.step_threads > 1024 || (cfg.step_threads > 0 && cfg.step_threads <= 32))
+        throw Fatal("step_threads = " + std::to_string(cfg.step_threads) +
+                    " unsupported: k_step runs 33 to 1024 threads per CTA (rounded up to a multiple of 32), or <= 0 for auto");
 
     view_ = CircleRange(cfg.type.view_radius, 0.0f, 1);
     attack_ = CircleRange(cfg.type.attack_radius, 0.5f, 1);   // inner radius = width / 2.0f (AgentType.cc:107)
@@ -617,6 +622,15 @@ void Engine::observe_groups(float *const d_view[kGroups], float *const d_feature
     S.obs_ticket += 2 * (obs_launches_++ % kObsTicketRing);
     kern<<<grid, kObsThreads, L.total, st>>>(P_, S, io);
     MF_CUDA(cudaGetLastError());
+    last_obs_tile_ = io.tile_agents;
+    last_obs_grid_ = (int)grid;
+}
+
+int Engine::step_threads() const {
+    int threads = cfg_.step_threads > 0 ? cfg_.step_threads : std::min(1024, std::max(64, P_.cap));
+    // a few environments cannot fill the GPU anyway: wider CTAs shorten the parallel phases (grid load, lists, scans)
+    if (cfg_.step_threads <= 0 && P_.E <= n_sm_ / 2) threads = std::max(threads, 256);
+    return round_up(threads, 32);
 }
 
 void Engine::step(const StepIO &io, cudaStream_t st) {
@@ -624,10 +638,7 @@ void Engine::step(const StepIO &io, cudaStream_t st) {
     const bool hbm = hbm_kernels() & HBM_STEP;
     const StepSmem L = step_smem_layout(P_.W, P_.H, P_.cap, P_.obs_cached);
     if (!hbm) raise_dynamic_smem((const void *)k_step<false>, L.total, device_);
-    int threads = cfg_.step_threads > 0 ? cfg_.step_threads : std::min(1024, std::max(64, P_.cap));
-    // a few environments cannot fill the GPU anyway: wider CTAs shorten the parallel phases (grid load, lists, scans)
-    if (cfg_.step_threads <= 0 && P_.E <= n_sm_ / 2) threads = std::max(threads, 256);
-    threads = round_up(threads, 32);
+    const int threads = step_threads();
     if (hbm) {
         k_step<true><<<P_.E, threads, kStepHbmSmem, st>>>(P_, S_, io);
     } else {

@@ -45,7 +45,7 @@ struct AgentTypeParams {   // the attributes of AgentType.h:21-45 that reach the
 struct EngineConfig {
     int n_envs = 1, width = 40, height = 40, capacity = 64, embedding_size = 10;
     int rng_mode = RNG_MINSTD, max_steps = 0, env_base = 0, device = -1 /* current */;
-    int step_threads = 0 /* auto */, obs_tile_agents = 0 /* auto: clamp(cap, 64, 256); 64 with the observation record */;
+    int step_threads = 0 /* <= 0 auto; else 33..1024, rounded up to a multiple of 32 */, obs_tile_agents = 0 /* auto: clamp(cap, 64, 256); 64 with the observation record */;
     int concurrent_step_envs = 0 /* envs of a sibling engine whose k_step runs (on another stream) while this engine's
                                     k_obs streams: k_obs then leaves SM slots free for it where the two do not fit together */;
     int random_sides = 0 /* auto-reset draws per env and episode whether the armies swap their starting blocks */;
@@ -130,6 +130,10 @@ public:
     // they run from HBM instead: a mask of HBM_* (mfb_query "hbm_kernels")
     enum { HBM_STEP = 1, HBM_OBS = 2, HBM_RECORD = 4, HBM_LOCAL_MEAN = 8 };
     int hbm_kernels() const;
+    // launch shape: k_step's CTA width after the auto rules; k_obs's tile and grid of the last observe (0 before one)
+    int step_threads() const;
+    int last_obs_tile() const { return last_obs_tile_; }
+    int last_obs_grid() const { return last_obs_grid_; }
 
 private:
     void alloc_state(int cap);
@@ -155,6 +159,7 @@ private:
     unsigned obs_launches_ = 0;            // k_obs launches so far (picks the ticket pair)
     int obs_ctas_per_sm_[2] = {2, 2};      // resident k_obs CTAs per SM at that size (occupancy query)
     int obs_grid_limit_ = 0;               // MFMARL_OBS_GRID: cap on k_obs CTAs (leaves SM slots to a concurrent k_step)
+    int last_obs_tile_ = 0, last_obs_grid_ = 0;   // tile_agents and grid of the last k_obs launch
     int obs_debug_ = 0;                    // MFMARL_OBS_DEBUG at construction (profiling experiments only)
     std::map<float, LocalMeanIO> local_discs_;   // K7 disc tables by radius (n_offsets, delta filled)
     bool obs_cached_off_ = false;          // the record was switched off explicitly (config or MFMARL_OBS_CACHED=0)

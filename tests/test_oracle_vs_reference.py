@@ -104,14 +104,20 @@ def test_mean_info_matches():
 
 
 @needs_ref
-@pytest.mark.parametrize("size", [100, 104])
+@pytest.mark.parametrize("size", [100, 104, 1001])
 def test_large_map_mode_moves_run_band_by_band(size):
     """W*H > 99*99 switches the reference to large_map_mode (GridWorld.cc:79-88): moves are filed into x-band
     buffers at set_action (:443-463) and resolved band by band, then the boundary buffer (:662-672) -- a different
-    collision order than plain set_action order.  Dense blocks that straddle several bands, crowded fight stream."""
+    collision order than plain set_action order.  Dense blocks that straddle several bands, crowded fight stream.
+    Above W*H = 10^6 there are 16 bands instead of 8: at 1001 the bands are 63 wide (126 with 8).  There the armies
+    are two strips stacked in y (x 430..499, meeting at y = 493 / 494 next to the centre), so that the moves cross
+    x = 441, a boundary of the 16 bands but not of the 8, and its boundary-buffer cells (x % 63 < 4 or > 59)."""
     from scenarios import block_positions
     ref, ora = RefEngine(size), OracleEngine(size)
-    left, right = block_positions(20, 30, 28, 20, stride=1), block_positions(size - 50, 30, 28, 20, stride=1)
+    if size < 1000:
+        left, right = block_positions(20, 30, 28, 20, stride=1), block_positions(size - 50, 30, 28, 20, stride=1)
+    else:
+        left, right = block_positions(430, 486, 70, 8, stride=1), block_positions(430, 494, 70, 8, stride=1)
     setup_pair([ref, ora], left, right)
     st = run_lockstep(ref, ora, steps=50, seed=size, stream="fight", check_obs_every=10)
     assert st["deaths"] > 20, st
