@@ -65,7 +65,7 @@ int gridworld_add_reward_rule(EnvHandle game, int on, int *receiver, float *valu
  * list in set_action call order) instead of shuffling with the engine RNG (GridWorld.cc:510-515).    */
 int mfmarl_inject_attack_order(EnvHandle game, const int *perm, int n);
 /* Test hook: how many env_step calls of this game were served by replaying the captured CUDA graph of the steady
- * play-loop step (0 with MAGENT_STEP_GRAPH=0); -1 for a null handle.                                             */
+ * play-loop step; -1 for a null handle.                                                                           */
 int mfmarl_step_graph_replays(EnvHandle game);
 const char *mfmarl_last_error(void);
 

@@ -52,9 +52,10 @@ struct Game {
     std::unique_ptr<Engine> eng;
     cudaStream_t st = nullptr;
 
-    // device staging for the host-buffer ABI
-    float *d_view = nullptr, *d_feat = nullptr; int obs_cap = 0;
-    int32_t *d_actions = nullptr, *d_perm = nullptr, *d_done = nullptr; int act_cap = 0;
+    // device staging for the host-buffer ABI, sized for staged_cap agents per group (d_done: one word)
+    float *d_view = nullptr, *d_feat = nullptr;
+    int32_t *d_actions = nullptr, *d_perm = nullptr, *d_events = nullptr, *d_done = nullptr;
+    int staged_cap = 0;
     std::vector<int> seq;          // groups in set_action call order since the last step
     bool inject_next = false;
 
@@ -74,31 +75,32 @@ struct Game {
     //     in the mirror are written back to the device, and the call proceeds as if nothing had been enqueued.
     char *pin = nullptr; int pin_cap = 0;
     struct Mirror { int32_t *pos, *id; uint32_t *state; float *hp, *rew, *lrew; int32_t *head; } mir[2] = {};
-    int cur = 0;                   // mir[cur] is the one the getters read (the aliases below point into it)
-    int32_t *m_pos = nullptr, *m_id = nullptr, *m_actions = nullptr; uint32_t *m_state = nullptr;
-    float *m_hp = nullptr, *m_rew = nullptr, *m_view = nullptr, *m_feat = nullptr;
-    bool state_fresh = false, obs_fresh = false;
+    int cur = 0;                   // mir[cur] is the one the getters read (view())
+    int32_t *m_actions = nullptr;
+    float *m_view = nullptr, *m_feat = nullptr;
     unsigned pending_mask = 0;     // groups whose staged actions have not reached the device yet
     cudaEvent_t ev_step = nullptr, ev_spec = nullptr;
-    bool speculate = true;         // MAGENT_SPECULATE=0 switches it off
-    bool spec_pending = false;     // clear_dead + observe are enqueued behind the last step, not asked for yet
-    bool spec_state = false;       // committed: mir[cur ^ 1] holds the records after clear_dead once ev_spec fires
-    bool spec_obs = false;         // committed: m_view / m_feat hold both groups' rows once ev_spec fires
+
+    // What the host holds of the agent records (state) and of both groups' observation rows (obs).  Fresh: they are in
+    // mir[cur] / m_view, m_feat.  OnEvent: they will be in mir[cur ^ 1] / m_view, m_feat once ev_spec fires.
+    // spec_enqueued: clear_dead + the observations are enqueued behind the last step and not committed yet.
+    // Invariant: spec_enqueued implies state == Fresh && obs == Stale.
+    enum Held { Stale, Fresh, OnEvent };
+    Held state = Stale, obs = Stale;
+    bool spec_enqueued = false;
 
     // The steady play-loop step (set_action x2 + step, then the speculative clear_dead + observe x2 + two copies) is
     // six enqueues, and at one 64 v 64 env the HOST side of those enqueues is what env_step costs.  Once the same
-    // sequence has run twice it is captured into a CUDA graph -- one per (mirror parity, set_action order) -- and
-    // replayed with one launch; the two events become external event-record nodes.  A cached graph is only reused
-    // while every pointer and parameter baked into it is unchanged (the key below); anything else re-captures.
-    // MAGENT_STEP_GRAPH=0 switches it off.
-    struct StepGraph {
-        cudaGraphExec_t exec = nullptr;
-        int into = -1, seq0 = -2, seq1 = -2, setact_mask = -1;
+    // sequence has run twice it is captured into a CUDA graph and replayed with one launch; the two events become
+    // external event-record nodes.  The key holds every value baked into a graph, so a graph is only replayed while
+    // all of them are unchanged, and anything else captures a new one.
+    struct GraphKey {
+        int into, seq0, seq1, setact_mask;
+        const void *pin, *d_view, *d_feat, *d_done, *d_perm;
         BattleParams P; BattleState S;
-        const void *pin = nullptr, *d_view = nullptr, *d_feat = nullptr, *d_done = nullptr, *d_perm = nullptr;
     };
+    struct StepGraph { GraphKey key; cudaGraphExec_t exec; };
     std::vector<StepGraph> graphs;
-    bool use_graphs = true;
     int plain_steps = 0;           // eligible steps enqueued call by call so far (the first two warm every attribute up)
     int graph_replays = 0;         // env_step calls served by a graph launch (mfmarl_step_graph_replays)
 
@@ -106,7 +108,6 @@ struct Game {
     std::string render_dir;
     bool first_render = true;
     int file_ct = 0, frame_ct = 0, frame_per_file = 10000;
-    int32_t *d_events = nullptr; int ev_cap = 0;
     std::vector<int32_t> events;   // (id, x, y) of the last step's attacks, processing order
 
     ~Game() {
@@ -122,25 +123,30 @@ struct Game {
         graphs.clear();
     }
 
-    void invalidate() { state_fresh = false; obs_fresh = false; spec_state = false; spec_obs = false; }
-
-    void use_mirror(int which) {
-        cur = which;
-        m_pos = mir[cur].pos; m_id = mir[cur].id; m_state = mir[cur].state; m_hp = mir[cur].hp; m_rew = mir[cur].rew;
-    }
+    const Mirror &view() const { return mir[cur]; }
     StepMirror mirror_io(int which) const {
         const Mirror &m = mir[which];
         return StepMirror{m.pos, m.id, m.state, m.hp, m.rew, m.lrew, m.head};
     }
 
+    // the host's copies no longer describe the device.  Only env_reset gets here with a speculative step still enqueued
+    // (every other path rolled it back first), and its placement overwrites what ran.
+    void invalidate() { state = Stale; obs = Stale; spec_enqueued = false; }
+
+    // env_step: the step left its records in mir[into]; `enqueued` = clear_dead + observe were enqueued behind it
+    void after_step(int into, bool enqueued) { cur = into; state = Fresh; obs = Stale; spec_enqueued = enqueued; }
+
+    // clear_dead right after a step: what was enqueued behind the step becomes the state once ev_spec fires
+    void commit_spec() { spec_enqueued = false; state = OnEvent; obs = OnEvent; }
+
     // something other than clear_dead followed a step: undo the speculative clear_dead (see above)
     void rollback() {
-        if (!spec_pending) return;
+        if (!spec_enqueued) return;
         MF_CUDA(cudaEventSynchronize(ev_spec));
-        const Mirror &m = mir[cur];                        // the records as the step left them
+        const Mirror &m = view();                          // the records as the step left them
         engine().restore_state(m.pos, m.id, m.state, m.hp, m.rew, m.lrew, m.head, m.head + 2, st);
         MF_CUDA(cudaStreamSynchronize(st));
-        spec_pending = false; obs_fresh = false;
+        spec_enqueued = false; obs = Stale;
     }
 
     void ensure_mirror() {
@@ -164,7 +170,7 @@ struct Game {
         for (int grp = 0; grp < 2 && old_cap > 0; grp++)      // staged actions survive a capacity growth
             memcpy(m_actions + (size_t)grp * cap, keep.data() + (size_t)grp * old_cap, (size_t)old_cap * 4);
         pin_cap = cap;
-        use_mirror(0);
+        cur = 0;
         invalidate();
     }
 
@@ -184,26 +190,26 @@ struct Game {
     void enqueue_state_download() {
         Engine &E = engine();
         const BattleState &S = E.state();
+        const Mirror &m = view();
         const size_t bytes = (size_t)2 * E.cap() * 4;
-        MF_CUDA(cudaMemcpyAsync(m_pos, S.pos, bytes, cudaMemcpyDeviceToHost, st));
-        MF_CUDA(cudaMemcpyAsync(m_id, S.id, bytes, cudaMemcpyDeviceToHost, st));
-        MF_CUDA(cudaMemcpyAsync(m_state, S.state, bytes, cudaMemcpyDeviceToHost, st));
-        MF_CUDA(cudaMemcpyAsync(m_hp, S.hp, bytes, cudaMemcpyDeviceToHost, st));
-        MF_CUDA(cudaMemcpyAsync(m_rew, S.next_rew, bytes, cudaMemcpyDeviceToHost, st));
+        MF_CUDA(cudaMemcpyAsync(m.pos, S.pos, bytes, cudaMemcpyDeviceToHost, st));
+        MF_CUDA(cudaMemcpyAsync(m.id, S.id, bytes, cudaMemcpyDeviceToHost, st));
+        MF_CUDA(cudaMemcpyAsync(m.state, S.state, bytes, cudaMemcpyDeviceToHost, st));
+        MF_CUDA(cudaMemcpyAsync(m.hp, S.hp, bytes, cudaMemcpyDeviceToHost, st));
+        MF_CUDA(cudaMemcpyAsync(m.rew, S.next_rew, bytes, cudaMemcpyDeviceToHost, st));
     }
 
     void fetch_state() {
         flush_actions();
-        if (state_fresh) return;
-        if (spec_state) {                          // the records after clear_dead were written behind the step
+        if (state == Fresh) return;
+        if (state == OnEvent) {                    // the records after clear_dead were written behind the step
             MF_CUDA(cudaEventSynchronize(ev_spec));
-            use_mirror(cur ^ 1);
-            spec_state = false; state_fresh = true;
-            return;
+            cur ^= 1;
+        } else {
+            enqueue_state_download();
+            MF_CUDA(cudaStreamSynchronize(st));
         }
-        enqueue_state_download();
-        MF_CUDA(cudaStreamSynchronize(st));
-        state_fresh = true;
+        state = Fresh;
     }
 
     const TypeDef &type_of(int group) const {
@@ -263,10 +269,6 @@ struct Game {
         MF_CUDA(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
         MF_CUDA(cudaEventCreateWithFlags(&ev_step, cudaEventDisableTiming));
         MF_CUDA(cudaEventCreateWithFlags(&ev_spec, cudaEventDisableTiming));
-        const char *sp = getenv("MAGENT_SPECULATE");
-        speculate = !(sp && atoi(sp) == 0);
-        const char *gr = getenv("MAGENT_STEP_GRAPH");
-        use_graphs = !(gr && atoi(gr) == 0);
     }
 
     void ensure_staging() {
@@ -274,18 +276,15 @@ struct Game {
         if (E.placement_pending()) invalidate();
         E.commit(st);
         const int cap = E.cap();
-        if (obs_cap < cap) {
-            cudaFree(d_view); cudaFree(d_feat);
+        if (staged_cap < cap) {
+            cudaFree(d_view); cudaFree(d_feat); cudaFree(d_actions); cudaFree(d_perm); cudaFree(d_events);
             MF_CUDA(cudaMalloc(&d_view, (size_t)2 * cap * kViewRow * 4 + 64));
             MF_CUDA(cudaMalloc(&d_feat, (size_t)2 * cap * E.params().feature_size * 4));
-            obs_cap = cap;
-        }
-        if (act_cap < cap) {
-            cudaFree(d_actions); cudaFree(d_perm);
             MF_CUDA(cudaMalloc(&d_actions, (size_t)2 * cap * 4));
             MF_CUDA(cudaMalloc(&d_perm, (size_t)2 * cap * 4));
+            MF_CUDA(cudaMalloc(&d_events, (size_t)(1 + 6 * cap) * 4));
             MF_CUDA(cudaMemset(d_actions, 0, (size_t)2 * cap * 4));
-            act_cap = cap;
+            staged_cap = cap;
         }
         if (!d_done) MF_CUDA(cudaMalloc(&d_done, 4));
         ensure_mirror();
@@ -361,7 +360,7 @@ int env_reset(EnvHandle game) {
     g->ensure_engine();
     g->eng->reset();
     g->seq.clear();
-    g->pending_mask = 0; g->invalidate(); g->spec_pending = false;   // (whatever was enqueued is overwritten by the placement)
+    g->pending_mask = 0; g->invalidate();         // (whatever was enqueued behind a step is overwritten by the placement)
     g->file_ct++; g->frame_ct = 0;                        // RenderGenerator::next_file (GridWorld.cc:102)
     API_END("env_reset")
 }
@@ -376,11 +375,11 @@ int env_get_observation(EnvHandle game, GroupHandle group, float **buffer) {
     g->flush_actions();                       // features carry the last action (GridWorld.cc:411-417)
     const int n = E.host_num(0, group), cap = E.cap(), FS = E.params().feature_size;
     if (n == 0) return 0;
-    if (!g->obs_fresh && g->spec_obs) {       // both groups' rows were computed and copied behind the last step
+    if (g->obs == Game::OnEvent) {            // both groups' rows were computed and copied behind the last step
         MF_CUDA(cudaEventSynchronize(g->ev_spec));
-        g->spec_obs = false; g->obs_fresh = true;
+        g->obs = Game::Fresh;
     }
-    if (!g->obs_fresh) {                      // both groups in one launch, one batch of copies, one synchronisation
+    if (g->obs != Game::Fresh) {              // both groups in one launch, one batch of copies, one synchronisation
         const int n0 = E.host_num(0, 0), n1 = E.host_num(0, 1);
         E.observe(g->d_view, g->d_feat, (n0 > 0 ? 1 : 0) | (n1 > 0 ? 2 : 0), g->st);
         for (int grp = 0; grp < 2; grp++) {
@@ -392,7 +391,7 @@ int env_get_observation(EnvHandle game, GroupHandle group, float **buffer) {
                                     (size_t)ng * FS * 4, cudaMemcpyDeviceToHost, g->st));
         }
         MF_CUDA(cudaStreamSynchronize(g->st));
-        g->obs_fresh = true;
+        g->obs = Game::Fresh;
     }
     memcpy(buffer[0], g->m_view + (size_t)group * cap * kViewRow, (size_t)n * kViewRow * 4);
     memcpy(buffer[1], g->m_feat + (size_t)group * cap * FS, (size_t)n * FS * 4);
@@ -436,14 +435,7 @@ int env_step(EnvHandle game, int *done) {
     }
     if (g->inject_next) E.set_rng_mode(RNG_INJECT);
     const bool want_events = !g->first_render;            // GridWorld.cc:533,559: recorded once a frame was rendered
-    if (want_events) {
-        if (g->ev_cap < cap) {
-            cudaFree(g->d_events);
-            MF_CUDA(cudaMalloc(&g->d_events, (size_t)(1 + 6 * cap) * 4));
-            g->ev_cap = cap;
-        }
-        io.attack_events = g->d_events;
-    }
+    if (want_events) io.attack_events = g->d_events;
     // what the play loop asks for next is enqueued behind the step: clear_dead (its records into the OTHER mirror),
     // both groups' observations, one copy per observation buffer
     auto enqueue = [&](bool with_spec, unsigned event_flags) {
@@ -459,19 +451,17 @@ int env_step(EnvHandle game, int *done) {
         MF_CUDA(cudaMemcpyAsync(g->m_feat, g->d_feat, (size_t)2 * cap * FS * 4, cudaMemcpyDeviceToHost, g->st));
         MF_CUDA(cudaEventRecordWithFlags(g->ev_spec, g->st, event_flags));
     };
-    const bool with_spec = !want_events && g->speculate;
-    const bool graphable = with_spec && g->use_graphs && !g->inject_next && io.phases == (PH_STEP | PH_SETACT);
-    bool launched = false;
+    const bool with_spec = !want_events;
+    const bool graphable = with_spec && !g->inject_next && io.phases == (PH_STEP | PH_SETACT);
     if (graphable && g->plain_steps >= 2) {
-        Game::StepGraph *hit = nullptr;
-        for (Game::StepGraph &sg : g->graphs)
-            if (sg.into == into && sg.seq0 == io.group_seq[0] && sg.seq1 == io.group_seq[1] && sg.setact_mask == io.setact_mask)
-                hit = &sg;
-        const bool valid = hit && hit->pin == g->pin && hit->d_view == g->d_view && hit->d_feat == g->d_feat &&
-                           hit->d_done == g->d_done && hit->d_perm == g->d_perm &&
-                           memcmp(&hit->P, &E.params(), sizeof(BattleParams)) == 0 &&
-                           memcmp(&hit->S, &E.state(), sizeof(BattleState)) == 0;
-        if (hit && !valid) { g->drop_graphs(); hit = nullptr; }       // something was re-allocated or re-configured
+        Game::GraphKey key;
+        memset(&key, 0, sizeof(key));         // memcmp compares the padding too
+        key.into = into; key.seq0 = io.group_seq[0]; key.seq1 = io.group_seq[1]; key.setact_mask = io.setact_mask;
+        key.pin = g->pin; key.d_view = g->d_view; key.d_feat = g->d_feat; key.d_done = g->d_done; key.d_perm = g->d_perm;
+        memcpy(&key.P, &E.params(), sizeof(BattleParams)); memcpy(&key.S, &E.state(), sizeof(BattleState));
+        const Game::StepGraph *hit = nullptr;
+        for (const Game::StepGraph &sg : g->graphs)
+            if (memcmp(&sg.key, &key, sizeof(key)) == 0) hit = &sg;
         if (!hit) {
             if (g->graphs.size() >= 8) g->drop_graphs();
             cudaGraph_t graph = nullptr;
@@ -479,22 +469,17 @@ int env_step(EnvHandle game, int *done) {
             try { enqueue(true, cudaEventRecordExternal); }
             catch (...) { cudaStreamEndCapture(g->st, &graph); if (graph) cudaGraphDestroy(graph); throw; }
             MF_CUDA(cudaStreamEndCapture(g->st, &graph));
-            Game::StepGraph sg;
-            const cudaError_t err = cudaGraphInstantiate(&sg.exec, graph, 0);
+            cudaGraphExec_t exec = nullptr;
+            const cudaError_t err = cudaGraphInstantiate(&exec, graph, 0);
             cudaGraphDestroy(graph);
             if (err != cudaSuccess) throw Fatal(std::string("cudaGraphInstantiate: ") + cudaGetErrorString(err));
-            sg.into = into; sg.seq0 = io.group_seq[0]; sg.seq1 = io.group_seq[1]; sg.setact_mask = io.setact_mask;
-            memcpy(&sg.P, &E.params(), sizeof(BattleParams)); memcpy(&sg.S, &E.state(), sizeof(BattleState));
-            sg.pin = g->pin; sg.d_view = g->d_view; sg.d_feat = g->d_feat; sg.d_done = g->d_done; sg.d_perm = g->d_perm;
-            g->graphs.push_back(sg);
+            g->graphs.push_back({key, exec});
             hit = &g->graphs.back();
         }
         MF_CUDA(cudaGraphLaunch(hit->exec, g->st));
         E.mark_stepped();                     // (Engine::step did not run on the host this time)
         g->graph_replays++;
-        launched = true;
-    }
-    if (!launched) {
+    } else {
         enqueue(with_spec, cudaEventRecordDefault);
         if (graphable) g->plain_steps++;
     }
@@ -504,13 +489,10 @@ int env_step(EnvHandle game, int *done) {
         g->events.clear();
         for (int i = 0; i < raw[0]; i++)
             if (raw[1 + 3 * i] >= 0) g->events.insert(g->events.end(), raw.begin() + 1 + 3 * i, raw.begin() + 4 + 3 * i);
-    } else if (with_spec) {
-        g->spec_pending = true;
     }
     MF_CUDA(cudaEventSynchronize(g->ev_step));            // rewards, alive flags, positions, done: in the mirror now
-    g->use_mirror(into);
-    g->state_fresh = true; g->obs_fresh = false; g->spec_state = false; g->spec_obs = false;
-    *done = g->mir[into].head[4];
+    g->after_step(into, with_spec);
+    *done = g->view().head[4];
     g->seq.clear();
     API_END("env_step")
 }
@@ -523,7 +505,7 @@ int env_get_reward(EnvHandle game, GroupHandle group, float *buffer) {
     g->ensure_staging();
     const int n = E.host_num(0, group);
     g->fetch_state();
-    const float *rew = g->m_rew + (size_t)group * E.cap();
+    const float *rew = g->view().rew + (size_t)group * E.cap();
     for (int i = 0; i < n; i++) buffer[i] = rew[i] + 0.0f;   // + Group::get_reward(), always 0 (GridWorld.cc:764-768)
     API_END("env_get_reward")
 }
@@ -589,7 +571,7 @@ int env_get_info(EnvHandle game, GroupHandle group, const char *name, void *void
             const int channel = ((i - group + ng) % ng + ng) % ng;
             const int n = E.host_num(0, i);
             g->fetch_state();
-            const int32_t *pos = g->m_pos + (size_t)i * cap;
+            const int32_t *pos = g->view().pos + (size_t)i * cap;
             for (int j = 0; j < n; j++)
                 fbuf[(((pos[j] >> 16) & 0xFFFF) / scale_h * vw + (pos[j] & 0xFFFF) / scale_w) * ng + channel] += 1.0f;
             for (int k = 0; k < vh * vw; k++) fbuf[k * ng + channel] /= (size_t)n;
@@ -603,19 +585,19 @@ int env_get_info(EnvHandle game, GroupHandle group, const char *name, void *void
         ibuf[0] = n;
     } else if (streq(name, "id")) {
         g->fetch_state();
-        memcpy(ibuf, g->m_id + (size_t)group * cap, (size_t)n * 4);
+        memcpy(ibuf, g->view().id + (size_t)group * cap, (size_t)n * 4);
     } else if (streq(name, "pos")) {
         g->fetch_state();
-        const int32_t *pos = g->m_pos + (size_t)group * cap;
+        const int32_t *pos = g->view().pos + (size_t)group * cap;
         for (int i = 0; i < n; i++) { ibuf[2 * i] = pos[i] & 0xFFFF; ibuf[2 * i + 1] = (pos[i] >> 16) & 0xFFFF; }
     } else if (streq(name, "alive")) {
         g->fetch_state();
-        const uint32_t *st = g->m_state + (size_t)group * cap;
+        const uint32_t *st = g->view().state + (size_t)group * cap;
         for (int i = 0; i < n; i++) bbuf[i] = !(st[i] & 1u);
     } else if (streq(name, "mean_info")) {                 // GridWorld.cc:849-870
         g->fetch_state();
-        const int32_t *pos = g->m_pos + (size_t)group * cap;
-        const uint32_t *st = g->m_state + (size_t)group * cap;
+        const int32_t *pos = g->view().pos + (size_t)group * cap;
+        const uint32_t *st = g->view().state + (size_t)group * cap;
         const int n_action = E.n_action();
         std::vector<int> counter(n_action + 1, 0);
         float sum_x = 0, sum_y = 0;
@@ -694,8 +676,8 @@ int env_render(EnvHandle game) {
     for (int grp = 0; grp < 2; grp++) {
         const int n = grp ? n1 : n0;
         g->fetch_state();
-        const int32_t *pos = g->m_pos + (size_t)grp * cap, *id = g->m_id + (size_t)grp * cap;
-        const float *hp = g->m_hp + (size_t)grp * cap;
+        const int32_t *pos = g->view().pos + (size_t)grp * cap, *id = g->view().id + (size_t)grp * cap;
+        const float *hp = g->view().hp + (size_t)grp * cap;
         for (int j = 0; j < n; j++) {
             const int pct = std::min(100, std::max(0, (int)(100 * hp[j] / t0.p.hp)));
             out << id[j] << " " << pct << " " << 270 /* NORTH: turn_mode is off, GridWorld.cc:264 */ << " " << (pos[j] & 0xFFFF) << " " << (pos[j] >> 16) << " " << grp << std::endl;
@@ -811,15 +793,13 @@ int gridworld_clear_dead(EnvHandle game) {
     // enqueued -- it runs back to back with whatever comes next (normally the observation kernel)
     for (int grp = 0; grp < 2; grp++) {
         const int n = E.host_num(0, grp);
-        const uint32_t *st = g->m_state + (size_t)grp * E.cap();
+        const uint32_t *st = g->view().state + (size_t)grp * E.cap();
         int alive = 0;
         for (int i = 0; i < n; i++) alive += !(st[i] & 1u);
         E.set_host_num(0, grp, alive);
     }
-    if (g->spec_pending) {                    // it already ran behind the step: commit
-        g->spec_pending = false;
-        g->state_fresh = false; g->obs_fresh = false;
-        g->spec_state = true; g->spec_obs = true;
+    if (g->spec_enqueued) {                   // it already ran behind the step: commit
+        g->commit_spec();
         return 0;
     }
     io.phases = PH_CLEAR; io.group_seq[0] = io.group_seq[1] = -1;

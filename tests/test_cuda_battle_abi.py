@@ -229,23 +229,12 @@ def test_speculation_rolls_back_when_the_caller_leaves_the_play_loop_order():
     run_lockstep(ora, cu, steps=30, seed=32, stream="fight")
 
 
-def test_speculation_switched_off_gives_the_same_results(monkeypatch):
-    monkeypatch.setenv("MAGENT_SPECULATE", "0")
-    ora, cu = OracleEngine(40), CudaEngine(40)
-    setup_pair([ora, cu], *generate_map_positions(40))
-    st = run_lockstep(ora, cu, steps=120, seed=8, stream="fight", skip_clear_every=5)
-    assert st["deaths"] > 10, st
-
-
-@pytest.mark.parametrize("graph", ["1", "0"])
-def test_step_graph_replay_follows_every_change_of_the_step_shape(graph, monkeypatch):
+def test_step_graph_replay_follows_every_change_of_the_step_shape():
     """After two plain steps env_step replays the steady sequence (set_action x2 + step + speculative clear_dead +
-    observe x2 + copies) as a CUDA graph keyed by mirror parity and set_action order (runtime_api.cu).  Everything
-    baked into a graph changes here while it is in use: the order of the set_action calls, a group that does not act,
-    a late add that grows the capacity (every buffer re-allocated), a new episode -- and the results stay the
-    oracle's bit for bit, with the graph on and off (MAGENT_STEP_GRAPH)."""
+    observe x2 + copies) as a CUDA graph (runtime_api.cu).  Everything baked into a graph changes here while it is in
+    use: the order of the set_action calls, a group that does not act, a late add that grows the capacity (every
+    buffer re-allocated), a new episode -- and the results stay the oracle's bit for bit."""
     from scenarios import fight_actions
-    monkeypatch.setenv("MAGENT_STEP_GRAPH", graph)
     ora, cu = OracleEngine(40), CudaEngine(40)
     left, right = generate_map_positions(40)
     rng = np.random.RandomState(17)
@@ -279,8 +268,7 @@ def test_step_graph_replay_follows_every_change_of_the_step_shape(graph, monkeyp
             # late adds: 64 -> 66 agents in episode 0 (the capacity grows, every buffer moves); in episode 1 right after
             # its FIRST step, which was a graph replay (nothing but the replay tells the engine that it has stepped)
             if (s == 25 and episode == 0) or (s == 0 and episode == 1):
-                if graph == "1":
-                    assert replays() == before + 1, "this step was meant to be a graph replay"
+                assert replays() == before + 1, "this step was meant to be a graph replay"
                 extra = np.array([[20, 3, 0], [21, 3, 0]], np.int32)
                 check(s)
                 for eng in (ora, cu):
@@ -289,4 +277,4 @@ def test_step_graph_replay_follows_every_change_of_the_step_shape(graph, monkeyp
                     assert_same("pos after add", ora.get_pos(g), cu.get_pos(g), s)
             else:
                 check(s)
-    assert (replays() > 80) if graph == "1" else (replays() == 0), replays()
+    assert replays() > 80, replays()
