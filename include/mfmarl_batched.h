@@ -67,6 +67,31 @@ int mfb_add_agents(mfb_engine *eng, int group, int n, const int *xs, const int *
  * Once used, mfb_add_agents / mfb_add_walls apply to every env's own template; auto_reset re-places each env from
  * ITS template. */
 int mfb_add_agents_per_env(mfb_engine *eng, int group, int n, const int *xs, const int *ys, int *n_added);
+/* Random placement: n agents of `group` go to cells drawn at random inside the rectangle [x0, x0+w) x [y0, y0+h)
+ * (w = h = 0: the whole map, i.e. the reference's get_random_blank).  Every env draws its own cells, at the commit
+ * that follows this call and again at every auto-reset, so each episode of each env starts from fresh draws.
+ *   - The op is appended to the engine's placement program; its n agents take the next n ids in call order, whatever
+ *     the draws.  An episode start places the fixed template first, then runs the random ops in call order.  After
+ *     mfb_add_agents_per_env they draw around each env's own template.  mfb_add_agents, mfb_add_agents_per_env and
+ *     mfb_add_walls after a random op are refused until mfb_reset (a random agent could take a fixed agent's cell).
+ *   - A candidate cell is blank when x + 1 < W, y + 1 < H (the reference's is_blank_area bound for a 1x1 body) and it
+ *     holds no wall, no fixed agent and no earlier random agent of this episode; candidates are drawn until one is.
+ *     MFB_RNG_MINSTD (and INJECT): candidate t is the next two draws r1, r2 of the env's own minstd stream ("rng"),
+ *     x = x0 + r1 % w, y = y0 + r2 % h (whole map: r1 % (W - 1), r2 % (H - 1)), and the stream continues from there
+ *     into the attack shuffles: at E = 1 with whole-map ops this is add_agents(method="random") of the single-env ABI,
+ *     cell for cell and draw for draw.  MFB_RNG_PHILOX: candidate t of op k (k counts the ops since mfb_reset) is
+ *     Philox4x32-10 with key (seed, env_base + e) and counter (t, k, episode, generation | 0x80000000), x = x0 +
+ *     mulhi(word0, w), y = y0 + mulhi(word1, h); generation counts the mfb_reset calls since mfb_create (a commit sets
+ *     episode to 0).  The top bit of word 3 keeps these draws apart from the attack shuffle's counter (i, step, 0, 0)
+ *     and random_sides' (episode, 0x51DE, 0, 0) under the same key.
+ *   - random_sides: an env that swaps sides swaps the groups of its random ops too, and their ids go with them.
+ *   - An agent gives up after W*H + 1 failed candidates (the reference's limit); it and the rest of its op are not
+ *     placed, and mfb_get "placement_short" counts them per env (the env's last placement).
+ *   - Returns -1 and changes nothing for a group other than 0 or 1, n < 0, a rectangle that leaves the map or has no
+ *     interior cell, and an op that cannot fit in some env: fewer blank cells in its rectangle (walls and fixed agents
+ *     excluded) than n plus the n of the earlier ops whose rectangles overlap it.  The capacity grows as for
+ *     mfb_add_agents. */
+int mfb_add_agents_random(mfb_engine *eng, int group, int n, int x0, int y0, int w, int h);
 int mfb_set_seed(mfb_engine *eng, unsigned long seed);
 
 /* sizes: key in {"capacity","n_envs","n_action","view_size","n_channel","feature_size","attack_base"}.
@@ -131,6 +156,7 @@ int mfb_local_mean_action(mfb_engine *eng, double radius, float *d_out0, float *
  *   "id" int32[E][2][cap], "alive" uint8[E][2][cap], "last_action" int32[E][2][cap],
  *   "step_ct" int32[E], "rng" uint32[E], "agent_steps" uint64[E] (agents stepped since creation),
  *   "side" int32[E] (1 = armies swapped this episode, random_sides), "episode" int32[E],
+ *   "placement_short" int32[E] (random agents the env's last placement could not place, mfb_add_agents_random),
  *   "walls" uint8[H][W] (1 = obstacle: the border ring and add_walls; the engine's, not per env)     */
 int mfb_get(mfb_engine *eng, const char *key, void *host_buf, void *stream);
 /* device pointer to the live int32[E][2] agent counts (for masking on the device) */
@@ -179,7 +205,11 @@ int mfb_state_device_ptr(mfb_engine *eng, const char *key, const void **out);
  *   - MFB_RNG_PHILOX: the attack shuffle is keyed by env_base + e too, so at another global id a loaded env draws its
  *     own attack orders from the first step.
  * At the source's global id a loaded env reproduces its source exactly in both modes (create the engine with a
- * matching env_base to replay any env). */
+ * matching env_base to replay any env).
+ * Random placement ops (mfb_add_agents_random) are engine configuration like max_steps: they are not in a record, and
+ * its template slices hold the fixed part only.  A record loaded into an engine with the same placement program (the
+ * same ops after as many mfb_reset calls) continues exactly through its next auto-resets too: MINSTD draws from the
+ * rng in the record, Philox from its episode and global id. */
 int mfb_save_envs(mfb_engine *eng, int n, const int32_t *envs, void *d_out /* device [n][R] */, void *stream);
 int mfb_load_envs(mfb_engine *eng, int n, const int32_t *envs, const void *d_in /* device [n][R] */, void *stream);
 

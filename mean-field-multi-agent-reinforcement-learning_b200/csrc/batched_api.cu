@@ -205,6 +205,11 @@ int mfb_add_agents_per_env(mfb_engine *h, int group, int n, const int *xs, const
     E(h).add_agents_per_env(group, n, xs, ys, n_added);
     MFB_END("mfb_add_agents_per_env")
 }
+int mfb_add_agents_random(mfb_engine *h, int group, int n, int x0, int y0, int w, int hgt) {
+    MFB_BEGIN
+    E(h).add_agents_random(group, n, x0, y0, w, hgt);
+    MFB_END("mfb_add_agents_random")
+}
 int mfb_set_seed(mfb_engine *h, unsigned long seed) { MFB_BEGIN E(h).set_seed(seed); MFB_END("mfb_set_seed") }
 
 int mfb_query(mfb_engine *h, const char *key, int *out) {
@@ -308,6 +313,7 @@ int mfb_get(mfb_engine *h, const char *key, void *host_buf, void *stream) {
     else if (k == "step_ct") copy(S.step_ct, ne * 4);
     else if (k == "side") copy(S.side, ne * 4);
     else if (k == "episode") copy(S.episode, ne * 4);
+    else if (k == "placement_short") copy(e.placement_short(), ne * 4);
     else if (k == "rng") copy(S.rng, ne * 4);
     else if (k == "agent_steps") copy(S.agent_steps, ne * 8);
     else if (k == "walls") memcpy(host_buf, e.host_walls().data(), e.host_walls().size());

@@ -191,6 +191,105 @@ __device__ __forceinline__ uint32_t minstd_jump(uint32_t s, uint32_t n) {
     return (uint32_t)acc;
 }
 
+// Random placement (mfb_add_agents_random), the second stage of an episode start: call after place_from_template and a
+// __syncthreads, from every thread of the CTA.  occ: scratch bitmap of W*H bits (shared or global memory).
+//
+// The reference's sequential loop (GridWorld.cc:236-255, Map::get_random_blank Map.cc:49-63; runtime_api.cu's host
+// loop): per agent, draw candidates until one is blank -- inside x + 1 < W, y + 1 < H, not a wall, not an agent -- and
+// give up after W*H + 1 failures (then the rest of the op is not placed either).  One warp runs it 32 candidates at a
+// time: lane l evaluates candidate t + l against the bitmap; a candidate is accepted if it is blank and the first blank
+// one of the batch on its cell (__match_any_sync), and a lane-uniform scan of the accepted mask replays the sequential
+// bookkeeping (agents placed, failures of the current agent) to find how many candidates the loop consumed.  MINSTD:
+// candidate t is draws 2t+1 and 2t+2 of the env's stream (x = x0 + r1 % w, y = y0 + r2 % h), and the stream is left
+// right after the last candidate consumed.  Philox: candidate t of op k is counter (t, k, episode, generation | 2^31)
+// under the key (seed, env_base + e), x = x0 + mulhi(word0, w), y = y0 + mulhi(word1, h); the top bit of word 3 keeps
+// it apart from the attack shuffle's (i, step, 0, 0) and random_sides' (episode, 0x51DE, 0, 0) counters.
+__device__ __forceinline__ void place_random(const BattleParams &P, const BattleState &S, const RandomPlacement &RP, int e,
+                                             int side, int episode, uint32_t *occ) {
+    const int tid = threadIdx.x, nt = blockDim.x, W = P.W, H = P.H, cap = P.cap, cells = W * H;
+    const int words = (cells + 31) >> 5;
+    const size_t ebase = (size_t)e * 2 * cap;
+    const uint8_t *walls = S.walls + (size_t)e * P.wall_stride;
+    for (int w = tid; w < words; w += nt) {
+        uint32_t bits = 0;
+        for (int b = 0; b < 32 && 32 * w + b < cells; b++) bits |= (uint32_t)(walls[32 * w + b] != 0) << b;
+        occ[w] = bits;
+    }
+    __syncthreads();
+    const int n0 = S.num[e * 2], n1 = S.num[e * 2 + 1];   // the fixed template, as place_from_template left it
+    for (int s = tid; s < 2 * cap; s += nt) {
+        const int g = s >= cap, i = s - g * cap;
+        if (i < (g ? n1 : n0)) {
+            const int p = S.pos[ebase + s], c = pos_y(p) * W + pos_x(p);
+            atomicOr(&occ[c >> 5], 1u << (c & 31));
+        }
+    }
+    __syncthreads();
+    if (tid >= 32) return;
+    const volatile uint32_t *vocc = occ;   // this warp's own atomics must be seen by its later loads (global: not L1)
+    const int lane = tid;
+    const unsigned full = 0xFFFFFFFFu, below = (1u << lane) - 1u;
+    const bool minstd = P.rng_mode != RNG_PHILOX;
+    const uint32_t max_fails = (uint32_t)cells + 1u;
+    uint32_t rs = minstd ? S.rng[e] : 0u;
+    int num0 = n0, num1 = n1, id_end = S.id_counter[e], short_ct = 0;
+    for (int k = 0; k < RP.n_ops; k++) {
+        const RandomOp op = RP.ops[k];
+        const int g = op.group ^ side, id0 = id_end + op.id0, base = g ? num1 : num0;
+        int placed = 0;
+        uint32_t fails = 0, t = 0;
+        bool gave_up = false;
+        while (placed < op.n && !gave_up) {
+            uint32_t x, y, rs_after = 0;
+            if (minstd) {
+                const uint32_t r1 = minstd_jump(rs, 2u * lane + 1u), r2 = minstd_next(r1);
+                x = (uint32_t)op.x0 + r1 % (uint32_t)op.w; y = (uint32_t)op.y0 + r2 % (uint32_t)op.h;
+                rs_after = r2;
+            } else {
+                const uint4 r = philox4x32_10(make_uint4(t + lane, (uint32_t)k, (uint32_t)episode, RP.generation | 0x80000000u),
+                                              make_uint2(P.seed, (uint32_t)(P.env_base + e)));
+                x = (uint32_t)op.x0 + __umulhi(r.x, (uint32_t)op.w); y = (uint32_t)op.y0 + __umulhi(r.y, (uint32_t)op.h);
+            }
+            const int c = (int)(y * W + x);
+            const bool blank = x + 1 < (uint32_t)W && y + 1 < (uint32_t)H && !((vocc[c >> 5] >> (c & 31)) & 1u);
+            const unsigned peers = __match_any_sync(full, blank ? c : -1 - lane);
+            unsigned ok = __ballot_sync(full, blank && lane == __ffs(peers) - 1);
+            // the sequential loop over this batch: accepted candidates in lane order, failures in between
+            unsigned acc = 0;
+            int consumed = 32, pos = 0;
+            for (;;) {
+                const int next = ok ? __ffs(ok) - 1 : 32;
+                const uint32_t gap = (uint32_t)(next - pos);
+                if (fails + gap >= max_fails) { consumed = pos + (int)(max_fails - fails); gave_up = true; break; }
+                if (next == 32) { fails += gap; break; }
+                acc |= 1u << next; ok &= ok - 1u; fails = 0; pos = next + 1;
+                if (placed + __popc(acc) == op.n) { consumed = pos; break; }
+            }
+            if ((acc >> lane) & 1u) {
+                const int idx = placed + __popc(acc & below), s = g * cap + base + idx;
+                S.pos[ebase + s] = pack_pos((int)x, (int)y);
+                S.id[ebase + s] = id0 + idx;
+                atomicOr(&occ[c >> 5], 1u << (c & 31));
+            }
+            placed += __popc(acc);
+            if (minstd) rs = __shfl_sync(full, rs_after, consumed - 1);
+            t += (uint32_t)consumed;
+            __syncwarp();
+        }
+        if (g) num1 += placed; else num0 += placed;
+        short_ct += op.n - placed;
+    }
+    if (lane == 0) {
+        S.num[e * 2] = num0; S.num[e * 2 + 1] = num1;
+        if (RP.n_ops > 0) {
+            const RandomOp last = RP.ops[RP.n_ops - 1];
+            S.id_counter[e] = id_end + last.id0 + last.n;
+        }
+        if (minstd) S.rng[e] = rs;
+        RP.place_short[e] = short_ct;
+    }
+}
+
 // ----------------------------------------------------------------------------------------------
 // K2: fused step
 // ----------------------------------------------------------------------------------------------
@@ -243,8 +342,10 @@ __host__ __device__ inline unsigned char *step_workspace(const BattleParams &P, 
 // that follows the observation records (always kept at such geometries) in their allocation -- the shared atomics
 // become global atomics on the env's own lines, served by L2.  Only s_misc and the minimap counts stay in shared
 // memory (kStepHbmSmem bytes), and the observation record is built in place.
-template <bool HBM>
-__global__ void k_step(const __grid_constant__ BattleParams P, const BattleState S, const StepIO io) {
+// RANDOM = true (engines with random placement ops): the auto-reset runs place_random after the template.  A separate
+// instantiation, so that an engine without random ops runs k_step with the registers and code it always had.
+template <bool HBM, bool RANDOM = false>
+__global__ void k_step(const __grid_constant__ BattleParams P, const BattleState S, const StepIO io, const RandomPlacement RP) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const StepSmem L = step_smem_layout(P.W, P.H, P.cap, P.obs_cached);
     unsigned char *const ws = HBM ? step_workspace(P, S) + (size_t)blockIdx.x * L.total : nullptr;
@@ -656,6 +757,11 @@ __global__ void k_step(const __grid_constant__ BattleParams P, const BattleState
             side = (int)(r.x & 1u);
         }
         place_from_template(P, S, e, side);
+        if constexpr (RANDOM) {   // the step's grid is dead by now: its shared memory holds the placer's bitmap
+            __syncthreads();
+            place_random(P, S, RP, e, side, episode,
+                         HBM ? RP.occ + (size_t)e * ((cells + 31) >> 5) : (uint32_t *)(smem_raw + L.grid));
+        }
         if (tid == 0) S.episode[e] = episode;
     } else if (phases & PH_CLEAR) {
         for (int g = 0; g < kGroups; g++) {
@@ -1254,11 +1360,18 @@ __global__ void __launch_bounds__(kLocalMaxTile) k_local_mean_action(const __gri
 }
 
 // ----------------------------------------------------------------------------------------------
-// episode (re)initialisation: every env gets the placement template
+// episode (re)initialisation: every env gets the placement template, then the random ops
 // ----------------------------------------------------------------------------------------------
-__global__ void k_place(const __grid_constant__ BattleParams P, const BattleState S) {
-    place_from_template(P, S, blockIdx.x, 0);
-    if (threadIdx.x == 0) S.episode[blockIdx.x] = 0;
+__global__ void k_place(const __grid_constant__ BattleParams P, const BattleState S, const RandomPlacement RP) {
+    const int e = blockIdx.x;
+    place_from_template(P, S, e, 0);
+    if (threadIdx.x == 0) S.episode[e] = 0;
+    if (RP.n_ops) {
+        __syncthreads();
+        place_random(P, S, RP, e, 0, 0, RP.occ + (size_t)e * ((P.W * P.H + 31) >> 5));
+    } else if (threadIdx.x == 0) {
+        RP.place_short[e] = 0;
+    }
 }
 
 }  // namespace mfmarl

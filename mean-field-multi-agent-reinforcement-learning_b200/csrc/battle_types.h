@@ -50,6 +50,22 @@ enum StepPhase : int {
     PH_AUTORESET = 16, // batched extension: re-place the armies when an episode ends
 };
 
+// One random placement op (mfb_add_agents_random): n agents of `group` on cells drawn in [x0, x0+w) x [y0, y0+h)
+// (the whole-map request is stored resolved: 0, 0, W-1, H-1).  Its agents take ids id0 .. id0+n-1 after the fixed
+// template's (id0 counts the n of the earlier ops).
+struct RandomOp { int group, n, x0, y0, w, h, id0, pad; };
+
+// The random part of the placement program, passed to k_place and k_step after their other parameters (so that the
+// kernels without random ops keep their parameter layout and code).
+struct RandomPlacement {
+    const RandomOp *ops;       // [n_ops] in call order
+    int n_ops;                 // 0 = the fixed template alone
+    uint32_t generation;       // mfb_reset calls since creation: keys the Philox draws (a commit restarts `episode` at 0)
+    int32_t *place_short;      // [E] random agents the env's last placement could not place
+    uint32_t *occ;             // [E][ceil(W*H / 32)] occupancy bitmaps where the placer cannot use shared memory (k_place,
+                               // k_step<true>); allocated once the engine has random ops
+};
+
 struct BattleParams {
     int E, W, H, cap;
     int env_base;           // global id of env 0 of this engine (multi-GPU sharding; keys Philox)

@@ -63,9 +63,54 @@ void Engine::split_template() {
     }
 }
 
+void Engine::refuse_after_random(const char *what) const {
+    // a random agent could take a fixed agent's (or wall's) cell, and that agent would be skipped in some episodes only
+    if (!h_random_.empty())
+        throw Fatal(std::string(what) + " after add_agents_random is not supported (call reset first): the fixed "
+                    "placement and the walls come before the random ops");
+}
+
+void Engine::add_agents_random(int group, int n, int x0, int y0, int w, int h) {
+    const int W = P_.W, H = P_.H;
+    if (group < 0 || group >= kGroups) throw Fatal("group = " + std::to_string(group) + " is not 0 or 1");
+    if (n < 0) throw Fatal("n = " + std::to_string(n) + " is negative");
+    if (stepped_) throw Fatal("add_agents_random after stepping is not supported (call reset first)");
+    const std::string rect = "rectangle x0 = " + std::to_string(x0) + ", y0 = " + std::to_string(y0) +
+                             ", w = " + std::to_string(w) + ", h = " + std::to_string(h);
+    if (w == 0 && h == 0) { x0 = 0; y0 = 0; w = W - 1; h = H - 1; }   // the whole map: Map::get_random_blank's draw
+    if (w <= 0 || h <= 0) throw Fatal(rect + ": w and h must both be positive, or both 0 for the whole map");
+    if (x0 < 0 || y0 < 0 || x0 > W - w || y0 > H - h)
+        throw Fatal(rect + " leaves the " + std::to_string(W) + "x" + std::to_string(H) + " map");
+    // cells that can be blank: inside the border ring (walls) and the is_blank_area bound x + 1 < W, y + 1 < H
+    const int ix0 = std::max(x0, 1), ix1 = std::min(x0 + w - 1, W - 2), iy0 = std::max(y0, 1), iy1 = std::min(y0 + h - 1, H - 2);
+    if (ix0 > ix1 || iy0 > iy1) throw Fatal(rect + " has no interior cell");
+    // the earlier ops whose rectangles overlap this one may take up to their n of its cells
+    long long taken = 0;
+    for (const RandomOp &o : h_random_)
+        if (o.x0 < x0 + w && x0 < o.x0 + o.w && o.y0 < y0 + h && y0 < o.y0 + o.h) taken += o.n;
+    const size_t T = h_env_.empty() ? 1 : h_env_.size();
+    for (size_t e = 0; e < T; e++) {
+        long long blank = 0;
+        for (int y = iy0; y <= iy1; y++)
+            for (int x = ix0; x <= ix1; x++) {
+                const size_t c = (size_t)y * W + x;
+                blank += (h_env_.empty() ? h_occ_[c] : h_env_[e].occ[c]) == 0;
+            }
+        if (blank < taken + n)
+            throw Fatal("n = " + std::to_string(n) + " does not fit" + (h_env_.empty() ? std::string() : " in env " + std::to_string(e)) +
+                        ": the " + rect + " has " + std::to_string(blank) + " blank cells, and earlier random ops whose "
+                        "rectangles overlap it place up to " + std::to_string(taken) + " agents");
+    }
+    RandomOp op{group, n, x0, y0, w, h, 0, 0};
+    if (!h_random_.empty()) op.id0 = h_random_.back().id0 + h_random_.back().n;
+    h_random_.push_back(op);
+    placement_dirty_ = true;
+}
+
 void Engine::add_agents_per_env(int group, int n, const int *xs, const int *ys, int *n_added) {
     if (group < 0 || group >= kGroups) throw Fatal("invalid group handle in add_agents_per_env");
     if (stepped_) throw Fatal("add_agents_per_env after stepping is not supported (call reset first)");
+    refuse_after_random("add_agents_per_env");
     split_template();
     for (int e = 0; e < P_.E; e++) {   // per env: GridWorld.cc:256-269; Map::add_agent Map.cc:75-97; add_or_error :180-187
         EnvTemplate &t = h_env_[(size_t)e];
@@ -212,8 +257,10 @@ Engine::Engine(const EngineConfig &cfg) : cfg_(cfg) {
     MF_CUDA(cudaMalloc(&S_.init_num, E * 2 * sizeof(int32_t)));
     MF_CUDA(cudaMalloc(&S_.side, E * sizeof(int32_t)));
     MF_CUDA(cudaMalloc(&S_.episode, E * sizeof(int32_t)));
+    MF_CUDA(cudaMalloc(&RP_.place_short, E * sizeof(int32_t)));
     MF_CUDA(cudaMemset(S_.side, 0, E * sizeof(int32_t)));
     MF_CUDA(cudaMemset(S_.episode, 0, E * sizeof(int32_t)));
+    MF_CUDA(cudaMemset(RP_.place_short, 0, E * sizeof(int32_t)));
     P_.tmpl_stride = 0; P_.random_sides = cfg.random_sides != 0;
     MF_CUDA(cudaMalloc(&S_.grid_template, grid_template_bytes()));
     {   // minimap cell of a position, as a table: the kernels never divide by the runtime scale
@@ -240,6 +287,7 @@ Engine::Engine(const EngineConfig &cfg) : cfg_(cfg) {
     set_seed(cfg.seed);   // seed 0 -> minstd state 1, as GridWorld.cc:31 random_engine.seed(0)
     alloc_state(std::max(4, round_up(cfg.capacity, 4)));
     reset();
+    RP_.generation = 0;
 }
 
 Engine::~Engine() {
@@ -247,6 +295,7 @@ Engine::~Engine() {
     cudaFree(S_.num); cudaFree(S_.dead_ct); cudaFree(S_.rng); cudaFree(S_.step_ct);
     cudaFree(S_.id_counter); cudaFree(S_.walls); cudaFree(S_.init_num); cudaFree(S_.agent_steps); cudaFree(S_.obs_ticket); cudaFree(S_.mini_lut); cudaFree(S_.grid_template);
     cudaFree(S_.side); cudaFree(S_.episode);
+    cudaFree(RP_.place_short); cudaFree(RP_.occ); cudaFree((void *)RP_.ops);
     cudaFree(d_state_io_);
     if (state_io_done_) cudaEventDestroy(state_io_done_);
 }
@@ -332,6 +381,8 @@ void Engine::reset() {   // GridWorld::reset (GridWorld.cc:76-124) + Map::reset 
     for (int g = 0; g < kGroups; g++) { h_tpos_[g].clear(); h_tid_[g].clear(); }
     h_id_counter_ = 0;
     h_env_.clear();
+    h_random_.clear();
+    RP_.generation++;   // (the constructor's own reset leaves it at 0)
     placement_dirty_ = true;
     stepped_ = false;
     std::fill(h_num_.begin(), h_num_.end(), 0);
@@ -339,6 +390,7 @@ void Engine::reset() {   // GridWorld::reset (GridWorld.cc:76-124) + Map::reset 
 
 int Engine::add_walls(int n, const int *xs, const int *ys) {   // GridWorld.cc:203-211, Map::add_wall Map.cc:108-115
     if (stepped_) throw Fatal("add_walls after stepping is not supported (call reset first)");
+    refuse_after_random("add_walls");
     int added = 0;
     for (int i = 0; i < n; i++) {
         const int x = xs[i], y = ys[i];
@@ -357,6 +409,7 @@ int Engine::add_walls(int n, const int *xs, const int *ys) {   // GridWorld.cc:2
 
 int Engine::add_agents(int group, int n, const int *xs, const int *ys) {
     if (group < 0 || group >= kGroups) throw Fatal("invalid group handle in add_agents");
+    refuse_after_random("add_agents");
     if (stepped_) {
         if (P_.E != 1) throw Fatal("add_agents after stepping is only supported for a single env");
         late_add_sync_down();
@@ -500,9 +553,22 @@ void Engine::grow(int need_cap) {
 void Engine::commit(cudaStream_t st) {
     if (!placement_dirty_) return;
     const bool per_env = !h_env_.empty();
-    size_t need = std::max(h_tpos_[0].size(), h_tpos_[1].size());
-    for (const EnvTemplate &t : h_env_) need = std::max(need, std::max(t.pos[0].size(), t.pos[1].size()));
+    size_t rnd[kGroups] = {0, 0};   // a group's random agents sit behind its fixed ones (random_sides swaps both)
+    for (const RandomOp &o : h_random_) rnd[o.group] += (size_t)o.n;
+    size_t need = std::max(h_tpos_[0].size() + rnd[0], h_tpos_[1].size() + rnd[1]);
+    for (const EnvTemplate &t : h_env_) need = std::max(need, std::max(t.pos[0].size() + rnd[0], t.pos[1].size() + rnd[1]));
     grow((int)need);
+    RP_.n_ops = (int)h_random_.size();
+    if (!h_random_.empty()) {
+        if (h_random_.size() > d_random_cap_) {
+            cudaFree((void *)RP_.ops); RP_.ops = nullptr;
+            RandomOp *ops = nullptr;
+            MF_CUDA(cudaMalloc(&ops, h_random_.size() * sizeof(RandomOp)));
+            RP_.ops = ops; d_random_cap_ = h_random_.size();
+        }
+        MF_CUDA(cudaMemcpyAsync((void *)RP_.ops, h_random_.data(), h_random_.size() * sizeof(RandomOp), cudaMemcpyHostToDevice, st));
+        if (!RP_.occ) MF_CUDA(cudaMalloc(&RP_.occ, (size_t)P_.E * ((P_.W * P_.H + 31) / 32) * 4));
+    }
     const int cap = P_.cap;
     const size_t T = per_env ? (size_t)P_.E : 1;
     std::vector<int32_t> tmpl(T * 4 * cap, 0), num(T * 2, 0);
@@ -530,13 +596,14 @@ void Engine::commit(cudaStream_t st) {
             if (h_walls_[(size_t)y * P_.W + x]) gtmpl[(size_t)(y + kView / 2) * PW + x + kView / 2] = (uint16_t)(1u << 14);
     MF_CUDA(cudaMemcpyAsync(S_.grid_template, gtmpl.data(), gtmpl.size() * 2, cudaMemcpyHostToDevice, st));
     MF_CUDA(cudaStreamSynchronize(st));
-    k_place<<<P_.E, 128, 0, st>>>(P_, S_);
+    k_place<<<P_.E, 128, 0, st>>>(P_, S_, RP_);
     MF_CUDA(cudaGetLastError());
     rebuild_obs_records(st);
     // a placement is a per-episode event: wait for it, so that whatever stream the next launch uses (the legacy
     // stream of mfb_query, a non-blocking side stream of the caller) it is ordered after the new state
     MF_CUDA(cudaStreamSynchronize(st));
     for (int e = 0; e < P_.E; e++) { const size_t t = per_env ? (size_t)e : 0; h_num_[e * 2] = num[t * 2]; h_num_[e * 2 + 1] = num[t * 2 + 1]; }
+    if (!h_random_.empty()) download_num(st);   // the draws decide how many agents each env holds
     placement_dirty_ = false;
     stepped_ = false;
 }
@@ -637,13 +704,13 @@ void Engine::step(const StepIO &io, cudaStream_t st) {
     commit(st);
     const bool hbm = hbm_kernels() & HBM_STEP;
     const StepSmem L = step_smem_layout(P_.W, P_.H, P_.cap, P_.obs_cached);
-    if (!hbm) raise_dynamic_smem((const void *)k_step<false>, L.total, device_);
+    // the random placer only ever runs in the auto-reset branch
+    const bool rnd = RP_.n_ops > 0 && (io.phases & PH_AUTORESET);
+    void (*kern)(const BattleParams, const BattleState, const StepIO, const RandomPlacement) =
+        hbm ? (rnd ? k_step<true, true> : k_step<true>) : (rnd ? k_step<false, true> : k_step<false>);
+    if (!hbm) raise_dynamic_smem((const void *)kern, L.total, device_);
     const int threads = step_threads();
-    if (hbm) {
-        k_step<true><<<P_.E, threads, kStepHbmSmem, st>>>(P_, S_, io);
-    } else {
-        k_step<false><<<P_.E, threads, L.total, st>>>(P_, S_, io);
-    }
+    kern<<<P_.E, threads, hbm ? kStepHbmSmem : L.total, st>>>(P_, S_, io, RP_);
     MF_CUDA(cudaGetLastError());
     if (io.phases & (PH_STEP | PH_CLEAR | PH_SETACT)) stepped_ = true;
 }

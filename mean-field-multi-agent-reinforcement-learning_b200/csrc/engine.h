@@ -70,6 +70,9 @@ public:
     // a placement of its own for every env: xs / ys are [E][n]; occupied or out-of-range cells are skipped PER ENV
     // (GridWorld.cc:180-187), so the envs may end up with different counts; n_added (may be null) receives [E] counts
     void add_agents_per_env(int group, int n, const int *xs, const int *ys, int *n_added);
+    // mfb_add_agents_random: appends a random op to the placement program (w = h = 0: the whole map); refuses, changing
+    // nothing, a bad group or n, a rectangle off the map or without an interior cell, and an op that cannot fit in some env
+    void add_agents_random(int group, int n, int x0, int y0, int w, int h);
     void set_seed(unsigned long seed);                         // set_config("seed")
 
     // ---- kernels ----
@@ -115,6 +118,7 @@ public:
     void push_rng0(uint32_t s);
     bool cell_blank_for_placement(int x, int y);   // Map::is_blank_area for a 1x1 body, host view
     const BattleState &state() const { return S_; }
+    const int32_t *placement_short() const { return RP_.place_short; }   // [E] (mfb_get "placement_short")
     int cap() const { return P_.cap; }
     int n_envs() const { return P_.E; }
     int n_action() const { return P_.n_move + P_.n_attack; }
@@ -173,6 +177,10 @@ private:
     struct EnvTemplate { std::vector<unsigned char> occ; std::vector<int> pos[kGroups], id[kGroups]; int id_counter = 0; };
     std::vector<EnvTemplate> h_env_;              // empty = shared template
     void split_template();                        // shared -> per-env
+    void refuse_after_random(const char *what) const;   // fixed placements and walls must come before the random ops
+    std::vector<RandomOp> h_random_;              // the random ops since the last reset, in call order
+    RandomPlacement RP_{};                        // what k_place / k_step see of them (ops uploaded at commit)
+    size_t d_random_cap_ = 0;                     // RandomOp slots allocated at RP_.ops
     bool placement_dirty_ = true;
     bool stepped_ = false;                        // a step has run since the last placement upload
     std::vector<int> h_num_;                      // [E][2] mirror, refreshed by download_num

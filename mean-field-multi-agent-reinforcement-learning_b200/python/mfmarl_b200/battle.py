@@ -128,6 +128,15 @@ class BatchedGridWorld:
         self._sizes = None
         return added
 
+    def add_agents_random(self, group, n, rect=None):
+        """n agents of `group` on cells drawn at random inside rect = (x0, y0, w, h) (None = the whole map, the
+        reference's add_agents(method="random")), drawn afresh in every env at the next placement and at every
+        auto-reset.  Fixed agents and walls must come first (until reset()).  get("placement_short") counts the agents
+        an env's last placement could not place."""
+        x0, y0, w, h = (0, 0, 0, 0) if rect is None else (int(v) for v in rect)
+        check(self.lib.mfb_add_agents_random(self._h, group, n, x0, y0, w, h))
+        self._sizes = None
+
     # ------------------------------------------------------------ sizes / buffers
     def query(self, key):
         out = ctypes.c_int()
@@ -292,7 +301,8 @@ class BatchedGridWorld:
             "id": ("i4", lambda E, c: (E, 2, c)), "alive": ("u1", lambda E, c: (E, 2, c)),
             "last_action": ("i4", lambda E, c: (E, 2, c)), "step_ct": ("i4", lambda E, c: (E,)),
             "rng": ("u4", lambda E, c: (E,)), "agent_steps": ("u8", lambda E, c: (E,)),
-            "side": ("i4", lambda E, c: (E,)), "episode": ("i4", lambda E, c: (E,))}
+            "side": ("i4", lambda E, c: (E,)), "episode": ("i4", lambda E, c: (E,)),
+            "placement_short": ("i4", lambda E, c: (E,))}
 
     def get(self, key):
         """mfb_get: the keys of _GET as numpy arrays, and "walls" uint8[H, W] (1 = obstacle)."""

@@ -31,6 +31,9 @@ def battle_parser(description, training):
         ap.add_argument("--mean_field", choices=("group", "local"), default="group",
                         help="mean action of the mean-field learners: 'group' = over the whole group (the reference's), "
                              "'local' = over each agent's group-mates within its view radius (needs --envs)")
+        ap.add_argument("--placement", choices=("blocks", "random"), default="blocks",
+                        help="with --envs, where the armies start: 'blocks' = the reference's two blocks, 'random' = "
+                             "cells drawn per env and round on the GPU in the left and right halves of the map")
         ap.add_argument("--replay", choices=("rows", "states"), default="rows",
                         help="with --envs, the Q learners' device replay: 'rows' stores every observation row (4.9 KB "
                              "each, so only the first envs fit), 'states' stores one env state record per recorded env "
@@ -42,6 +45,8 @@ def check_battle_args(ap, args):
     """combinations argparse cannot express; exits with a usage error like argparse itself"""
     if getattr(args, "mean_field", "group") == "local" and args.envs <= 0:
         ap.error("--mean_field local needs the batched engine: pass --envs N (N > 0)")
+    if getattr(args, "placement", "blocks") == "random" and args.envs <= 0:
+        ap.error("--placement random needs the batched engine: pass --envs N (N > 0)")
     if getattr(args, "replay", "rows") == "states":
         if args.envs <= 0:
             ap.error("--replay states needs the batched engine: pass --envs N (N > 0)")

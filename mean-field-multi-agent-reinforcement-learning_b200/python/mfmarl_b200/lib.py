@@ -43,6 +43,7 @@ def load_library(path=None):
         "mfb_add_walls": [vp, ci, vp, vp],
         "mfb_add_agents": [vp, ci, ci, vp, vp, ctypes.POINTER(ci)],
         "mfb_add_agents_per_env": [vp, ci, ci, vp, vp, vp],
+        "mfb_add_agents_random": [vp, ci, ci, ci, ci, ci, ci],
         "mfb_set_seed": [vp, ctypes.c_ulong],
         "mfb_query": [vp, cp, ctypes.POINTER(ci)],
         "mfb_observe": [vp, vp, vp, ci, vp],

@@ -25,6 +25,16 @@ def map_positions(map_size):
     return left, right
 
 
+def random_halves(map_size):
+    """The left and right interior halves of the map as (x0, y0, w, h) rectangles for random placement, with the gap of
+    map_positions between them (the columns from map_size // 2 - 3 to map_size // 2 + 2 stay empty), so the armies
+    do not start in contact."""
+    gap = 3
+    left = (1, 1, map_size // 2 - gap - 1, map_size - 2)
+    right = (map_size // 2 + gap, 1, map_size - 1 - (map_size // 2 + gap), map_size - 2)
+    return left, right
+
+
 def generate_map(env, map_size, handles):
     """senario_battle.py:8-38: which handle gets the left block is one random.randint(0, 1) draw; the left block is
     added first (and therefore gets the lower agent ids)."""
@@ -101,7 +111,7 @@ def battle(env, n_round, map_size, max_steps, handles, models, print_every, eps=
 # batched, device-resident form
 # ----------------------------------------------------------------------------------------------------------
 def play_batched(env, n_round, max_steps, models, eps=1.0, train=False, print_every=0, left_group=None,
-                 positions=None, obs_dtype=None, host_lag=None, mean_field="group", mf_radius=None):
+                 positions=None, obs_dtype=None, host_lag=None, mean_field="group", mf_radius=None, placement="blocks"):
     """E episodes in lockstep on a `BatchedGridWorld` (one per environment), everything on the device.
 
     Per environment this is the loop of `play`: observe both groups -> models[g].act on the group's rows (with the
@@ -123,9 +133,16 @@ def play_batched(env, n_round, max_steps, models, eps=1.0, train=False, print_ev
     group-mates inside the disc of radius `mf_radius` (None = the view radius) that acted last step
     (`BatchedGridWorld.local_mean_action`), zeros before the first step; the replay then stores each agent's own row.
 
+    placement: "blocks" puts the two armies on `positions` (default: the blocks of map_positions), the same cells in
+    every environment.  "random" draws every environment's cells on the GPU, as many agents per army as a block holds,
+    inside the two halves of random_halves: the left half goes to `left_group`, which is added first and so gets the
+    low ids.
+
     Returns (max_nums [E, 2], nums [E, 2], mean_rewards [E, 2], total_rewards [E, 2]) as numpy arrays.
     """
     import torch
+    if placement not in ("blocks", "random"):
+        raise ValueError("placement must be 'blocks' or 'random', not %r" % (placement,))
     if mean_field not in ("group", "local"):
         raise ValueError("mean_field must be 'group' or 'local', not %r" % (mean_field,))
     local = mean_field == "local"
@@ -137,8 +154,13 @@ def play_batched(env, n_round, max_steps, models, eps=1.0, train=False, print_ev
     if left_group is None:
         left_group = random.randint(0, 1)
     env.reset()
-    env.add_agents(left_group, positions[0])
-    env.add_agents(1 - left_group, positions[1])
+    if placement == "random":
+        halves = random_halves(env.map_size)
+        env.add_agents_random(left_group, len(positions[0]), halves[0])
+        env.add_agents_random(1 - left_group, len(positions[1]), halves[1])
+    else:
+        env.add_agents(left_group, positions[0])
+        env.add_agents(1 - left_group, positions[1])
     n_action = env.sizes["n_action"]
     if local:
         local_mean = env.local_mean_action(radius=mf_radius)    # nobody has acted yet: all rows zero

@@ -35,8 +35,8 @@ class BatchedEnvAdapter:
     """What Runner / spawn_ai ask of `env` (space queries) on top of a BatchedGridWorld, plus a `play` handle that
     reduces the per-environment statistics of play_batched to the scalars Runner logs (means over environments)."""
 
-    def __init__(self, benv, rollout_bf16=False, mean_field="group"):
-        self.benv, self.rollout_bf16, self.mean_field = benv, rollout_bf16, mean_field
+    def __init__(self, benv, rollout_bf16=False, mean_field="group", placement="blocks"):
+        self.benv, self.rollout_bf16, self.mean_field, self.placement = benv, rollout_bf16, mean_field, placement
 
     def get_view_space(self, handle):
         s = self.benv.sizes
@@ -57,7 +57,7 @@ class BatchedEnvAdapter:
         max_nums, nums, mean_r, total_r = play_batched(self.benv, n_round, max_steps, models, eps=eps, train=train,
                                                        print_every=print_every, left_group=n_round % 2,
                                                        obs_dtype=torch.bfloat16 if self.rollout_bf16 else None,
-                                                       mean_field=self.mean_field)
+                                                       mean_field=self.mean_field, placement=self.placement)
         stats = np.stack([max_nums.mean(axis=0), nums.mean(axis=0), mean_r.mean(axis=0), total_r.mean(axis=0)])
         stats = all_ranks_mean(stats, self.benv.device)     # one decision (self-play update, win count) on every rank
         return tuple(list(row) for row in stats)
@@ -110,7 +110,8 @@ def main(argv=None):
         cap = max(64, int(args.map_size * args.map_size * 0.04))
         benv = BatchedGridWorld(args.envs, map_size=args.map_size, capacity=cap, device=args.device, rng="philox",
                                 env_base=rank * args.envs)
-        env = BatchedEnvAdapter(benv, rollout_bf16=args.rollout_bf16, mean_field=args.mean_field)
+        env = BatchedEnvAdapter(benv, rollout_bf16=args.rollout_bf16, mean_field=args.mean_field,
+                                placement=args.placement)
         handles, play = [0, 1], env.play
     else:
         import magent
